@@ -21,6 +21,11 @@ Primary line  : tracking channel-ms/s on BASELINE.json config 4 ("batched tracki
 `cpu_baseline`: the numpy oracle (a restatement of the reference's loops, oracle/gnss_oracle.py) timed
                 on one host core on a bounded sample.
 `--impl reference` times that CPU path on all host cores (one process per channel / PRN group).
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of each GPU leg returned (rank 0's
+                shard) as DIR/<name>.npy in float64: a fixed, seeded sample of the tracking output's code periods
+                and the acquisition, preamble-search, navigation and config-3 results, each leg within a fixed
+                share of 60 MB (a leg whose output is larger keeps its first recordings).  The inputs are generated
+                from fixed seeds, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -32,6 +37,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                 # the tree may be read-only; leave no __pycache__ in it
 for _v in ("OMP_NUM_THREADS", "OPENBLAS_NUM_THREADS", "MKL_NUM_THREADS"):
     os.environ.setdefault(_v, "1")
 
@@ -45,6 +51,9 @@ ACQ_REC_PER_GPU = 32
 BYTES_PER_CHANNEL_MS = 38192 + 13 * 8          # SURVEY.md 8(d)
 FLOP_PER_CELL = 330.0                          # reference formulation, SURVEY.md 8(d)
 TRACK_CPU_MS = 1000                            # bounded CPU sample (code periods per channel)
+# --dump-outputs: float64 bytes per leg, fixed in advance so that what one leg dumps never depends on another leg's
+# outputs; 60 MB in all, under 64 MB with the npy headers
+DUMP_BUDGET = {"track": 40 * 10 ** 6, "acq": 2 * 10 ** 6, "preamble": 8 * 10 ** 6, "nav": 8 * 10 ** 6, "c3": 2 * 10 ** 6}
 
 
 _RESULT_FD = None
@@ -57,6 +66,35 @@ def emit(line):
         sys.stdout.flush()
     else:
         os.write(_RESULT_FD, data)
+
+
+def track_sample(out, budget):
+    """Tracking output [R, C, 13, ms] at a fixed, seeded set of code periods (every channel, every series) and
+    those periods, as many as fit `budget` bytes in float64; all of it when it fits whole."""
+    import torch
+    r, c, f, ms = out.shape
+    n = max(1, min(ms, budget // ((r * c * f + 1) * 8)))
+    t = np.sort(np.random.default_rng(0).choice(ms, n, replace=False)) if n < ms else np.arange(ms)
+    return out[..., torch.from_numpy(t).to(out.device)].cpu().numpy(), t
+
+
+def leading_rows(arrays, budget):
+    """The arrays of one leg (name -> array, axis 0 = recording or channel), cut to the same first rows so that
+    they fit `budget` bytes in float64; whole when they fit."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    per_row = sum(a[:1].size * 8 for a in arrays.values())
+    n = max(1, budget // max(1, per_row))
+    return {k: a[:n] for k, a in arrays.items()}
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> numeric array; written as path/<name>.npy in float64."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= sum(DUMP_BUDGET.values()), "output dump of %d bytes exceeds the budget" % total
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def peaks():
@@ -209,6 +247,7 @@ def run_gpu(args, rank, world):
     value = world * units / (ms_per_step / 1e3)
     kernel_ms = float(np.mean([ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]))
     lock = out[:, :, 3, 500:].abs().mean().item() / max(out[:, :, 7, 500:].abs().mean().item(), 1e-9) if ms > 600 else None
+    dump = {} if args.dump_outputs and rank == 0 else None     # name -> what the last timed step of a leg returned
 
     # ---- end to end through the C ABI with host buffers --------------------------------------------
     e2e = None
@@ -250,7 +289,7 @@ def run_gpu(args, rank, world):
                 step_host()
             barrier()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            ksteps = max(1, min(args.steps, 3))
+            ksteps = args.steps
             e0.record()
             for _ in range(ksteps):
                 step_host()
@@ -300,6 +339,8 @@ def run_gpu(args, rank, world):
         if world > 1:
             dist.all_reduce(ta, op=dist.ReduceOp.MAX)
         a_ms = float(ta.item()) / args.steps
+        if dump is not None:
+            dump.update(leading_rows({"acq_" + k: v for k, v in res.items()}, DUMP_BUDGET["acq"]))
         ahost = torch.empty((areq, an), dtype=torch.int8, pin_memory=True)
         ahost.copy_(adev)
         ah = ahost.numpy()
@@ -380,6 +421,9 @@ def run_gpu(args, rank, world):
         if world > 1:
             dist.all_reduce(tb, op=dist.ReduceOp.MAX)
         b_ms = float(tb.item()) / args.steps
+        if dump is not None:
+            dump.update(leading_rows(dict(preamble_first=first, preamble_bits=nbits, preamble_valid=nvalid),
+                                     DUMP_BUDGET["preamble"]))
         nch = recs * CHANNELS
         bsync = {"metric": "preamble search channels/s", "value": world * nch / (b_ms / 1e3), "unit": "channels/s",
                  "ms_per_step": b_ms, "gpu_launches": int(L.launches() - bl0),
@@ -426,6 +470,9 @@ def run_gpu(args, rank, world):
         if world > 1:
             dist.all_reduce(tq, op=dist.ReduceOp.MAX)
         q_ms = float(tq.item()) / args.steps
+        if dump is not None:
+            dump.update(leading_rows({"nav_" + k: v for k, v in nout.items() if isinstance(v, np.ndarray)},
+                                     DUMP_BUDGET["nav"]))
         n_fix = int(nout["n_epochs"].sum())
         from softgnss_python_b200 import navsynth
         rx = navsynth.build_scenario(seed=2000 + rank * recs)[1]["rx"]
@@ -485,12 +532,15 @@ def run_gpu(args, rank, world):
             barrier()
             z0, z1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             z0.record()
-            r3 = sd.acquire_sharded(c3dev, cs, stream=stream)
+            for _ in range(args.steps):
+                r3 = sd.acquire_sharded(c3dev, cs, stream=stream)
             z1.record()
             barrier()
-            tz = torch.tensor([z0.elapsed_time(z1)], dtype=torch.float64, device="cuda")
+            tz = torch.tensor([z0.elapsed_time(z1) / args.steps], dtype=torch.float64, device="cuda")
             if world > 1:
                 dist.all_reduce(tz, op=dist.ReduceOp.MAX)
+            if dump is not None:
+                dump.update(leading_rows({"c3_%s_%s" % (name, k): v for k, v in r3.items()}, DUMP_BUDGET["c3"] // 2))
             cells3 = c3n * 32 * 141 * N_CODE
             c3[name] = {"value": cells3 / (float(tz.item()) / 1e3), "unit": "cells/s", "ms_per_step": float(tz.item()),
                         "recordings": c3n, "bins": 141, "prn_per_rank": 32 // world,
@@ -508,10 +558,11 @@ def run_gpu(args, rank, world):
         barrier()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         g0.record()
-        rs = sd.acquire_sharded(adev, aset, stream=stream)
+        for _ in range(args.steps):
+            rs = sd.acquire_sharded(adev, aset, stream=stream)
         g1.record()
         barrier()
-        tg = torch.tensor([g0.elapsed_time(g1)], dtype=torch.float64, device="cuda")
+        tg = torch.tensor([g0.elapsed_time(g1) / args.steps], dtype=torch.float64, device="cuda")
         dist.all_reduce(tg, op=dist.ReduceOp.MAX)
         coll["acquire_sharded_by_prn"] = {"ms": float(tg.item()), "cells_per_s": areq * 32 * 29 * N_CODE / (float(tg.item()) / 1e3),
                                            "note": "the SAME %d recordings on every rank, 32/%d PRNs each, gather included"
@@ -520,19 +571,21 @@ def run_gpu(args, rank, world):
         sd.gather_results(packed, 32 // world * world, axis=2)
         barrier()
         g0.record()
-        for _ in range(10):
+        for _ in range(args.steps):
             sd.gather_results(packed, 32 // world * world, axis=2)
         g1.record()
         barrier()
-        coll["acq_results_gather"] = {"ms": g0.elapsed_time(g1) / 10, "bytes_per_rank": int(packed.numel() * 8),
+        coll["acq_results_gather"] = {"ms": g0.elapsed_time(g1) / args.steps, "bytes_per_rank": int(packed.numel() * 8),
                                       "note": "latency only (SURVEY.md 8(e))"}
         sd.gather_results(out[:1], world, axis=0)
         barrier()
         g0.record()
-        full = sd.gather_results(out, world * recs, axis=0)          # trackResults of all ranks, GPU to GPU
+        for _ in range(args.steps):
+            full = None                                              # at most one gathered copy alive
+            full = sd.gather_results(out, world * recs, axis=0)      # trackResults of all ranks, GPU to GPU
         g1.record()
         barrier()
-        tg = torch.tensor([g0.elapsed_time(g1)], dtype=torch.float64, device="cuda")
+        tg = torch.tensor([g0.elapsed_time(g1) / args.steps], dtype=torch.float64, device="cuda")
         dist.all_reduce(tg, op=dist.ReduceOp.MAX)
         nbytes = int(out.numel() * 8)
         coll["track_results_gather"] = {"ms": float(tg.item()), "bytes_per_rank": nbytes, "total_bytes": nbytes * world,
@@ -549,6 +602,11 @@ def run_gpu(args, rank, world):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if dump is not None:
+        # `out` still holds the last timed tracking step: the later legs only read it
+        dump["track_ms_done"] = done
+        dump["track_out_sample"], dump["track_out_sample_ms"] = track_sample(out, DUMP_BUDGET["track"] - done.size * 8)
+        dump_outputs(args.dump_outputs, dump)
     peak, how = peaks()
     achieved = units * BYTES_PER_CHANNEL_MS / (kernel_ms / 1e3) / 1e9
     traffic = None
@@ -706,7 +764,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-acq", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of every GPU leg to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

@@ -9,14 +9,14 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_module_names_resolve_in_a_clean_interpreter():
+def test_module_names_resolve_in_a_clean_interpreter(tmp_path):
     code = ("import sys; sys.path.insert(0, %r); import acquisition, tracking; "
             "a = acquisition.AcquisitionResult; t = tracking.TrackingResult; "
             "print(all(hasattr(a, m) for m in ('acquire','preRun','showChannelStatus','plot','carrFreq','codePhase','peakMetric','channels','settings','results')), "
             "all(hasattr(t, m) for m in ('track','plot','results','channels','settings')), "
             "callable(acquisition.acquisition), callable(acquisition.preRun), callable(tracking.tracking))"
             % os.path.join(ROOT, "dropin"))
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=str(tmp_path))
     assert out.returncode == 0, out.stderr
     assert out.stdout.split() == ["True"] * 5
 
