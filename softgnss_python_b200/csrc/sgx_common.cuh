@@ -157,6 +157,16 @@ __device__ __forceinline__ unsigned lds_u32(const void* base, unsigned base_s, i
   return v;
 #endif
 }
+__device__ __forceinline__ uint4 lds_u32x4(const void* base, unsigned base_s, int byte_off) {   // 16-byte aligned
+#ifdef SGX_EMUL
+  (void)base_s; return *reinterpret_cast<const uint4*>(reinterpret_cast<const char*>(base) + byte_off);
+#else
+  (void)base; uint4 v;
+  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
+               : "r"(base_s + (unsigned)byte_off));
+  return v;
+#endif
+}
 __device__ __forceinline__ double2 lds_f64x2(const void* base, unsigned base_s, int byte_off) {   // 16-byte aligned
 #ifdef SGX_EMUL
   (void)base_s; return *reinterpret_cast<const double2*>(reinterpret_cast<const char*>(base) + byte_off);

@@ -43,6 +43,9 @@ namespace sgx {
 constexpr int TRK_THREADS = 256;
 constexpr int TRK_WARPS = TRK_THREADS / 32;
 constexpr int TRK_MARGIN = 256;  // extra samples staged beyond samplesPerCode
+// SGX_TRK_PROF phases, stamped by lane 0 of every warp: window wait + prefetch issue, correlate, reduce + barrier,
+// bookkeeping (loop filters, next period's parameters and tables), end-of-period barrier
+constexpr int TRK_PROF_N = 5;
 
 struct TrackArgs {
   const int8_t* rec;
@@ -58,7 +61,7 @@ struct TrackArgs {
   int resume;           // continue every channel from `state` (streaming ingest: the recording arrives in chunks)
   long long avail;      // bytes of every recording that are resident so far (>= rec_len when complete)
   struct TrackState* state;  // [R*C]
-  long long* prof;      // optional [R*C][4] cycle counters (SGX_TRK_PROF=1): correlate, reduce+barrier, bookkeeping, barrier
+  long long* prof;      // optional [R*C][warp][TRK_PROF_N] cycle counters per period phase (SGX_TRK_PROF=1)
   int win;              // bytes per staging buffer, multiple of 16
   long long skip;
   long long abs_base;   // sample index of rec[0] in the file (streamed windows start at the first byte that is needed)
@@ -162,44 +165,62 @@ struct TrackState {   // loop state of one channel between two launches of a str
   int status;   // SGX_OK (finished), SGX_PAUSED, or an error
 };
 
-// T3 + T4 parameters + T5 carry for the next period (code thread)
-__device__ void prepare_code(const TrackArgs& a, CodeState& st, long long rec_len, MsParams& p) {
-  double step = st.codeFreq / a.fs;                                   // :148
-  int blk = (int)ceil((a.codeLength - st.remCodePhase) / step);       // :150
-  p.blk = blk;
-  p.pos = st.pos;
-  p.stop = 0;
-  long long aligned = st.pos & ~15LL;
-  if (st.pos + blk > rec_len) { p.stop = SGX_ERR_SHORT; return; }     // :159
-  if (st.pos + blk > a.avail) { p.stop = SGX_PAUSED; return; }         // wait for the next chunk of the file
-  if (blk <= 0 || (st.pos - aligned) + blk > a.win) { p.stop = SGX_ERR_RANGE; return; }
-  double rem = st.remCodePhase, spc = a.spc, bs = (double)blk * step;
-  p.startE = rem - spc;                                               // :166
-  p.stepE = (((bs + rem) - spc) - p.startE) / (double)blk;
-  p.startL = rem + spc;                                               // :174
-  p.stepL = (((bs + rem) + spc) - p.startL) / (double)blk;
-  p.startP = rem;                                                     // :182
-  p.stepP = ((bs + rem) - p.startP) / (double)blk;
-  p.inv_step = 1.0 / step;
-  p.h_fix = __double2ll_rn(0.5 * p.inv_step * 1099511627776.0);
-  p.q0_fix = __double2ll_rn(-rem * p.inv_step * 1099511627776.0);
-  st.nextRemCode = (lin_y(blk - 1, p.stepP, p.startP) + step) - 1023.0;  // :190
+// T3 + T4 parameters + T5 carry for the next period.  Run by all 32 lanes of one warp with the same state, so that
+// the independent float64 divisions of the chain go to different lanes of one instruction instead of running one
+// after another; lane 0 writes p.
+__device__ void prepare_code(const TrackArgs& a, CodeState& st, long long rec_len, MsParams& p, int lane) {
+  const double step = st.codeFreq / a.fs;                             // :148
+  // lane 0: the block size quotient (:150), lane 1: 1/step (used only to predict event indices)
+  const double q = (lane == 1 ? 1.0 : a.codeLength - st.remCodePhase) / step;
+  const int blk = (int)ceil(__shfl_sync(0xffffffffu, q, 0));
+  const double inv_step = __shfl_sync(0xffffffffu, q, 1);
+  const long long aligned = st.pos & ~15LL;
+  int stop = 0;
+  if (st.pos + blk > rec_len) stop = SGX_ERR_SHORT;                   // :159
+  else if (st.pos + blk > a.avail) stop = SGX_PAUSED;                  // wait for the next chunk of the file
+  else if (blk <= 0 || (st.pos - aligned) + blk > a.win) stop = SGX_ERR_RANGE;
+  if (lane == 0) { p.blk = blk; p.pos = st.pos; p.stop = stop; }
+  if (stop) return;
+  const double rem = st.remCodePhase, spc = a.spc, bs = (double)blk * step;
+  const double startE = rem - spc, startL = rem + spc, startP = rem;  // :166, :174, :182
+  // lanes 0, 1, 2: the E, L, P slopes of np.linspace
+  const double num = lane == 0 ? ((bs + rem) - spc) - startE : lane == 1 ? ((bs + rem) + spc) - startL : (bs + rem) - startP;
+  const double d = num / (double)blk;
+  const double stepE = __shfl_sync(0xffffffffu, d, 0), stepL = __shfl_sync(0xffffffffu, d, 1),
+               stepP = __shfl_sync(0xffffffffu, d, 2);
+  if (lane == 0) {
+    p.startE = startE; p.stepE = stepE;
+    p.startL = startL; p.stepL = stepL;
+    p.startP = startP; p.stepP = stepP;
+    p.inv_step = inv_step;
+    p.h_fix = __double2ll_rn(0.5 * inv_step * 1099511627776.0);
+    p.q0_fix = __double2ll_rn(-rem * inv_step * 1099511627776.0);
+  }
+  st.nextRemCode = (lin_y(blk - 1, stepP, startP) + step) - 1023.0;  // :190
 }
 
-// T6: carrier NCO parameters of the next period (carrier thread)
-__device__ void prepare_carr(const TrackArgs& a, CarrState& st, MsParams& p) {
+// T6: carrier NCO parameters of the next period; returns cps (written to p when `write`)
+__device__ double prepare_carr(const TrackArgs& a, CarrState& st, MsParams& p, bool write) {
   st.w = st.carrFreq * 2.0 * 3.141592653589793;                       // :195
-  p.cps = (st.w / a.fs) * 0.15915494309189535;
-  p.rem_cyc = st.remCarrPhase * 0.15915494309189535;
-  p.w = st.w;
-  p.rem_rad = st.remCarrPhase;
-  p.fs = a.fs;
+  const double cps = (st.w / a.fs) * 0.15915494309189535;
+  if (write) {
+    p.cps = cps;
+    p.w = st.w;
+    p.fs = a.fs;
+  }
+  return cps;
 }
 
-// T6 carry (tracking.py:197): remCarrPhase after a block of `blk` samples
-__device__ double carry_carr_phase(const TrackArgs& a, const CarrState& st, int blk) {
+// T6 phase of the next period (remCarrPhase); p.rem_rad is the loop's copy of it
+__device__ __forceinline__ void set_carr_phase(MsParams& p, double rem) {
+  p.rem_cyc = rem * 0.15915494309189535;
+  p.rem_rad = rem;
+}
+
+// T6 carry (tracking.py:197): remCarrPhase after a block of `blk` samples, from the period's own w and remCarrPhase
+__device__ double carry_carr_phase(double w, double rem, int blk, double fs) {
   const double TWO_PI = 6.283185307179586;  // == 2*np.pi
-  double arg_end = st.w * ((double)blk / a.fs) + st.remCarrPhase;
+  double arg_end = w * ((double)blk / fs) + rem;
   double m;
   if (arg_end >= 0.0) {
     // exact remainder without the iterative fmod: with the right integer quotient the fused
@@ -531,14 +552,23 @@ __device__ __forceinline__ void cis_cycles_f64(double cyc, double& c, double& s)
   sincospi(2.0 * cyc, &s, &c);
 }
 
-// executed by the 32 lanes of the carrier thread's warp once the next period's cps is known
+// executed by the 32 lanes of the carrier warp once the next period's cps is known
 template <int NW>
 __device__ __forceinline__ void build_exact_tables(ExactTables& T, double cps, int lane) {
   constexpr int LMAX = 4 * NW;
   constexpr int ND = ExactDigits<NW>::value;
-  if (lane < LMAX) {
+  // twiddle w^lane on lanes 0 .. LMAX-1, rotor step j (power LMAX-4+j) on lane Z0+j: on the spare lanes next to the
+  // twiddle lanes in the same sincospi when there are enough of them, else in a second pass
+  constexpr int Z0 = (LMAX + 5 <= 32) ? LMAX : 0;
+  const bool tw = lane < LMAX, zs = lane >= Z0 && lane < Z0 + 5;
+  if (tw || (Z0 > 0 && zs)) {
     double c, s;
-    cis_cycles_f64((double)lane * cps, c, s);
+    cis_cycles_f64((double)(tw ? lane : LMAX - 4 + (lane - Z0)) * cps, c, s);
+    if (!tw) {
+      T.z[lane - Z0][0] = c;
+      T.z[lane - Z0][1] = s;
+      return;
+    }
     const double one = (double)(1LL << (8 * ND - 2));      // Q30 (4 digits) or Q38 (5 digits)
     long long w[2] = {__double2ll_rn(c * one), __double2ll_rn(s * one)};
 #pragma unroll
@@ -553,12 +583,7 @@ __device__ __forceinline__ void build_exact_tables(ExactTables& T, double cps, i
       T.tw[q][ND - 1][lane] = (signed char)v;           // |v| <= 65
     }
   }
-  // rotor steps: on spare lanes next to the twiddle lanes when there are any, else afterwards
-  constexpr int Z0 = (LMAX + 5 <= 32) ? LMAX : 0;
-  if (lane >= Z0 && lane < Z0 + 5) {
-    const int j = lane - Z0;
-    cis_cycles_f64((double)(LMAX - 4 + j) * cps, T.z[j][0], T.z[j][1]);
-  }
+  if (Z0 == 0 && zs) cis_cycles_f64((double)(LMAX - 4 + lane) * cps, T.z[lane][0], T.z[lane][1]);
 }
 
 // ---- cold paths of the exact correlator, kept out of line: the unrolled segment loop has to stay inside the SM's
@@ -647,6 +672,15 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
   };
   int a = boundary(n0, qf);
   if ((a & ~IRREGULAR) >= P.blk) return;
+  // Thread 0's first segment (n = -1: the samples before the first prompt threshold) is empty unless the block starts
+  // at or before a threshold.  Skipping it makes that thread's first rotor evaluation (start_rotor, below) fall in
+  // the same iteration as its warp's other lanes: one evaluation per warp instead of two (measured at 32 recordings:
+  // warp 0's correlation ended ~820 cycles after the other warps' with the second evaluation, ~460 without).
+  int s0 = 0;
+  if (n0 < 0) {
+    const int b0 = boundary(0, qf + P.h_fix);
+    if ((b0 & ~IRREGULAR) == (a & ~IRREGULAR)) { s0 = 1; qf += P.h_fix; a = b0; }
+  }
   // packed twiddle digits: tw[c][d] word q holds samples 4q .. 4q+3
   int twr[ND][NW], twi[ND][NW];
 #pragma unroll
@@ -665,7 +699,7 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
   bool fresh = true;
   const unsigned cur_s = smem_addr(cur), z_s = smem_addr(&T.z[0][0]);
 #pragma unroll 1
-  for (int s = 0; s < SEGS; ++s) {
+  for (int s = s0; s < SEGS; ++s) {
     qf += P.h_fix;
     const int b = boundary(n0 + s + 1, qf);
     const int len = (b & ~IRREGULAR) - (a & ~IRREGULAR);
@@ -688,11 +722,25 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
           fresh = false;
         }
         const int sh = ((off + a) & 3) * 8;
-        unsigned raw[NW + 1];
+        unsigned raw[NW + 1];   // the NW + 1 words from the one holding sample a onwards
         {
-          const int wo = (off + a) & ~3;
+          // 16-byte loads from the aligned base: lanes sit ~150 bytes apart, which put the 32-bit loads of a warp
+          // on ~6 distinct banks (6 wavefronts per load); a 16-byte load spreads a quarter warp over 8 bank quads
+          // (2 wavefronts per quarter).  The last quad is fetched only by the lanes that need a word of it.
+          constexpr int NQ = (NW + 7) / 4;          // quads covering words j .. j + NW for every j in 0 .. 3
+          const int ab = (off + a) & ~15, j = ((off + a) >> 2) & 3;
+          unsigned wd[4 * NQ];
 #pragma unroll
-          for (int q = 0; q <= NW; ++q) raw[q] = lds_u32(cur, cur_s, wo + 4 * q);
+          for (int q = 0; q < NQ; ++q) {
+            uint4 v = make_uint4(0u, 0u, 0u, 0u);
+            if (q < NQ - 1 || j + NW >= 4 * (NQ - 1)) v = lds_u32x4(cur, cur_s, ab + 16 * q);
+            wd[4 * q] = v.x; wd[4 * q + 1] = v.y; wd[4 * q + 2] = v.z; wd[4 * q + 3] = v.w;
+          }
+          unsigned t[NW + 2];
+#pragma unroll
+          for (int q = 0; q < NW + 2; ++q) t[q] = (j & 2) ? wd[q + 2] : wd[q];
+#pragma unroll
+          for (int q = 0; q <= NW; ++q) raw[q] = (j & 1) ? t[q + 1] : t[q];
         }
         // bytes at and beyond len are not part of this segment: the last word is always masked, the others only
         // in a short segment (fewer than LMAX - 4 samples: block edges)
@@ -752,11 +800,14 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
   __shared__ float codeS[1040];  // 1025 used; the tail absorbs indices reached only by masked samples
   __shared__ unsigned long long mbar[2];
   __shared__ ExactTables xt;
-  __shared__ CodeState cstS;   // loop state lives in shared memory: only threads 0 / 32 touch it, and keeping it
-  __shared__ CarrState rstS;   // out of the register file leaves the correlator loop without spills
+  __shared__ CodeState cstS;   // loop state lives in shared memory: only warps 0 / 1 touch it, and keeping it
+  __shared__ CarrState rstS;   // out of the register file leaves the correlator loop the registers
   __shared__ __align__(4) unsigned char codeB[EXACT ? 1040 : 4];   // code sign bytes: 0 = +1, 0x80 = -1
+  __shared__ long long stampS[NWARPS][TRK_PROF_N + 1];   // SGX_TRK_PROF phase stamps of the current period
+  __shared__ double remNextS;  // remCarrPhase of the next period (thread 64)
 
   const int tid = threadIdx.x;
+  const int lane = tid & 31;
   const int cid = blockIdx.x;  // recording * n_channels + channel
   const int rid = cid / a.n_channels;
   const sgx_channel chn = a.ch[cid];
@@ -783,28 +834,29 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
     const TrackState* ts = a.state + cid;
     if (ts->status != SGX_PAUSED) return;   // finished (or failed) in an earlier launch
     k_start = ts->k;
-    if (tid == 0) { CodeState c = ts->c; prepare_code(a, c, rec_len, prm); cstS = c; }
-    if (tid == 32) { CarrState r = ts->r; prepare_carr(a, r, prm); rstS = r; }
+    if (tid < 32) { CodeState c = ts->c; prepare_code(a, c, rec_len, prm, lane); if (lane == 0) cstS = c; }
+    if (tid == 32) { CarrState r = ts->r; prepare_carr(a, r, prm, true); set_carr_phase(prm, r.remCarrPhase); rstS = r; }
     if (tid == 0 && BULK) { mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); }
   } else {
-    if (tid == 0) {
+    if (tid < 32) {
       CodeState c;
       c.codeFreq = a.codeFreqBasis;          // :114
       c.remCodePhase = 0.0;
       c.oldCodeNco = c.oldCodeError = 0.0;
       c.nextRemCode = 0.0;
       c.pos = a.skip + (long long)chn.codePhase;  // :107
-      prepare_code(a, c, rec_len, prm);
-      cstS = c;
-      if (BULK) { mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); }
+      prepare_code(a, c, rec_len, prm, lane);
+      if (lane == 0) cstS = c;
     }
+    if (tid == 0 && BULK) { mbar_init(&mbar[0], 1); mbar_init(&mbar[1], 1); }
     if (tid == 32) {
       CarrState r;
       r.carrFreq = chn.acquiredFreq;         // :118
       r.carrFreqBasis = chn.acquiredFreq;
       r.remCarrPhase = 0.0;
       r.oldCarrNco = r.oldCarrError = 0.0;
-      prepare_carr(a, r, prm);
+      prepare_carr(a, r, prm, true);
+      set_carr_phase(prm, r.remCarrPhase);
       rstS = r;
     }
   }
@@ -839,6 +891,11 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
         if (tid == 0) bulk_load(par ? buf1 : buf0, rec + (prm.pos & ~15LL), (unsigned)nb, &mbar[par]);
         if (par) pending1 = true; else pending0 = true;
       }
+      // and the window of the second period (later windows are issued at the end of the bookkeeping); the loop
+      // records it as pending at the start of the first period
+      const long long npos = prm.pos + prm.blk;
+      const int nb1 = stage(par ? buf0 : buf1, npos);
+      if (tid == 0 && nb1 > 0 && k_start < a.ms) bulk_load(par ? buf0 : buf1, rec + (npos & ~15LL), (unsigned)nb1, &mbar[par ^ 1]);
     }
   }
 
@@ -846,8 +903,11 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
   for (; k < a.ms; ++k) {
     const MsParams P = prm;
     if (P.stop != 0) break;
-    long long t0 = 0, t1 = 0, t2 = 0, t3 = 0;
-    if (a.prof && (tid == 0 || tid == 64)) t0 = clock64();
+    const bool stamp = a.prof && (tid & 31) == 0;
+    // (stamps go to shared memory: a register array would hold registers across the whole period, and the compiler
+    // kept it in local memory, with a load on every period's path even with profiling off)
+    long long* ts = stampS[tid >> 5];
+    if (stamp) ts[0] = clock64();
     int8_t* cur = (k & 1) ? buf1 : buf0;
     int8_t* nxt = (k & 1) ? buf0 : buf1;
     // ---- make this period's samples visible ------------------------------------------------
@@ -858,21 +918,26 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
       if (k == k_start) { cp_async_wait_all(); __syncthreads(); }
     }
     // ---- prefetch the next period's window -------------------------------------------------
+    // (bulk copy: issued by thread 0 at the end of the previous period's bookkeeping, or before the loop -- issued
+    // here it delayed warp 0's correlation by ~200 cycles every period)
     {
       long long npos = P.pos + P.blk;
       int nb = stage(nxt, npos);
       if (BULK && nb > 0) {
-        if (tid == 0) bulk_load(nxt, rec + (npos & ~15LL), (unsigned)nb, &mbar[(k + 1) & 1]);
         if (k & 1) pending0 = true; else pending1 = true;
       }
     }
+    // T6 carry (tracking.py:197): remCarrPhase after this period's block needs only this period's parameters; computed
+    // here, on a warp that is not the last to finish its correlation, it is off the bookkeeping's path
+    if (tid == 64) remNextS = carry_carr_phase(P.w, P.rem_rad, P.blk, P.fs);
+    if (stamp) ts[1] = clock64();
 
     double tEr = 0.0, tEi = 0.0, tPr = 0.0, tPi = 0.0, tLr = 0.0, tLi = 0.0;
     if (EXACT)       correlate_exact<(NW > 0 ? NW : 1), 2048 / NT>(P, prm, cur, codeB, xt, tid, tEr, tEi, tPr, tPi, tLr, tLi);
     else if (NW > 0) correlate_segments<(NW > 0 ? NW : 1)>(P, cur, codeS, tid, tEr, tEi, tPr, tPi, tLr, tLi);
     else             correlate_groups(P, cur, codeS, tid, tEr, tEi, tPr, tPi, tLr, tLi);
     // I arm = sin (imaginary part), Q arm = cos (real part): tracking.py:205-207
-    if (a.prof && (tid == 0 || tid == 64)) t1 = clock64();
+    if (stamp) ts[2] = clock64();
     double v0 = warp_sum_f64(tEi), v1 = warp_sum_f64(tEr), v2 = warp_sum_f64(tPi), v3 = warp_sum_f64(tPr),
            v4 = warp_sum_f64(tLi), v5 = warp_sum_f64(tLr);
     if ((tid & 31) == 0) {
@@ -881,55 +946,72 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
     }
     if (!BULK) cp_async_wait_all();
     __syncthreads();
-    if (a.prof && (tid == 0 || tid == 64)) t2 = clock64();
-    if (tid == 0) {          // ---- code thread: DLL (tracking.py:238-251), T5, T3/T4 of the next period
+    if (stamp) ts[3] = clock64();
+    // Bookkeeping: every lane of warp 0 runs the code loop and every lane of warp 1 the carrier loop (same values on
+    // all lanes, so that independent operations of a chain can be spread over lanes); lane 0 writes the results.
+    if (tid < 32) {          // ---- code loop: DLL (tracking.py:238-251), T5, T3/T4 of the next period
       CodeState cst = cstS;
+      const int blk = prm.blk;   // (P.blk would stay live in a register across the correlation)
+      __syncwarp();   // every lane has read the state before lane 0 writes it back
       double I_E = 0.0, Q_E = 0.0, I_L = 0.0, Q_L = 0.0;
       for (int w = 0; w < NWARPS; ++w) { I_E += red[w][0]; Q_E += red[w][1]; I_L += red[w][4]; Q_L += red[w][5]; }
       cst.remCodePhase = cst.nextRemCode;
-      cst.pos = P.pos + P.blk;
-      double em = sqrt(I_E * I_E + Q_E * Q_E), lm = sqrt(I_L * I_L + Q_L * Q_L);
+      cst.pos = cst.pos + blk;   // cst.pos is this period's P.pos
+      const double mag = sqrt(lane == 1 ? I_L * I_L + Q_L * Q_L : I_E * I_E + Q_E * Q_E);   // lane 0: early, 1: late
+      const double em = __shfl_sync(0xffffffffu, mag, 0), lm = __shfl_sync(0xffffffffu, mag, 1);
       double codeError = (em - lm) / (em + lm);
       double codeNco = cst.oldCodeNco + a.c1code * (codeError - cst.oldCodeError) + codeError * a.c2code;
       cst.oldCodeNco = codeNco;
       cst.oldCodeError = codeError;
       cst.codeFreq = a.codeFreqBasis - codeNco;
-      if (k + 1 < a.ms) prepare_code(a, cst, rec_len, prm);
-      double* o = a.out + (long long)cid * SGX_TRACK_FIELDS * a.ms + k;   // record (tracking.py:255-275)
-      const long long m = a.ms;
-      o[0 * m] = (double)(cst.pos + a.abs_base);  // fid.tell() after the read
-      o[1 * m] = cst.codeFreq;
-      o[4 * m] = I_E; o[5 * m] = I_L; o[6 * m] = Q_E; o[8 * m] = Q_L;
-      o[9 * m] = codeError; o[10 * m] = codeNco;
-      cstS = cst;
-    } else if (tid == 32) {  // ---- carrier thread: T6 carry, PLL (tracking.py:223-235), T6 of the next period
+      if (k + 1 < a.ms) prepare_code(a, cst, rec_len, prm, lane);
+      if (lane == 0) {
+        cstS = cst;
+        // window of the period after next, into this period's buffer (all warps are done with it)
+        if (BULK && k + 1 < a.ms && prm.stop == 0) {
+          const long long npos = prm.pos + prm.blk;
+          const int nb = stage(cur, npos);
+          if (nb > 0) bulk_load(cur, rec + (npos & ~15LL), (unsigned)nb, &mbar[k & 1]);
+        }
+        double* o = a.out + (long long)cid * SGX_TRACK_FIELDS * a.ms + k;   // record (tracking.py:255-275)
+        const long long m = a.ms;
+        o[0 * m] = (double)(cst.pos + a.abs_base);  // fid.tell() after the read
+        o[1 * m] = cst.codeFreq;
+        o[4 * m] = I_E; o[5 * m] = I_L; o[6 * m] = Q_E; o[8 * m] = Q_L;
+        o[9 * m] = codeError; o[10 * m] = codeNco;
+      }
+    } else if (tid < 64) {   // ---- carrier loop: PLL (tracking.py:223-235), T6 of the next period, twiddle tables
       CarrState rst = rstS;
+      __syncwarp();   // every lane has read the state before lane 0 writes it back
       double I_P = 0.0, Q_P = 0.0;
       for (int w = 0; w < NWARPS; ++w) { I_P += red[w][2]; Q_P += red[w][3]; }
-      rst.remCarrPhase = carry_carr_phase(a, rst, P.blk);
       double carrError = atan(Q_P / I_P) * 0.5 / 3.141592653589793;   // x/2.0 == x*0.5 exactly
       double carrNco = rst.oldCarrNco + a.c1carr * (carrError - rst.oldCarrError) + carrError * a.c2carr;
       rst.oldCarrNco = carrNco;
       rst.oldCarrError = carrError;
       rst.carrFreq = rst.carrFreqBasis + carrNco;
-      if (k + 1 < a.ms) prepare_carr(a, rst, prm);
-      double* o = a.out + (long long)cid * SGX_TRACK_FIELDS * a.ms + k;
-      const long long m = a.ms;
-      o[2 * m] = rst.carrFreq;
-      o[3 * m] = I_P; o[7 * m] = Q_P;
-      o[11 * m] = carrError; o[12 * m] = carrNco;
-      rstS = rst;
+      if (k + 1 < a.ms) {
+        const double cps = prepare_carr(a, rst, prm, lane == 0);
+        if (EXACT) build_exact_tables<(NW > 0 ? NW : 1)>(xt, cps, lane);
+      }
+      if (lane == 0) {
+        double* o = a.out + (long long)cid * SGX_TRACK_FIELDS * a.ms + k;
+        const long long m = a.ms;
+        o[2 * m] = rst.carrFreq;
+        o[3 * m] = I_P; o[7 * m] = Q_P;
+        o[11 * m] = carrError; o[12 * m] = carrNco;
+        rstS = rst;
+      }
+    } else if (tid == 64) {  // ---- T6 carry, computed at the start of the period
+      set_carr_phase(prm, remNextS);
     }
-    if (EXACT && (tid >> 5) == 1 && k + 1 < a.ms) {
-      const double cps = __shfl_sync(0xffffffffu, tid == 32 ? prm.cps : 0.0, 0);
-      build_exact_tables<(NW > 0 ? NW : 1)>(xt, cps, tid & 31);
-    }
-    if (a.prof && tid == 0) t3 = clock64();
+    if (stamp) ts[4] = clock64();
     __syncthreads();
-    if (a.prof && (tid == 0 || tid == 64)) {
-      const long long t4 = clock64();
-      long long* pr = a.prof + (long long)cid * 8 + (tid == 0 ? 0 : 4);
-      pr[0] += t1 - t0; pr[1] += t2 - t1; pr[2] += (tid == 0 ? t3 - t2 : 0); pr[3] += t4 - (tid == 0 ? t3 : t2);
+    if (stamp) {
+      ts[5] = clock64();
+      long long* pr = a.prof + ((long long)cid * NWARPS + (tid >> 5)) * TRK_PROF_N;
+#pragma unroll
+      for (int i = 0; i < TRK_PROF_N; ++i) pr[i] += ts[i + 1] - ts[i];
     }
   }
   if (BULK) {  // never exit with a bulk copy in flight
@@ -944,7 +1026,11 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
     a.status[cid] = status;
     if (a.state) { a.state[cid].c = cstS; a.state[cid].k = k; a.state[cid].status = status; }
   }
-  if (tid == 32 && a.state) a.state[cid].r = rstS;
+  if (tid == 32 && a.state) {
+    CarrState r = rstS;
+    r.remCarrPhase = prm.rem_rad;
+    a.state[cid].r = r;
+  }
 }
 
 // --------------------------------------------------------------------------- host entry
@@ -1034,9 +1120,10 @@ static int track_core(const int8_t* rec, int64_t rec_stride, const int64_t* rec_
   a.avail = 0x7fffffffffffffffLL;
   a.state = g_trk.state.as<TrackState>();
   a.prof = nullptr;
+  const size_t prof_n = (size_t)nch * TRK_WARPS * TRK_PROF_N;
   if (getenv("SGX_TRK_PROF")) {
-    if (g_trk.prof.reserve(sizeof(long long) * 8 * nch)) return fail(SGX_ERR_CUDA, "cudaMalloc", "prof");
-    SGX_CUDA(cudaMemsetAsync(g_trk.prof.p, 0, sizeof(long long) * 8 * nch, s));
+    if (g_trk.prof.reserve(sizeof(long long) * prof_n)) return fail(SGX_ERR_CUDA, "cudaMalloc", "prof");
+    SGX_CUDA(cudaMemsetAsync(g_trk.prof.p, 0, sizeof(long long) * prof_n, s));
     a.prof = g_trk.prof.as<long long>();
   }
   a.win = win;
@@ -1153,15 +1240,19 @@ static int track_core(const int8_t* rec, int64_t rec_stride, const int64_t* rec_
   SGX_CUDA(cudaMemcpyAsync(ms_done, a.ms_done, sizeof(int) * nch, cudaMemcpyDeviceToHost, s));
   SGX_CUDA(cudaMemcpyAsync(h_status, a.status, sizeof(int) * nch, cudaMemcpyDeviceToHost, s));
   SGX_CUDA(cudaStreamSynchronize(s));
-  if (a.prof) {
-    long long* hp = (long long*)malloc(sizeof(long long) * 8 * nch);
-    cudaMemcpy(hp, a.prof, sizeof(long long) * 8 * nch, cudaMemcpyDeviceToHost);
-    double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    for (int i = 0; i < nch; ++i) for (int j = 0; j < 8; ++j) acc[j] += (double)hp[i * 8 + j];
+  if (a.prof) {   // mean cycles per period of every warp over all channels and periods of the last launch
+    std::vector<long long> hp(prof_n);
+    cudaMemcpy(hp.data(), a.prof, sizeof(long long) * prof_n, cudaMemcpyDeviceToHost);
     const double per = (double)nch * ms;
-    fprintf(stderr, "[sgx prof] cycles/period thread0: correlate %.0f reduce+bar %.0f bookkeeping %.0f bar %.0f | thread64: correlate %.0f reduce+bar %.0f wait-for-bookkeeping %.0f\n",
-            acc[0] / per, acc[1] / per, acc[2] / per, acc[3] / per, acc[4] / per, acc[5] / per, acc[7] / per);
-    free(hp);
+    fprintf(stderr, "[sgx prof] cycles/period  warp:  wait+prefetch  correlate  reduce+bar  bookkeeping  bar  | period\n");
+    for (int w = 0; w < TRK_WARPS; ++w) {
+      double acc[TRK_PROF_N] = {}, tot = 0.0;
+      for (int i = 0; i < nch; ++i)
+        for (int j = 0; j < TRK_PROF_N; ++j) acc[j] += (double)hp[((size_t)i * TRK_WARPS + w) * TRK_PROF_N + j];
+      for (int j = 0; j < TRK_PROF_N; ++j) tot += acc[j];
+      fprintf(stderr, "[sgx prof] %d: %8.0f %8.0f %8.0f %8.0f %8.0f | %8.0f\n", w, acc[0] / per, acc[1] / per, acc[2] / per,
+              acc[3] / per, acc[4] / per, tot / per);
+    }
   }
   int rc = SGX_OK;
   for (int i = 0; i < nch; ++i)
