@@ -3,4 +3,4 @@ import os
 import sys
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from softgnss_python_b200.tracking import TrackingResult, tracking  # noqa: E402,F401
+from softgnss_python_b200.tracking import TrackingResult, cno_vsm, tracking  # noqa: E402,F401

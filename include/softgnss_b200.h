@@ -195,6 +195,39 @@ int sgx_pseudoranges(const double* track_out, int32_t n_recordings, int32_t n_ch
                      double samples_per_code, double start_offset, double c, double* pseudoranges,
                      void* cuda_stream);
 
+/* ---- tracking quality: C/N0 and carrier lock per window (extension; no reference behaviour) ---------------- */
+/* Settings of sgx_track_quality.  The Matlab SoftGNSS line computes the same estimator in CNoVSM.m with
+ * settings.CNo.VSMinterval = 40 and settings.CNo.accTime = 0.001. */
+typedef struct sgx_quality_settings {
+  double acc_time;      /* s per I/Q sample: 0.001 */
+  double cn0_min;       /* dB-Hz: a window is locked only if cn0 >= cn0_min */
+  double pll_lock_min;  /* cos 2dphi: ... and pll_lock >= pll_lock_min */
+  int32_t window_ms;    /* W >= 2 code periods per estimate */
+  int32_t reserved;
+} sgx_quality_settings;
+
+/* Variance-summing-method C/N0 and the narrow-band carrier-lock indicator of n_channels tracked channels, one value
+ * per window of W = window_ms code periods, n_win = ms / W (windows w = 0 .. n_win-1 hold periods w*W .. w*W+W-1).
+ * With I_k, Q_k the prompt samples of the window and all arithmetic in float64:
+ *   Z_k = I_k^2 + Q_k^2,  Zm = mean(Z),  Zv = sum((Z_k - Zm)^2) / (W - 1)
+ *   Pav = sqrt(Zm^2 - Zv),  Nv = 0.5 * (Zm - Pav),  cn0 = 10 * log10(Pav / (2 * Nv * acc_time))   [dB-Hz]
+ *   pll_lock = sum(I_k^2 - Q_k^2) / sum(I_k^2 + Q_k^2)        (cos 2dphi; independent of the nav-bit signs)
+ *   locked = cn0 >= cn0_min && pll_lock >= pll_lock_min       (NaN compares false)
+ * cn0 is NaN unless Zm^2 - Zv > 0 and Nv > 0 (CNoVSM.m instead takes abs() of the complex value it gets there);
+ * pll_lock is NaN when its denominator is 0.  A window is valid iff (w+1)*W <= ms_done[c]; invalid windows get NaN,
+ * NaN, 0 (idle channels of sgx_track have ms_done = 0).  Deterministic: fixed reduction order, no atomics.
+ *   i_p, q_p  double [n_channels][stride], ms values used per row; both host or both device memory.  Reads
+ *             sgx_track's output in place: i_p = out + 3*ms, q_p = out + 7*ms, stride = SGX_TRACK_FIELDS*ms,
+ *             n_channels = n_recordings * channels.  Host rows are copied row by row (2 * n_channels rows of ms).
+ *   ms_done   host int32 [n_channels] periods completed per channel, each in [0, ms]; NULL: all ms
+ *   cn0, pll_lock (double), locked (uint8)  [n_channels][n_win], all three host or all three device memory; host
+ *             outputs synchronise the stream, device outputs leave the call asynchronous.
+ * SGX_ERR_ARG for window_ms < 2, acc_time not finite and > 0, stride < ms, ms_done outside [0, ms], a NULL pointer
+ * or mixed host/device operands.  n_win == 0 succeeds without work. */
+int sgx_track_quality(const double* i_p, const double* q_p, int64_t stride, int32_t n_channels, int32_t ms,
+                      const int32_t* ms_done, const sgx_quality_settings* qs, double* cn0, double* pll_lock,
+                      uint8_t* locked, void* cuda_stream);
+
 /* ---- navigation solution (SURVEY.md section 8(f) row 4, second half) -------------------------------------- */
 /* Broadcast-ephemeris terms read by geoFunctions.satpos (geoFunctions/__init__.py:779-885), one per channel,
  * in the units ephemeris.py decodes them to (seconds, radians, metres). */

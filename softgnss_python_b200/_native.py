@@ -20,7 +20,7 @@ SGX_ERR_SHORT = -3
 
 EXPORTS = ("sgx_abi_version", "sgx_last_error", "sgx_device_count", "sgx_set_device", "sgx_fp32_peak",
            "sgx_kernel_launch_count", "sgx_acquire", "sgx_track", "sgx_track_file", "sgx_synth_generate", "sgx_fft_c2c",
-           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve")
+           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality")
 
 
 class NativeError(RuntimeError):
@@ -43,6 +43,11 @@ class SgxNavSettings(ctypes.Structure):
     _fields_ = [("samples_per_code", ctypes.c_double), ("start_offset", ctypes.c_double), ("c", ctypes.c_double),
                 ("nav_sol_period", ctypes.c_double), ("elevation_mask", ctypes.c_double),
                 ("use_trop_corr", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
+class SgxQualitySettings(ctypes.Structure):
+    _fields_ = [("acc_time", ctypes.c_double), ("cn0_min", ctypes.c_double), ("pll_lock_min", ctypes.c_double),
+                ("window_ms", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
 class SgxSynthSpec(ctypes.Structure):
@@ -174,6 +179,21 @@ class Lib(object):
                                              float(samples_per_code), float(start_offset), float(c), _ptr(out),
                                              ctypes.c_void_p(stream)))
         return out
+
+    def track_quality(self, i_p, q_p, stride, n_channels, ms, ms_done, qs, cn0, pll_lock, locked, stream=0):
+        """Per-window C/N0 / carrier lock (sgx_track_quality).  i_p, q_p: float64 numpy arrays, CUDA tensors or
+        addresses whose channel rows are `stride` apart; ms_done: int32 [n_channels] or None; qs: SgxQualitySettings;
+        cn0, pll_lock (float64) and locked (uint8) [n_channels][ms // qs.window_ms], written in place.  Returns rc."""
+        self.require_device()
+        if ms_done is not None:
+            ms_done = np.ascontiguousarray(ms_done, dtype=np.int32).reshape(-1)
+            assert ms_done.size == n_channels
+        vp, i32 = ctypes.c_void_p, ctypes.c_int32
+        self.dll.sgx_track_quality.argtypes = [vp, vp, ctypes.c_int64, i32, i32, vp, ctypes.POINTER(SgxQualitySettings),
+                                               vp, vp, vp, vp]
+        return self.dll.sgx_track_quality(_ptr(i_p), _ptr(q_p), int(stride), int(n_channels), int(ms), _ptr(ms_done),
+                                          ctypes.byref(qs), _ptr(cn0), _ptr(pll_lock), _ptr(locked),
+                                          ctypes.c_void_p(stream))
 
     def nav_solve(self, abs_sample, stride, n_rec, n_ch, ms, sub_frame_start, ready, eph, tow, n_epochs, nav_settings,
                   want_sat=True, stream=0):

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsoftgnss_b200.so")
-SOURCES = ["sgx_api.cu", "sgx_track.cu", "sgx_synth.cu", "sgx_acq.cu", "sgx_pfa.cu", "sgx_fine.cu", "sgx_bitsync.cu", "sgx_nav.cu"]
+SOURCES = ["sgx_api.cu", "sgx_track.cu", "sgx_synth.cu", "sgx_acq.cu", "sgx_pfa.cu", "sgx_fine.cu", "sgx_bitsync.cu", "sgx_nav.cu", "sgx_quality.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false", "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--use_fast_math=false"]
 

@@ -16,6 +16,10 @@ Extension attributes (not in the reference; defaults reproduce it):
 ``acqDopplerStep`` (500 Hz, literal at ``acquisition.py:101``),
 ``acqCoherentMs`` (1) and ``acqNonCoherentBlocks`` (2, the pick-max of two 1 ms
 blocks at ``acquisition.py:129-133``).
+Tracking-quality extensions, read by ``tracking.cno_vsm`` / ``track_quality_batch`` (with these defaults when an
+object lacks them): ``CNoVSMinterval`` (40 code periods per C/N0 estimate, Matlab ``settings.CNo.VSMinterval``),
+``CNoAccTime`` (0.001 s per prompt sample, ``settings.CNo.accTime``), ``lockCNoMin`` (30.0 dB-Hz) and ``lockPllMin``
+(0.5, cos 2 dphi): a window counts as locked when its C/N0 and its carrier-lock indicator reach both.
 """
 import ctypes
 
@@ -73,6 +77,7 @@ class Settings(object):
         navSolPeriod=500.0, elevationMask=10.0, useTropCorr=True, plotTracking=True,
         # extensions (defaults == reference behaviour)
         acqDopplerStep=500.0, acqCoherentMs=1, acqNonCoherentBlocks=2,
+        CNoVSMinterval=40, CNoAccTime=0.001, lockCNoMin=30.0, lockPllMin=0.5,
     )
 
     def __init__(self, **overrides):

@@ -11,6 +11,9 @@ the reference's recarray (``tracking.py:285-294``): one record per channel whose
 ``status`` ('S1'), thirteen float64[msToProcess] series as object fields, ``PRN`` int64.
 On a short recording the reference prints a message and returns None (``tracking.py:159-163``);
 so does this.
+
+Extension (no reference behaviour): the per-channel C/N0 and lock detector of the later Matlab SoftGNSS releases
+(``CNoVSM``), as ``track_quality_batch`` on a batched tracking result and ``cno_vsm`` on the recarray.
 """
 import numpy as np
 
@@ -111,6 +114,81 @@ def track_batch(recordings, rec_len, channel_sets, settings, out=None, stream=0)
     stride = recordings.stride(0) if hasattr(recordings, "data_ptr") else recordings.strides[0]
     rc, done = L.track(recordings, stride, rec_len, chans, pod, _native.ca_chips_int8(), out, stream)
     return rc, out, done
+
+
+QUALITY_DTYPE = [('PRN', 'int64'), ('VSMValue', 'object'), ('VSMIndex', 'object'), ('pllLock', 'object'),
+                 ('locked', 'object')]
+
+
+def quality_pod(settings=None):
+    """``sgx_quality_settings`` from the extension attributes ``CNoVSMinterval``, ``CNoAccTime``, ``lockCNoMin`` and
+    ``lockPllMin``; an object without them (the reference's own Settings, or None) gets their defaults."""
+    g = lambda name, default: getattr(settings, name, default)
+    return _native.SgxQualitySettings(acc_time=float(g("CNoAccTime", 0.001)), cn0_min=float(g("lockCNoMin", 30.0)),
+                                      pll_lock_min=float(g("lockPllMin", 0.5)),
+                                      window_ms=int(g("CNoVSMinterval", 40)), reserved=0)
+
+
+def track_quality_batch(track_out, ms_done=None, settings=None, stream=0):
+    """C/N0 (variance-summing method) and carrier lock per window of ``settings.CNoVSMinterval`` code periods for
+    every channel of a tracking result, computed by ``sgx_track_quality`` (csrc/sgx_quality.cu).
+
+    ``track_out``: float64 ``[R, C, 13, ms]`` as ``track_batch`` returns it, a numpy array or a contiguous CUDA
+    tensor; the I_P and Q_P fields are read in place.  ``ms_done``: ``[R, C]`` periods completed (``track_batch``'s
+    third result) or None for all ``ms``.  Returns ``dict(cn0, pllLock, locked, index)``: the first three ``[R, C,
+    n_win]`` (float64, float64, uint8; numpy for a numpy input, CUDA tensors on the input's device otherwise, written
+    asynchronously on ``stream``), ``index`` int64 ``[n_win]`` = ``(w + 1) * W``, the period count at which window w
+    is complete (Matlab's ``VSMIndex``).  There is no host implementation: without a device this raises NativeError."""
+    L = _native.lib()
+    L.require_device()
+    qs = quality_pod(settings)
+    nf = len(FIELDS)
+    on_device = hasattr(track_out, "data_ptr")
+    if not on_device:
+        track_out = np.ascontiguousarray(track_out, dtype=np.float64)
+    r, c, f, ms = track_out.shape
+    assert f == nf, "track_out must be [R, C, %d, ms]" % nf
+    n_win = ms // qs.window_ms if qs.window_ms >= 2 else 0   # W < 2 is refused by the library
+    if on_device:
+        import torch
+        assert track_out.is_cuda and track_out.dtype == torch.float64 and track_out.is_contiguous()
+        base = track_out.data_ptr()
+        res = dict(cn0=torch.empty((r, c, n_win), dtype=torch.float64, device=track_out.device),
+                   pllLock=torch.empty((r, c, n_win), dtype=torch.float64, device=track_out.device),
+                   locked=torch.empty((r, c, n_win), dtype=torch.uint8, device=track_out.device))
+    else:
+        base = track_out.ctypes.data
+        res = dict(cn0=np.empty((r, c, n_win)), pllLock=np.empty((r, c, n_win)),
+                   locked=np.empty((r, c, n_win), dtype=np.uint8))
+    done = None if ms_done is None else np.ascontiguousarray(ms_done, dtype=np.int32).reshape(r * c)
+    i_p, q_p = base + 8 * FIELDS.index("I_P") * ms, base + 8 * FIELDS.index("Q_P") * ms
+    if n_win or qs.window_ms < 2:           # (an empty CUDA tensor has no address to pass)
+        L.check(L.track_quality(i_p, q_p, nf * ms, r * c, ms, done, qs, res["cn0"], res["pllLock"], res["locked"],
+                                stream))
+    res["index"] = (np.arange(n_win, dtype=np.int64) + 1) * qs.window_ms
+    return res
+
+
+def cno_vsm(trackResults, settings):
+    """Function-style mirror of the Matlab SoftGNSS ``CNoVSM`` stage on the tracking recarray: one record per tracked
+    channel with ``PRN`` and the object fields ``VSMValue`` (C/N0 per window, dB-Hz, NaN where undefined),
+    ``VSMIndex`` (``(w + 1) * CNoVSMinterval``), ``pllLock`` (cos 2 dphi per window) and ``locked`` (uint8).  Computed
+    on the device by ``sgx_track_quality``; raises NativeError without one."""
+    L = _native.lib()
+    L.require_device()
+    qs = quality_pod(settings)
+    n = len(trackResults)
+    if n == 0:
+        return np.recarray((0,), dtype=QUALITY_DTYPE)
+    i_p = np.ascontiguousarray(np.stack([np.asarray(trackResults[k].I_P, dtype=np.float64) for k in range(n)]))
+    q_p = np.ascontiguousarray(np.stack([np.asarray(trackResults[k].Q_P, dtype=np.float64) for k in range(n)]))
+    ms = i_p.shape[1]
+    n_win = ms // qs.window_ms if qs.window_ms >= 2 else 0   # W < 2 is refused by the library
+    cn0, pll, locked = np.empty((n, n_win)), np.empty((n, n_win)), np.empty((n, n_win), dtype=np.uint8)
+    L.check(L.track_quality(i_p, q_p, ms, n, ms, None, qs, cn0, pll, locked))
+    index = (np.arange(n_win, dtype=np.int64) + 1) * qs.window_ms
+    recs = [(int(trackResults[k].PRN), cn0[k], index.copy(), pll[k], locked[k]) for k in range(n)]
+    return np.rec.fromrecords(recs, dtype=QUALITY_DTYPE)
 
 
 def tracking(fid, channel, settings):

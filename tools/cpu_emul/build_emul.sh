@@ -9,7 +9,7 @@ SRC=$ROOT/softgnss_python_b200/csrc
 mkdir -p "$HERE/obj"
 NEWEST_HDR=$(ls -t "$SRC"/*.cuh "$SRC"/*.h "$HERE/cuda_emul.h" "$ROOT/include/softgnss_b200.h" | head -1)
 OBJS=""
-for f in sgx_api.cu sgx_track.cu sgx_synth.cu sgx_acq.cu sgx_pfa.cu sgx_fine.cu sgx_bitsync.cu sgx_nav.cu; do
+for f in sgx_api.cu sgx_track.cu sgx_synth.cu sgx_acq.cu sgx_pfa.cu sgx_fine.cu sgx_bitsync.cu sgx_nav.cu sgx_quality.cu; do
   [ -f "$SRC/$f" ] || continue
   o="$HERE/obj/${f%.cu}.o"
   OBJS="$OBJS $o"
