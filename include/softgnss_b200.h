@@ -275,6 +275,58 @@ int sgx_nav_solve(const double* abs_sample, int64_t stride, int32_t n_recordings
                   double* corrected_p, double* el, double* az, double* sat_pos, double* sat_clk, uint8_t* active,
                   double* sol, void* cuda_stream);
 
+/* ---- velocity and clock drift from Doppler (extension; no reference behaviour) -------------------------------- */
+typedef struct sgx_vel_settings {
+  double IF;               /* Hz: settings.IF, subtracted from the PLL's carrier frequency */
+  double c;                /* m/s: settings.c */
+  double f_L1;             /* Hz: 1575.42e6 */
+  double nav_sol_period;   /* ms between epochs: settings.navSolPeriod, as in sgx_nav_settings */
+  int32_t doppler_avg_ms;  /* N >= 1 code periods averaged per Doppler (default 100) */
+  int32_t reserved;
+} sgx_vel_settings;
+
+#define SGX_NAV_VEL_FIELDS 8   /* VX VY VZ (ECEF, m/s) clock drift (m/s) VE VN VU (m/s) channels used */
+
+/* Receiver velocity and clock drift at the measurement epochs of sgx_nav_solve, from the carrier frequency the PLL
+ * tracked (field 2 of sgx_track's output).  Float64 throughout.  For recording r, epoch e < n_epochs[r], channel c:
+ *   m = sub_frame_start[c] + (int)nav_sol_period * e (K8's msOfTheSignal); transmit time t = tow[r] advanced by e
+ *   repeated additions of nav_sol_period / 1000 (as sgx_nav_solve)
+ *   D = sum(carr_freq[m-N+1 .. m], increasing index) / N - IF   with N = doppler_avg_ms; D = NaN (channel excluded)
+ *       when m-N+1 < 0 or m >= ms_done[c].  The window trails the epoch by (N-1)/2 ms.
+ *   measured range rate rr = -(c / f_L1) * D
+ *   satellite position, clock and their analytic time derivatives from the ephemeris at t (the arithmetic of
+ *   satpos, geoFunctions/__init__.py:779-885): Edot = n / (1 - e cosE), nudot = Edot sqrt(1-e^2) / (1 - e cosE),
+ *   udot = nudot (1 + 2 (C_us cos2phi - C_uc sin2phi)), rdot = a e sinE Edot + 2 nudot (C_rs cos2phi - C_rc sin2phi),
+ *   idot = iDot + 2 nudot (C_is cos2phi - C_ic sin2phi), Omegadot = omegaDot - 7.2921151467e-5;
+ *   satellite clock drift = a_f1 + 2 a_f2 dt + F e sqrtA cosE Edot
+ *   Earth rotation: tau = |x_s - x_r| / c once, x_r the epoch's fix (sol X Y Z); x_s and v_s rotated about z by
+ *   7.292115147e-5 * tau (e_r_corr's constant).  The rate of that rotation angle (< 1 cm/s) is ignored.
+ *   channels used: active[r][e][c] == 1 and D finite.  With u_c = (x_s,rot - x_r) / |x_s,rot - x_r| the row is
+ *   [-u_c, 1] and y_c = rr_c - u_c . v_s,rot + c * satellite clock drift; the 4x4 normal equations are solved by
+ *   Cholesky for (vx, vy, vz, c * receiver clock drift).  The epoch is NaN when its fix is NaN, when fewer than 4
+ *   channels are used, or when a Cholesky pivot is not above 1e-13 of the trace.
+ *   carr_freq        double: the carrFreq series of channel (r, c) starts at carr_freq + (r*n_channels + c)*stride and
+ *                    holds ms values (sgx_track's output + 2*ms, stride = SGX_TRACK_FIELDS*ms; host or device; host
+ *                    rows are copied one row each)
+ *   ms_done          host int32 [R][C] periods completed, each in [0, ms]; NULL: all ms
+ *   sub_frame_start, eph, tow, n_epochs, max_epochs  as given to sgx_nav_solve
+ *   active           uint8 [R][E][C], sol double [R][E][SGX_NAV_SOL_FIELDS]: sgx_nav_solve's outputs (host or device)
+ * Outputs (each host or device; a host output makes the call synchronous), E = max_epochs:
+ *   vel       double [R][E][SGX_NAV_VEL_FIELDS]: VX VY VZ, clock drift, VE VN VU (rotated at sol's latitude and
+ *             longitude), channels used (the count of the rule above, also when the epoch is NaN)
+ *   doppler   double [R][E][C] D in Hz of the channels used, NaN elsewhere
+ *   rr_resid  double [R][E][C] post-fit range-rate residual y_c - row_c . x (m/s), NaN unless used in a solution
+ *   sat_vel   double [R][E][C][3], sat_clk_drift double [R][E][C] (s/s): unrotated satellite velocity and clock drift
+ *             of the active channels, NaN elsewhere (optional, may be NULL)
+ * Epochs >= n_epochs[r] are NaN with 0 channels used.  Deterministic: fixed summation order, no atomics.
+ * SGX_ERR_ARG for NULL required pointers, 1..32 channels, ms <= 0, stride < ms, ms_done outside [0, ms],
+ * doppler_avg_ms < 1, nav_sol_period < 1, c, f_L1 not finite and > 0 or IF not finite. */
+int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t n_recordings, int32_t n_channels, int32_t ms,
+                     const int32_t* ms_done, const int32_t* sub_frame_start, const sgx_eph* eph, const double* tow,
+                     const int32_t* n_epochs, int32_t max_epochs, const uint8_t* active, const double* sol,
+                     const sgx_vel_settings* vs, double* vel, double* doppler, double* rr_resid, double* sat_vel,
+                     double* sat_clk_drift, void* cuda_stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -20,7 +20,7 @@ SGX_ERR_SHORT = -3
 
 EXPORTS = ("sgx_abi_version", "sgx_last_error", "sgx_device_count", "sgx_set_device", "sgx_fp32_peak",
            "sgx_kernel_launch_count", "sgx_acquire", "sgx_track", "sgx_track_file", "sgx_synth_generate", "sgx_fft_c2c",
-           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality")
+           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality", "sgx_nav_velocity")
 
 
 class NativeError(RuntimeError):
@@ -37,6 +37,7 @@ class SgxChannel(ctypes.Structure):
 EPH_FIELDS = ("t_oc", "a_f2", "a_f1", "a_f0", "T_GD", "sqrtA", "t_oe", "deltan", "M_0", "e", "omega",
               "C_uc", "C_us", "C_rc", "C_rs", "i_0", "iDot", "C_ic", "C_is", "omega_0", "omegaDot")   # sgx_eph, in order
 NAV_SOL_FIELDS = ("X", "Y", "Z", "dt", "GDOP", "PDOP", "HDOP", "VDOP", "TDOP", "latitude", "longitude", "height")
+NAV_VEL_FIELDS = ("VX", "VY", "VZ", "clkDrift", "VE", "VN", "VU", "nUsed")                  # SGX_NAV_VEL_FIELDS
 
 
 class SgxNavSettings(ctypes.Structure):
@@ -48,6 +49,11 @@ class SgxNavSettings(ctypes.Structure):
 class SgxQualitySettings(ctypes.Structure):
     _fields_ = [("acc_time", ctypes.c_double), ("cn0_min", ctypes.c_double), ("pll_lock_min", ctypes.c_double),
                 ("window_ms", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
+class SgxVelSettings(ctypes.Structure):
+    _fields_ = [("IF", ctypes.c_double), ("c", ctypes.c_double), ("f_L1", ctypes.c_double),
+                ("nav_sol_period", ctypes.c_double), ("doppler_avg_ms", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
 class SgxSynthSpec(ctypes.Structure):
@@ -90,6 +96,9 @@ class Lib(object):
         d.sgx_track.argtypes = [vp, i64, vp, i32, vp, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, vp]
         d.sgx_track_file.argtypes = [ctypes.c_char_p, i32, vp, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, i64, vp, vp]
         d.sgx_synth_generate.argtypes = [vp, i64, i64, i64, i32, vp, vp, vp, vp, vp]
+        if hasattr(d, "sgx_nav_velocity"):
+            d.sgx_nav_velocity.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
+                                           ctypes.POINTER(SgxVelSettings), vp, vp, vp, vp, vp, vp]
         if hasattr(d, "sgx_acquire"):
             d.sgx_acquire.argtypes = [vp, i64, i64, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, i32, i32,
                                       vp, vp, vp, vp, vp, vp]
@@ -221,6 +230,37 @@ class Lib(object):
                                           _ptr(out["satClkCorr"]), _ptr(out["active"]), _ptr(out["sol"]),
                                           ctypes.c_void_p(stream)))
         out["n_epochs"] = n_epochs
+        return out
+
+    def nav_velocity(self, carr_freq, stride, n_rec, n_ch, ms, ms_done, sub_frame_start, eph, tow, n_epochs, active, sol,
+                     vel_settings, want_sat=False, out=None, stream=0):
+        """Velocity and clock drift per epoch (sgx_nav_velocity).  carr_freq: float64 numpy array, CUDA tensor or address
+        whose channel rows are `stride` apart; ms_done int32 [n_rec][n_ch] or None; sub_frame_start / eph / tow /
+        n_epochs as for nav_solve; active uint8 [n_rec][E][n_ch] and sol float64 [n_rec][E][12]: nav_solve's outputs
+        (numpy or CUDA tensors).  ``out``: optional dict of preallocated outputs (vel, doppler, rrResid and, with
+        want_sat, satVel, satClkDrift; numpy or CUDA tensors); by default numpy arrays are allocated.  Returns that dict."""
+        self.require_device()
+        if ms_done is not None:
+            ms_done = np.ascontiguousarray(ms_done, dtype=np.int32).reshape(n_rec, n_ch)
+        sub_frame_start = np.ascontiguousarray(sub_frame_start, dtype=np.int32).reshape(n_rec, n_ch)
+        eph = np.ascontiguousarray(eph, dtype=np.float64).reshape(n_rec, n_ch, len(EPH_FIELDS))
+        tow = np.ascontiguousarray(tow, dtype=np.float64).reshape(n_rec)
+        n_epochs = np.ascontiguousarray(n_epochs, dtype=np.int32).reshape(n_rec)
+        if isinstance(active, np.ndarray):
+            active = np.ascontiguousarray(active, dtype=np.uint8)
+        if isinstance(sol, np.ndarray):
+            sol = np.ascontiguousarray(sol, dtype=np.float64)
+        e_max = int(sol.shape[1])
+        assert tuple(active.shape) == (n_rec, e_max, n_ch) and tuple(sol.shape) == (n_rec, e_max, len(NAV_SOL_FIELDS))
+        shp = (n_rec, e_max, n_ch)
+        if out is None:
+            out = dict(vel=np.empty((n_rec, e_max, len(NAV_VEL_FIELDS))), doppler=np.empty(shp), rrResid=np.empty(shp),
+                       satVel=np.empty(shp + (3,)) if want_sat else None, satClkDrift=np.empty(shp) if want_sat else None)
+        self.check(self.dll.sgx_nav_velocity(_ptr(carr_freq), int(stride), n_rec, n_ch, int(ms), _ptr(ms_done),
+                                             _ptr(sub_frame_start), _ptr(eph), _ptr(tow), _ptr(n_epochs), e_max,
+                                             _ptr(active), _ptr(sol), ctypes.byref(vel_settings), _ptr(out["vel"]),
+                                             _ptr(out["doppler"]), _ptr(out["rrResid"]), _ptr(out.get("satVel")),
+                                             _ptr(out.get("satClkDrift")), ctypes.c_void_p(stream)))
         return out
 
     # ------------------------------------------------------------------ synthetic recordings

@@ -18,6 +18,11 @@
 // -fmad=false); what differs from numpy is the last-ulp rounding of sin/cos/atan2/pow and the solver of the
 // 8x4 least-squares step (Cholesky on the normal equations instead of LAPACK gelsd) -- see DESIGN.md for
 // the tolerance this gives (1e-5 m on the fix).
+//
+// nav_velocity_kernel (K10, an extension with no reference behaviour) reuses satpos_one and the helpers above: receiver
+// velocity and clock drift at the same epochs from the PLL's carrier frequency, one warp per (recording, epoch).
+#include <math.h>
+
 #include "sgx_common.cuh"
 
 namespace sgx {
@@ -424,6 +429,183 @@ __global__ void __launch_bounds__(128) nav_solve_kernel(NavArgs a) {
   }
 }
 
+// ---- K10: receiver velocity and clock drift from the PLL's Doppler (extension; contract in softgnss_b200.h) -------
+struct VelArgs {
+  const double* carr_freq;    // row (r, c) = carr_freq + (r*n_ch + c)*stride, ms values
+  long long stride;
+  const int* ms_done;         // [R][C] or null (all ms)
+  const int* sub_frame_start; // [R][C]
+  const sgx_eph* eph;         // [R][C]
+  const double* tow;          // [R]
+  const int* n_epochs;        // [R]
+  const unsigned char* active;// [R][E][C]
+  const double* sol;          // [R][E][SGX_NAV_SOL_FIELDS]
+  int n_rec, n_ch, ms, max_epochs;
+  sgx_vel_settings st;
+  double* vel;                // [R][E][SGX_NAV_VEL_FIELDS]
+  double* doppler;            // [R][E][C]
+  double* rr_resid;           // [R][E][C]
+  double* sat_vel;            // [R][E][C][3] or null
+  double* sat_clk_drift;      // [R][E][C] or null
+};
+
+// Time derivatives of satpos_one's position and clock at the same transmit time: its anomaly chain recomputed with the
+// same expressions, then every term of the ECEF formulas differentiated (dt/dt of the transmit time taken as 1).
+__device__ void satvel_one(double transmit_time, const sgx_eph& e, double vs[3], double& clk_drift) {
+  const double gps_pi = 3.14159265359, omegae_dot = 7.2921151467e-05, gm = 3.986005e+14, f_rel = -4.442807633e-10;
+  const double two_pi = 2 * gps_pi;
+  const double dt = check_t(transmit_time - e.t_oc);
+  double clk = (e.a_f2 * dt + e.a_f1) * dt + e.a_f0 - e.T_GD;
+  const double time = transmit_time - clk;
+  const double a = e.sqrtA * e.sqrtA;
+  const double tk = check_t(time - e.t_oe);
+  const double n = sqrt(gm / (a * a * a)) + e.deltan;
+  double m = e.M_0 + n * tk;
+  m = py_mod(m + two_pi, two_pi);
+  double ea = m;
+  for (int i = 0; i < 10; ++i) {
+    const double old = ea;
+    ea = m + e.e * sin(ea);
+    const double d = py_mod(ea - old, two_pi);
+    if (fabs(d) < 1e-12) break;
+  }
+  ea = py_mod(ea + two_pi, two_pi);
+  double se, ce;
+  sincos(ea, &se, &ce);
+  const double nu = atan2(sqrt(1 - e.e * e.e) * se, ce - e.e);
+  const double phi = py_mod(nu + e.omega, two_pi);
+  double s2, c2;
+  sincos(2 * phi, &s2, &c2);
+  const double u = phi + e.C_uc * c2 + e.C_us * s2;
+  const double r = a * (1 - e.e * ce) + e.C_rc * c2 + e.C_rs * s2;
+  const double inc = e.i_0 + e.iDot * tk + e.C_ic * c2 + e.C_is * s2;
+  double om = e.omega_0 + (e.omegaDot - omegae_dot) * tk - omegae_dot * e.t_oe;
+  om = py_mod(om + two_pi, two_pi);
+  const double one_m_ecose = 1 - e.e * ce;
+  const double ea_dot = n / one_m_ecose;
+  const double nu_dot = ea_dot * sqrt(1 - e.e * e.e) / one_m_ecose;
+  const double u_dot = nu_dot * (1 + 2 * (e.C_us * c2 - e.C_uc * s2));
+  const double r_dot = a * e.e * se * ea_dot + 2 * nu_dot * (e.C_rs * c2 - e.C_rc * s2);
+  const double i_dot = e.iDot + 2 * nu_dot * (e.C_is * c2 - e.C_ic * s2);
+  const double om_dot = e.omegaDot - omegae_dot;
+  double su, cu, so, co, si, ci;
+  sincos(u, &su, &cu);
+  sincos(om, &so, &co);
+  sincos(inc, &si, &ci);
+  const double xp = r * cu, yp = r * su;                       // position in the orbital plane
+  const double xp_dot = r_dot * cu - r * su * u_dot, yp_dot = r_dot * su + r * cu * u_dot;
+  vs[0] = xp_dot * co - xp * so * om_dot - yp_dot * ci * so + yp * si * i_dot * so - yp * ci * co * om_dot;
+  vs[1] = xp_dot * so + xp * co * om_dot + yp_dot * ci * co - yp * si * i_dot * co - yp * ci * so * om_dot;
+  vs[2] = yp_dot * si + yp * ci * i_dot;
+  clk_drift = e.a_f1 + 2 * e.a_f2 * dt + f_rel * e.e * e.sqrtA * ce * ea_dot;
+}
+
+// One warp per (recording, epoch), lane = channel.  Epochs are independent: K8's `active` already carries the
+// elevation feedback between them.
+__global__ void __launch_bounds__(128) nav_velocity_kernel(VelArgs a) {
+  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (warp >= (long long)a.n_rec * a.max_epochs) return;
+  const int rec = (int)(warp / a.max_epochs), ep = (int)(warp % a.max_epochs);
+  const int C = a.n_ch;
+  const bool mine = lane < C;
+  const long long o = warp * C + lane;                           // [R][E][C] index of (rec, ep, lane)
+  double* vel = a.vel + warp * SGX_NAV_VEL_FIELDS;
+  const int n_ep = min(a.n_epochs[rec], a.max_epochs);
+  if (ep >= n_ep) {
+    if (mine) {
+      a.doppler[o] = nan_f64(); a.rr_resid[o] = nan_f64();
+      if (a.sat_clk_drift) a.sat_clk_drift[o] = nan_f64();
+      if (a.sat_vel) { a.sat_vel[o * 3] = nan_f64(); a.sat_vel[o * 3 + 1] = nan_f64(); a.sat_vel[o * 3 + 2] = nan_f64(); }
+    }
+    if (lane < SGX_NAV_VEL_FIELDS) vel[lane] = lane == 7 ? 0.0 : nan_f64();
+    return;
+  }
+  const double* sol = a.sol + warp * SGX_NAV_SOL_FIELDS;
+  const double c_light = a.st.c, dtr_deg = 3.141592653589793 / 180;
+  double transmit_time = a.tow[rec];                             // advanced as nav_solve_kernel does, bit for bit
+  for (int k = 0; k < ep; ++k) transmit_time += a.st.nav_sol_period / 1000;
+  const bool act = mine && a.active[o] != 0;
+  // ---- Doppler: mean of the N carrFreq values ending at the epoch's code period, summed in index order ------------
+  double dop = nan_f64();
+  if (act) {
+    const long long rc = (long long)rec * C + lane;
+    const int idx = a.sub_frame_start[rc] + (int)a.st.nav_sol_period * ep;
+    const int first = idx - a.st.doppler_avg_ms + 1;
+    const int done = a.ms_done ? a.ms_done[rc] : a.ms;
+    if (first >= 0 && idx < done) {
+      const double* row = a.carr_freq + rc * a.stride;
+      double s = 0.0;
+      for (int k = first; k <= idx; ++k) s += row[k];
+      dop = s / a.st.doppler_avg_ms - a.st.IF;
+    }
+  }
+  // ---- satellite state --------------------------------------------------------------------------------------------
+  double xs[3] = {0.0, 0.0, 0.0}, vs[3] = {0.0, 0.0, 0.0}, clk = 0.0, clk_drift = 0.0;
+  if (act) {
+    const sgx_eph e = a.eph[(long long)rec * C + lane];
+    satpos_one(transmit_time, e, xs, clk);
+    satvel_one(transmit_time, e, vs, clk_drift);
+  }
+  const bool use = act && isfinite(dop);
+  const int n_used = __popc(__ballot_sync(0xffffffffu, use));
+  const double px = sol[0], py = sol[1], pz = sol[2];
+  const bool fix = !isnan(px) && !isnan(py) && !isnan(pz);
+  // ---- least squares on the 4x4 normal equations ------------------------------------------------------------------
+  double row[4] = {0.0, 0.0, 0.0, 0.0}, y = 0.0, x[4] = {0.0, 0.0, 0.0, 0.0};
+  bool ok = false;
+  if (fix && n_used >= 4) {
+    if (use) {
+      const double d0 = xs[0] - px, d1 = xs[1] - py, d2 = xs[2] - pz;
+      const double omegatau = 7.292115147e-05 * (sqrt(d0 * d0 + d1 * d1 + d2 * d2) / c_light);   // e_r_corr's constant
+      double so, co;
+      sincos(omegatau, &so, &co);
+      const double rx0 = co * xs[0] + so * xs[1], rx1 = -so * xs[0] + co * xs[1], rx2 = xs[2];
+      const double rv0 = co * vs[0] + so * vs[1], rv1 = -so * vs[0] + co * vs[1], rv2 = vs[2];
+      const double l0 = rx0 - px, l1 = rx1 - py, l2 = rx2 - pz;
+      const double rho = sqrt(l0 * l0 + l1 * l1 + l2 * l2);
+      const double u0 = l0 / rho, u1 = l1 / rho, u2 = l2 / rho;
+      const double rr = -(c_light / a.st.f_L1) * dop;
+      y = rr - (u0 * rv0 + u1 * rv1 + u2 * rv2) + c_light * clk_drift;
+      row[0] = -u0; row[1] = -u1; row[2] = -u2; row[3] = 1.0;
+    }
+    double nrm[10], rhs[4];
+    int k = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+#pragma unroll
+      for (int j = i; j < 4; ++j) nrm[k++] = warp_add(row[i] * row[j]);
+      rhs[i] = warp_add(row[i] * y);
+    }
+    ok = chol4(nrm, rhs, x, nullptr);
+  }
+  // ---- results ------------------------------------------------------------------------------------------------------
+  if (mine) {
+    a.doppler[o] = use ? dop : nan_f64();
+    a.rr_resid[o] = (ok && use) ? y - (row[0] * x[0] + row[1] * x[1] + row[2] * x[2] + row[3] * x[3]) : nan_f64();
+    if (a.sat_clk_drift) a.sat_clk_drift[o] = act ? clk_drift : nan_f64();
+    if (a.sat_vel) {
+      a.sat_vel[o * 3] = act ? vs[0] : nan_f64();
+      a.sat_vel[o * 3 + 1] = act ? vs[1] : nan_f64();
+      a.sat_vel[o * 3 + 2] = act ? vs[2] : nan_f64();
+    }
+  }
+  if (lane == 0) {
+    if (ok) {
+      double sl, cl, sb, cb;
+      sincos(sol[10] * dtr_deg, &sl, &cl);
+      sincos(sol[9] * dtr_deg, &sb, &cb);
+      vel[0] = x[0]; vel[1] = x[1]; vel[2] = x[2]; vel[3] = x[3];
+      vel[4] = -sl * x[0] + cl * x[1];
+      vel[5] = (-sb * cl) * x[0] + (-sb * sl) * x[1] + cb * x[2];
+      vel[6] = (cb * cl) * x[0] + (cb * sl) * x[1] + sb * x[2];
+    } else {
+      for (int i = 0; i < 7; ++i) vel[i] = nan_f64();
+    }
+    vel[7] = (double)n_used;
+  }
+}
+
 }  // namespace sgx
 
 using namespace sgx;
@@ -500,5 +682,73 @@ extern "C" int sgx_nav_solve(const double* abs_sample, int64_t stride, int32_t n
   if ((r = copy_back(active, a.active, rec, s))) return r;
   if ((r = copy_back(sol, a.sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, s))) return r;
   if (!is_device_ptr(sol)) SGX_CUDA(cudaStreamSynchronize(s));
+  return SGX_OK;
+}
+
+extern "C" int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t n_recordings, int32_t n_channels,
+                                int32_t ms, const int32_t* ms_done, const int32_t* sub_frame_start, const sgx_eph* eph,
+                                const double* tow, const int32_t* n_epochs, int32_t max_epochs, const uint8_t* active,
+                                const double* sol, const sgx_vel_settings* vs, double* vel, double* doppler,
+                                double* rr_resid, double* sat_vel, double* sat_clk_drift, void* cuda_stream) {
+  if (sgx_device_count() <= 0) return fail(SGX_ERR_NODEV, "sgx_nav_velocity", "no CUDA device");
+  SGX_API_GUARD();
+  if (!carr_freq || !sub_frame_start || !eph || !tow || !n_epochs || !active || !sol || !vs || !vel || !doppler ||
+      !rr_resid || n_channels < 1 || n_channels > 32 || ms <= 0 || stride < ms || n_recordings < 0 || max_epochs < 0)
+    return fail(SGX_ERR_ARG, "sgx_nav_velocity", "bad argument (NULL pointer, 1..32 channels, ms > 0, stride >= ms)");
+  if (vs->doppler_avg_ms < 1 || !(vs->nav_sol_period >= 1.0) || !isfinite(vs->nav_sol_period) || !isfinite(vs->c) ||
+      !(vs->c > 0) || !isfinite(vs->f_L1) || !(vs->f_L1 > 0) || !isfinite(vs->IF))
+    return fail(SGX_ERR_ARG, "sgx_nav_velocity",
+                "bad settings (doppler_avg_ms >= 1, nav_sol_period >= 1, c and f_L1 finite and > 0, IF finite)");
+  const size_t rc = (size_t)n_recordings * n_channels;
+  if (ms_done)
+    for (size_t i = 0; i < rc; ++i)
+      if (ms_done[i] < 0 || ms_done[i] > ms) return fail(SGX_ERR_ARG, "sgx_nav_velocity", "ms_done outside [0, ms]");
+  if (n_recordings == 0 || max_epochs == 0) return SGX_OK;
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  static DevBuf b_carr, b_done, b_sfs, b_eph, b_tow, b_nep, b_act, b_sol, b_vel, b_dop, b_res, b_svel, b_sclk;
+  const size_t rec = rc * max_epochs;
+  VelArgs a;
+  int r;
+  a.carr_freq = carr_freq;
+  a.stride = stride;
+  if (!is_device_ptr(carr_freq)) {                    // only the carrFreq rows travel, packed [R*C][ms]
+    const size_t row = sizeof(double) * (size_t)ms;
+    if (b_carr.reserve(row * rc)) return fail(SGX_ERR_CUDA, "cudaMalloc", "carrFreq rows");
+    SGX_CUDA(cudaMemcpy2DAsync(b_carr.p, row, carr_freq, sizeof(double) * (size_t)stride, row, rc,
+                               cudaMemcpyHostToDevice, s));
+    a.carr_freq = b_carr.as<double>();
+    a.stride = ms;
+  }
+  a.ms_done = nullptr;                                // NULL: every channel completed all ms periods
+  if (ms_done) {
+    if (b_done.reserve(sizeof(int) * rc)) return fail(SGX_ERR_CUDA, "cudaMalloc", "ms_done");
+    SGX_CUDA(cudaMemcpyAsync(b_done.p, ms_done, sizeof(int) * rc, cudaMemcpyHostToDevice, s));
+    a.ms_done = b_done.as<int>();
+  }
+  if ((r = stage_in(sub_frame_start, rc, b_sfs, a.sub_frame_start, s))) return r;
+  if ((r = stage_in(eph, rc, b_eph, a.eph, s))) return r;
+  if ((r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s))) return r;
+  if ((r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s))) return r;
+  if ((r = stage_in(active, rec, b_act, a.active, s))) return r;
+  if ((r = stage_in(sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, b_sol, a.sol, s))) return r;
+  const size_t n_vel = (size_t)n_recordings * max_epochs * SGX_NAV_VEL_FIELDS;
+  if ((r = stage_out(vel, n_vel, b_vel, a.vel))) return r;
+  if ((r = stage_out(doppler, rec, b_dop, a.doppler))) return r;
+  if ((r = stage_out(rr_resid, rec, b_res, a.rr_resid))) return r;
+  if ((r = stage_out(sat_vel, rec * 3, b_svel, a.sat_vel))) return r;
+  if ((r = stage_out(sat_clk_drift, rec, b_sclk, a.sat_clk_drift))) return r;
+  a.n_rec = n_recordings; a.n_ch = n_channels; a.ms = ms; a.max_epochs = max_epochs; a.st = *vs;
+  const int threads = 128;                            // 4 (recording, epoch) warps per CTA
+  const unsigned blocks = (unsigned)(((long long)n_recordings * max_epochs * 32 + threads - 1) / threads);
+  SGX_COUNTED_LAUNCH(nav_velocity_kernel, dim3(blocks), dim3(threads), 0, s, a);
+  SGX_CUDA(cudaGetLastError());
+  if ((r = copy_back(vel, a.vel, n_vel, s))) return r;
+  if ((r = copy_back(doppler, a.doppler, rec, s))) return r;
+  if ((r = copy_back(rr_resid, a.rr_resid, rec, s))) return r;
+  if ((r = copy_back(sat_vel, a.sat_vel, rec * 3, s))) return r;
+  if ((r = copy_back(sat_clk_drift, a.sat_clk_drift, rec, s))) return r;
+  const bool host_out = !is_device_ptr(vel) || !is_device_ptr(doppler) || !is_device_ptr(rr_resid) ||
+                        (sat_vel && !is_device_ptr(sat_vel)) || (sat_clk_drift && !is_device_ptr(sat_clk_drift));
+  if (host_out) SGX_CUDA(cudaStreamSynchronize(s));
   return SGX_OK;
 }

@@ -9,6 +9,10 @@ Mirrors, with the reference's names and conventions:
 * ``navBitsBin(trackResults, firstSubFrame, channelNr)`` -> list of ``'0'``/``'1'`` strings
   (postNavigation.py:125-139), ready for ``ephemeris.ephemeris(bits[1:], bits[0])``.
 
+Extension (no reference behaviour): receiver velocity and clock drift from the PLL's Doppler at the same epochs
+(``nav_velocity_batch``, ``post_navigate_batch(..., velocity=True)``, ``postNavigateVelocity``), computed by
+``sgx_nav_velocity`` (csrc/sgx_nav.cu).
+
 ``find_preambles_batch`` is the batched entry point over a float64 ``[channels, ms]`` array or CUDA tensor
 (e.g. field 3 of ``track_batch``'s device-resident output).  There is no CPU implementation here: the
 work is done by ``sgx_find_preambles`` (csrc/sgx_bitsync.cu) and the call fails without a CUDA device.
@@ -192,6 +196,50 @@ def nav_solve_batch(abs_sample, sub_frame_start, ready, eph, tow, settings, stri
                                    nav_settings(settings), want_sat=want_sat, stream=stream)
 
 
+def vel_settings(settings):
+    """``sgx_vel_settings`` from ``IF``, ``c``, ``navSolPeriod`` and the extension attributes ``L1Freq`` and
+    ``dopplerAvgMs``; an object without the latter (the reference's own Settings) gets 1575.42e6 Hz and 100."""
+    return _native.SgxVelSettings(IF=float(settings.IF), c=float(settings.c),
+                                  f_L1=float(getattr(settings, "L1Freq", 1575.42e6)),
+                                  nav_sol_period=float(settings.navSolPeriod),
+                                  doppler_avg_ms=int(getattr(settings, "dopplerAvgMs", 100)), reserved=0)
+
+
+def nav_velocity_batch(track_out, nav_out, sub_frame_start, eph, tow, settings, ms_done=None, want_sat=False, stream=0):
+    """Receiver velocity and clock drift at the epochs of ``nav_out`` from the Doppler the PLL tracked, computed by
+    ``sgx_nav_velocity`` (csrc/sgx_nav.cu; contract in include/softgnss_b200.h).
+
+    ``track_out``: ``track_batch``'s float64 ``[R, C, 13, ms]`` output, numpy array or contiguous CUDA tensor (carrFreq,
+    field 2, is read in place), or a ``[R, C, ms]`` carrFreq array.  ``nav_out``: the dict of :func:`nav_solve_batch` or
+    :func:`post_navigate_batch` (``active``, ``sol``, ``n_epochs`` are read).  ``sub_frame_start`` ``[R, C]``, ``eph``
+    ``[R, C, 21]`` and ``tow`` ``[R]``: what the fix was computed from.  ``ms_done`` ``[R, C]``: periods tracked
+    (``track_batch``'s third result), None for all.  Returns numpy ``vel`` ``[R, E, 8]`` (``_native.NAV_VEL_FIELDS``),
+    ``doppler`` and ``rrResid`` ``[R, E, C]``, and with ``want_sat`` ``satVel`` ``[R, E, C, 3]`` and ``satClkDrift``.
+    There is no host implementation: without a device this raises NativeError."""
+    L = _native.lib()
+    L.require_device()
+    shape = tuple(track_out.shape)
+    r, c, ms = shape[0], shape[1], shape[-1]
+    on_device = hasattr(track_out, "data_ptr")
+    if not on_device:
+        track_out = np.ascontiguousarray(track_out, dtype=np.float64)
+        base = track_out.ctypes.data
+    else:
+        import torch
+        assert track_out.is_cuda and track_out.dtype == torch.float64 and track_out.is_contiguous()
+        base = track_out.data_ptr()
+    if len(shape) == 4:
+        assert shape[2] == len(_native.TRACK_FIELDS), "track_out must be [R, C, 13, ms] or [R, C, ms]"
+        carr, stride = base + 8 * _native.TRACK_FIELDS.index("carrFreq") * ms, len(_native.TRACK_FIELDS) * ms
+    else:
+        carr, stride = base, ms
+    out = L.nav_velocity(carr, stride, r, c, ms, ms_done, sub_frame_start, eph, tow, nav_out["n_epochs"],
+                         nav_out["active"], nav_out["sol"], vel_settings(settings), want_sat=want_sat, stream=stream)
+    if not want_sat:
+        out.pop("satVel"), out.pop("satClkDrift")
+    return out
+
+
 def eph_rows(eph, prn):
     """Rows of ``_native.EPH_FIELDS`` for the channels' PRNs from the reference's ephemeris recarray
     (postNavigation.py:120-140: ``eph[PRN - 1].<field>``); channels without an ephemeris get zeros."""
@@ -213,6 +261,13 @@ def navSolutions(trackResults, subFrameStart, readyChnList, eph, TOW, settings):
     (postNavigation.py:176-197): returns (navSolutions, channel) -- ``navSolutions.X/Y/Z/dt/latitude/longitude/
     height`` of length E, ``.DOP`` ``[5, E]``; ``channel.PRN/el/az/rawP/correctedP`` ``[numberOfChannels, E]``.
     UTM fields (``E, N, U, utmZone``) are left to the reference's ``cart2utm``."""
+    nav, channel, _ = _nav_solutions(trackResults, subFrameStart, readyChnList, eph, TOW, settings)
+    return nav, channel
+
+
+def _nav_solutions(trackResults, subFrameStart, readyChnList, eph, TOW, settings):
+    """navSolutions plus the dict of nav_solve_batch and the inputs it was given (``subFrameStart``, ``ephRows``,
+    ``tow``)."""
     n_ch = settings.numberOfChannels
     ms = len(trackResults[0].absoluteSample)
     abs_sample = np.zeros((1, n_ch, ms))
@@ -222,8 +277,8 @@ def navSolutions(trackResults, subFrameStart, readyChnList, eph, TOW, settings):
         prn[c] = trackResults[c].PRN
     ready = np.zeros((1, n_ch), dtype=np.uint8)
     ready[0, np.asarray(readyChnList, dtype=int)] = 1
-    out = nav_solve_batch(abs_sample, np.asarray(subFrameStart)[None, :n_ch], ready, eph_rows(eph, prn)[None],
-                          [float(TOW)], settings)
+    rows = eph_rows(eph, prn)[None]
+    out = nav_solve_batch(abs_sample, np.asarray(subFrameStart)[None, :n_ch], ready, rows, [float(TOW)], settings)
     sol = out["sol"][0]
     channel = np.rec.array([(np.where(out["active"][0].T > 0, prn[:, None], 0).astype(np.float64), out["el"][0].T.copy(),
                              out["az"][0].T.copy(), out["rawP"][0].T.copy(), out["correctedP"][0].T.copy())],
@@ -231,7 +286,8 @@ def navSolutions(trackResults, subFrameStart, readyChnList, eph, TOW, settings):
     nav = np.rec.array([(channel, sol[:, 4:9].T.copy(), sol[:, 0].copy(), sol[:, 1].copy(), sol[:, 2].copy(),
                          sol[:, 3].copy(), sol[:, 9].copy(), sol[:, 10].copy(), sol[:, 11].copy())],
                        formats=['O'] * 9, names='channel,DOP,X,Y,Z,dt,latitude,longitude,height')
-    return nav, channel
+    out.update(subFrameStart=np.asarray(subFrameStart)[None, :n_ch], ephRows=rows, tow=np.array([float(TOW)]))
+    return nav, channel, out
 
 
 def _decode_channels(bits, valid, first, prn, candidates):
@@ -257,28 +313,60 @@ def postNavigate(trackResults, settings):
     (``sgx_nav_solve``).  Returns ``(navSolutions, eph)`` -- ``(None, None)`` with the reference's messages when
     the record is too short or fewer than four satellites have an ephemeris.  ``navSolutions`` is the recarray of
     :func:`navSolutions` (no UTM fields); ``eph`` a list of 32 dicts/None indexed by PRN-1."""
+    r = _post_navigate(trackResults, settings)
+    return (None, None) if r is None else (r[0], r[1])
+
+
+def _post_navigate(trackResults, settings):
+    """postNavigate's chain; (navSolutions, eph, nav_solve dict) or None with the reference's messages."""
     tracked = (trackResults.status != '-') if trackResults.status.dtype.kind != 'S' else (trackResults.status != b'-')
     if settings.msToProcess < 36000 or int(tracked.sum()) < 4:                                # :104-111
         print('Record is to short or too few satellites tracked. Exiting!')
-        return None, None
+        return None
     subFrameStart, activeChnList, bits, valid = findPreambles(trackResults, settings, return_bits=True)   # :115
     prn = [int(trackResults[c].PRN) for c in range(len(trackResults))]
     eph, TOW, ready = _decode_channels(bits, valid, subFrameStart, prn, activeChnList) if bits is not None \
         else ([None] * 32, None, np.zeros(0, dtype=int))
     if ready.size < 4:                                                                        # :149-156
         print('Too few satellites with ephemeris data for position calculations. Exiting!')
-        return None, None
-    nav, _ = navSolutions(trackResults, subFrameStart, ready, eph, TOW, settings)
-    return nav, eph
+        return None
+    nav, _, out = _nav_solutions(trackResults, subFrameStart, ready, eph, TOW, settings)
+    return nav, eph, out
 
 
-def post_navigate_batch(track_out, prn, settings, stream=0):
+def postNavigateVelocity(trackResults, settings):
+    """:func:`postNavigate` plus the receiver velocity and clock drift of every measurement epoch (extension; no
+    reference behaviour).  Returns ``(navSolutions, eph, navVelocities)``, ``(None, None, None)`` where postNavigate
+    returns ``(None, None)``.  ``navVelocities`` is a one-record recarray with the length-E fields ``VX VY VZ`` (ECEF,
+    m/s), ``clkDrift`` (m/s), ``VE VN VU`` (m/s, at the fix's latitude and longitude), ``nUsed`` (channels in the
+    solution) and ``doppler`` ``[numberOfChannels, E]`` (Hz, NaN for channels not used).  The Doppler of a channel is
+    the mean carrFreq of the ``settings.dopplerAvgMs`` code periods that end at the epoch, minus ``settings.IF``."""
+    r = _post_navigate(trackResults, settings)
+    if r is None:
+        return None, None, None
+    nav, eph, out = r
+    n_ch = settings.numberOfChannels
+    ms = len(trackResults[0].carrFreq)
+    carr = np.zeros((1, n_ch, ms))
+    for c in range(min(n_ch, len(trackResults))):
+        carr[0, c] = trackResults[c].carrFreq
+    v = nav_velocity_batch(carr, out, out["subFrameStart"], out["ephRows"], out["tow"], settings)
+    vel = v["vel"][0]
+    cols = [vel[:, k].copy() for k in range(len(_native.NAV_VEL_FIELDS))]
+    velocities = np.rec.array([tuple(cols) + (v["doppler"][0].T.copy(),)], formats=['O'] * 9,
+                              names=','.join(_native.NAV_VEL_FIELDS) + ',doppler')
+    return nav, eph, velocities
+
+
+def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_done=None):
     """The same chain for R recordings whose tracking result ``track_out`` (float64 ``[R, C, 13, ms]``, numpy or
     CUDA tensor as written by ``track_batch``) stays where it is: ``I_P`` and ``absoluteSample`` are read in
     place by the two device stages; only the 1501 hard bits per channel and the solutions cross to the host.
     ``prn``: int ``[R, C]`` (0 = channel not tracked).  Returns the dict of :func:`nav_solve_batch` plus
     ``subFrameStart`` ``[R, C]``, ``ready`` ``[R, C]``, ``tow`` ``[R]`` and ``eph`` (R lists indexed by PRN-1);
-    recordings with fewer than four usable satellites get ``n_epochs = 0``."""
+    recordings with fewer than four usable satellites get ``n_epochs = 0``.  With ``velocity=True`` the dict also
+    carries ``vel``, ``doppler`` and ``rrResid`` of :func:`nav_velocity_batch` (carrFreq read in place; ``ms_done``
+    ``[R, C]`` as returned by ``track_batch``, None for all ms)."""
     r, c, nf, ms = track_out.shape
     prn = np.asarray(prn).reshape(r, c)
     if isinstance(track_out, np.ndarray):
@@ -308,6 +396,8 @@ def post_navigate_batch(track_out, prn, settings, stream=0):
     out = _native.lib().nav_solve(abs_in, stride, r, c, ms, first, ready, rows, tow, n_ep, nav_settings(settings),
                                   stream=stream)
     out.update(subFrameStart=first, ready=ready, tow=tow, eph=ephs)
+    if velocity:
+        out.update(nav_velocity_batch(track_out, out, first, rows, tow, settings, ms_done=ms_done, stream=stream))
     return out
 
 

@@ -20,6 +20,8 @@ Tracking-quality extensions, read by ``tracking.cno_vsm`` / ``track_quality_batc
 object lacks them): ``CNoVSMinterval`` (40 code periods per C/N0 estimate, Matlab ``settings.CNo.VSMinterval``),
 ``CNoAccTime`` (0.001 s per prompt sample, ``settings.CNo.accTime``), ``lockCNoMin`` (30.0 dB-Hz) and ``lockPllMin``
 (0.5, cos 2 dphi): a window counts as locked when its C/N0 and its carrier-lock indicator reach both.
+Velocity extensions, read by ``postnav.nav_velocity_batch`` / ``postNavigateVelocity`` (same defaults for an object
+without them): ``dopplerAvgMs`` (100 code periods of carrFreq averaged per Doppler) and ``L1Freq`` (1575.42e6 Hz).
 """
 import ctypes
 
@@ -78,6 +80,7 @@ class Settings(object):
         # extensions (defaults == reference behaviour)
         acqDopplerStep=500.0, acqCoherentMs=1, acqNonCoherentBlocks=2,
         CNoVSMinterval=40, CNoAccTime=0.001, lockCNoMin=30.0, lockPllMin=0.5,
+        dopplerAvgMs=100, L1Freq=1575.42e6,
     )
 
     def __init__(self, **overrides):
