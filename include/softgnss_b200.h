@@ -11,6 +11,15 @@
  * owns all buffers.  Return value: 0 or a negative sgx_status; sgx_last_error() gives text.
  * There is no CPU fallback: without a CUDA device every compute call fails with
  * SGX_ERR_NODEV.
+ *
+ * Operands of the stages after tracking (sgx_find_preambles, sgx_pseudoranges, sgx_track_quality,
+ * sgx_nav_solve, sgx_nav_velocity):
+ *   - device operands are read and written in place, in the order of cuda_stream;
+ *   - host inputs are copied to device scratch first.  An input that holds one series of ms values per
+ *     channel, `stride` elements apart, is read in exactly those rows: nothing between or after them;
+ *   - host outputs are written from device scratch, and then the call synchronises the stream before it
+ *     returns.  A call whose outputs are all device memory (NULL optional outputs do not count) does not
+ *     synchronise: its results are complete in stream order.
  */
 #ifndef SOFTGNSS_B200_H
 #define SOFTGNSS_B200_H
@@ -164,15 +173,16 @@ int sgx_fft_c2c(const float* in, float* out, int32_t n, int32_t batch, int32_t i
 /* Replaces NavigationResult.findPreambles (postNavigation.py:524-631) and the 20 ms bit summation of
  * postNavigate (postNavigation.py:125-134) for n_channels tracked channels (the downstream consumer of
  * the tracking result; SURVEY.md section 8(f) row 3).
- *   i_p             double [n_channels][stride] prompt in-phase series (host or device; e.g. field 3 of
- *                   sgx_track's output with stride = SGX_TRACK_FIELDS * ms), ms values used per row
- *   first_subframe  int32 [n_channels] (host or device): ms index of the first preamble that has a
+ *   i_p             double [n_channels][stride] prompt in-phase series (e.g. field 3 of sgx_track's
+ *                   output with stride = SGX_TRACK_FIELDS * ms), ms values used per row
+ *   first_subframe  int32 [n_channels]: ms index of the first preamble that has a
  *                   preamble-like pattern 6000 ms later and whose TLM and HOW words pass the parity
  *                   check; 0 when there is none (the reference's convention)
  *   nav_bits        optional uint8 [n_channels][SGX_NAV_BITS]: hard bits 0/1 of
  *                   I_P[first-20 : first+30000] summed over 20 ms (bit 0 = last bit of the previous
  *                   subframe), what the caller hands to ephemeris()
- *   nav_bits_valid  optional int32 [n_channels]: 1 when that window lies inside the record
+ *   nav_bits_valid  optional int32 [n_channels]: 1 when that window lies inside the record; written only
+ *                   when nav_bits is given
  * Candidates nearer than 40 ms to the start of the record are passed over (the reference reads
  * I_P[k-40:...] with a negative start there and raises). */
 int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_channels, int32_t ms,
@@ -182,8 +192,8 @@ int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_channels, in
 /* Replaces NavigationResult.calculatePseudoranges (postNavigation.py:27-72), batched over recordings and
  * measurement epochs (SURVEY.md section 8(f) row 4, first half; satellite positions and the least-squares
  * fix stay with the reference's host code).
- *   track_out     double [n_recordings][n_channels][SGX_TRACK_FIELDS][ms] as written by sgx_track (host or
- *                 device); only field 0 (absoluteSample) is read
+ *   track_out     double [n_recordings][n_channels][SGX_TRACK_FIELDS][ms] as written by sgx_track; only
+ *                 field 0 (absoluteSample) is read
  *   ms_index      int32 [n_recordings][n_epochs][n_channels]: msOfTheSignal per channel
  *   active        uint8 [n_recordings][n_epochs][n_channels]: 1 = channel is in channelList (others get +inf
  *                 travel time, i.e. an infinite pseudorange, as in the reference)
@@ -218,10 +228,9 @@ typedef struct sgx_quality_settings {
  * NaN, 0 (idle channels of sgx_track have ms_done = 0).  Deterministic: fixed reduction order, no atomics.
  *   i_p, q_p  double [n_channels][stride], ms values used per row; both host or both device memory.  Reads
  *             sgx_track's output in place: i_p = out + 3*ms, q_p = out + 7*ms, stride = SGX_TRACK_FIELDS*ms,
- *             n_channels = n_recordings * channels.  Host rows are copied row by row (2 * n_channels rows of ms).
+ *             n_channels = n_recordings * channels.
  *   ms_done   host int32 [n_channels] periods completed per channel, each in [0, ms]; NULL: all ms
- *   cn0, pll_lock (double), locked (uint8)  [n_channels][n_win], all three host or all three device memory; host
- *             outputs synchronise the stream, device outputs leave the call asynchronous.
+ *   cn0, pll_lock (double), locked (uint8)  [n_channels][n_win], all three host or all three device memory.
  * SGX_ERR_ARG for window_ms < 2, acc_time not finite and > 0, stride < ms, ms_done outside [0, ms], a NULL pointer
  * or mixed host/device operands.  n_win == 0 succeeds without work. */
 int sgx_track_quality(const double* i_p, const double* q_p, int64_t stride, int32_t n_channels, int32_t ms,
@@ -254,15 +263,14 @@ typedef struct sgx_nav_settings {
  * the elevation mask of an epoch uses the elevations of the epoch before, :201/:241).  UTM conversion
  * (findUtmZone, cart2utm) and ephemeris decoding stay with the caller.
  *   abs_sample       double: the absoluteSample series of channel (r, c) starts at abs_sample + (r*n_channels + c)*stride
- *                    and holds ms values (sgx_track's output: pointer to its first element, stride = SGX_TRACK_FIELDS*ms;
- *                    host or device)
+ *                    and holds ms values (sgx_track's output: pointer to its first element, stride = SGX_TRACK_FIELDS*ms)
  *   sub_frame_start  int32 [R][C]   subFrameStart of findPreambles (0: none)
  *   ready            uint8 [R][C]   1 = channel is in readyChnList (preamble found and ephemeris decoded, :166)
  *   eph              sgx_eph [R][C] ephemeris of the channel's PRN (read for ready channels only)
  *   tow              double [R]     transmitTime of the first measurement (:168)
  *   n_epochs         int32 [R]      int(fix(msToProcess - max(subFrameStart)) / navSolPeriod) (:199); epochs beyond
  *                                   it keep the reference's initial values (NaN, DOP 0)
- * Outputs (host or device, same kind as `sol`), E = max_epochs:
+ * Outputs (the same kind as `sol`), E = max_epochs:
  *   raw_p, corrected_p, el, az  double [R][E][C]  channel[0].rawP / .correctedP / .el / .az (:212, :243, :227)
  *   sat_pos   double [R][E][C][3], sat_clk double [R][E][C]: satpos outputs per listed channel (optional, may be NULL)
  *   active    uint8 [R][E][C]   1 = channel was in activeChnList of that epoch (channel[0].PRN != 0)
@@ -306,12 +314,11 @@ typedef struct sgx_vel_settings {
  *   Cholesky for (vx, vy, vz, c * receiver clock drift).  The epoch is NaN when its fix is NaN, when fewer than 4
  *   channels are used, or when a Cholesky pivot is not above 1e-13 of the trace.
  *   carr_freq        double: the carrFreq series of channel (r, c) starts at carr_freq + (r*n_channels + c)*stride and
- *                    holds ms values (sgx_track's output + 2*ms, stride = SGX_TRACK_FIELDS*ms; host or device; host
- *                    rows are copied one row each)
+ *                    holds ms values (sgx_track's output + 2*ms, stride = SGX_TRACK_FIELDS*ms)
  *   ms_done          host int32 [R][C] periods completed, each in [0, ms]; NULL: all ms
  *   sub_frame_start, eph, tow, n_epochs, max_epochs  as given to sgx_nav_solve
- *   active           uint8 [R][E][C], sol double [R][E][SGX_NAV_SOL_FIELDS]: sgx_nav_solve's outputs (host or device)
- * Outputs (each host or device; a host output makes the call synchronous), E = max_epochs:
+ *   active           uint8 [R][E][C], sol double [R][E][SGX_NAV_SOL_FIELDS]: sgx_nav_solve's outputs
+ * Outputs, E = max_epochs:
  *   vel       double [R][E][SGX_NAV_VEL_FIELDS]: VX VY VZ, clock drift, VE VN VU (rotated at sol's latitude and
  *             longitude), channels used (the count of the rule above, also when the epoch is NaN)
  *   doppler   double [R][E][C] D in Hz of the channels used, NaN elsewhere

@@ -18,6 +18,22 @@ TRACK_FIELDS = ("absoluteSample", "codeFreq", "carrFreq", "I_P", "I_E", "I_L", "
                 "dllDiscr", "dllDiscrFilt", "pllDiscr", "pllDiscrFilt")
 SGX_ERR_SHORT = -3
 
+
+def track_field(track_out, field):
+    """Rows of one field of a ``[R, C, 13, ms]`` tracking result, for the entry points that take a channel's series as
+    (address, stride): a numpy array (made contiguous float64) or a contiguous float64 CUDA tensor.  Returns
+    ``(address, row stride in elements, object to keep alive while the address is in use)``."""
+    r, c, nf, ms = track_out.shape
+    assert nf == len(TRACK_FIELDS), "a tracking result is [R, C, %d, ms]" % len(TRACK_FIELDS)
+    if hasattr(track_out, "data_ptr"):
+        import torch
+        assert track_out.is_cuda and track_out.dtype == torch.float64 and track_out.is_contiguous()
+        base = track_out.data_ptr()
+    else:
+        track_out = np.ascontiguousarray(track_out, dtype=np.float64)
+        base = track_out.ctypes.data
+    return base + 8 * TRACK_FIELDS.index(field) * ms, nf * ms, track_out
+
 EXPORTS = ("sgx_abi_version", "sgx_last_error", "sgx_device_count", "sgx_set_device", "sgx_fp32_peak",
            "sgx_kernel_launch_count", "sgx_acquire", "sgx_track", "sgx_track_file", "sgx_synth_generate", "sgx_fft_c2c",
            "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality", "sgx_nav_velocity")
@@ -86,22 +102,27 @@ class Lib(object):
                                     "(needs nvcc; there is no CPU fallback)" % path)
         self.path = path
         self.dll = ctypes.CDLL(path)
-        vp, i32, i64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64
+        vp, i32, i64, f64 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, ctypes.c_double
         d = self.dll
         d.sgx_abi_version.restype = ctypes.c_int
         d.sgx_last_error.restype = ctypes.c_char_p
         d.sgx_device_count.restype = ctypes.c_int
         d.sgx_set_device.argtypes = [ctypes.c_int]
+        d.sgx_fp32_peak.argtypes = [vp, vp]
         d.sgx_kernel_launch_count.restype = i64
+        d.sgx_acquire.argtypes = [vp, i64, i64, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, i32, i32,
+                                  vp, vp, vp, vp, vp, vp]
         d.sgx_track.argtypes = [vp, i64, vp, i32, vp, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, vp]
         d.sgx_track_file.argtypes = [ctypes.c_char_p, i32, vp, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, i64, vp, vp]
         d.sgx_synth_generate.argtypes = [vp, i64, i64, i64, i32, vp, vp, vp, vp, vp]
-        if hasattr(d, "sgx_nav_velocity"):
-            d.sgx_nav_velocity.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
-                                           ctypes.POINTER(SgxVelSettings), vp, vp, vp, vp, vp, vp]
-        if hasattr(d, "sgx_acquire"):
-            d.sgx_acquire.argtypes = [vp, i64, i64, i32, ctypes.POINTER(SgxSettings), vp, vp, vp, i32, i32,
-                                      vp, vp, vp, vp, vp, vp]
+        d.sgx_fft_c2c.argtypes = [vp, vp, i32, i32, i32, vp]
+        d.sgx_find_preambles.argtypes = [vp, i64, i32, i32, vp, vp, vp, vp]
+        d.sgx_pseudoranges.argtypes = [vp, i32, i32, i32, vp, vp, i32, f64, f64, f64, vp, vp]
+        d.sgx_track_quality.argtypes = [vp, vp, i64, i32, i32, vp, ctypes.POINTER(SgxQualitySettings), vp, vp, vp, vp]
+        d.sgx_nav_solve.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, i32, ctypes.POINTER(SgxNavSettings),
+                                    vp, vp, vp, vp, vp, vp, vp, vp, vp]
+        d.sgx_nav_velocity.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
+                                       ctypes.POINTER(SgxVelSettings), vp, vp, vp, vp, vp, vp]
 
     def check(self, rc):
         if rc != 0:
@@ -153,8 +174,6 @@ class Lib(object):
         self.require_device()
         x = np.ascontiguousarray(np.atleast_2d(x), dtype=np.complex64)
         out = np.empty_like(x)
-        self.dll.sgx_fft_c2c.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32,
-                                         ctypes.c_int32, ctypes.c_void_p]
         self.check(self.dll.sgx_fft_c2c(_ptr(x), _ptr(out), x.shape[1], x.shape[0], int(bool(inverse)) | (2 if persistent else 0),
                                         ctypes.c_void_p(stream)))
         return out
@@ -167,8 +186,6 @@ class Lib(object):
         first = np.zeros(n_channels, dtype=np.int32)
         bits = np.zeros((n_channels, 1501), dtype=np.uint8) if want_bits else None
         valid = np.zeros(n_channels, dtype=np.int32) if want_bits else None
-        self.dll.sgx_find_preambles.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
-                                                ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
         self.check(self.dll.sgx_find_preambles(_ptr(i_p), int(stride), int(n_channels), int(ms), _ptr(first),
                                                _ptr(bits), _ptr(valid), ctypes.c_void_p(stream)))
         return first, bits, valid
@@ -181,9 +198,6 @@ class Lib(object):
         active = np.ascontiguousarray(active, dtype=np.uint8).reshape(n_rec, -1, n_ch)
         n_ep = ms_index.shape[1]
         out = np.empty((n_rec, n_ep, n_ch), dtype=np.float64)
-        self.dll.sgx_pseudoranges.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
-                                              ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_double,
-                                              ctypes.c_double, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]
         self.check(self.dll.sgx_pseudoranges(_ptr(track_out), n_rec, n_ch, int(ms), _ptr(ms_index), _ptr(active), n_ep,
                                              float(samples_per_code), float(start_offset), float(c), _ptr(out),
                                              ctypes.c_void_p(stream)))
@@ -197,9 +211,6 @@ class Lib(object):
         if ms_done is not None:
             ms_done = np.ascontiguousarray(ms_done, dtype=np.int32).reshape(-1)
             assert ms_done.size == n_channels
-        vp, i32 = ctypes.c_void_p, ctypes.c_int32
-        self.dll.sgx_track_quality.argtypes = [vp, vp, ctypes.c_int64, i32, i32, vp, ctypes.POINTER(SgxQualitySettings),
-                                               vp, vp, vp, vp]
         return self.dll.sgx_track_quality(_ptr(i_p), _ptr(q_p), int(stride), int(n_channels), int(ms), _ptr(ms_done),
                                           ctypes.byref(qs), _ptr(cn0), _ptr(pll_lock), _ptr(locked),
                                           ctypes.c_void_p(stream))
@@ -220,9 +231,6 @@ class Lib(object):
         out = dict(rawP=np.empty(shp), correctedP=np.empty(shp), el=np.empty(shp), az=np.empty(shp),
                    satPositions=np.empty(shp + (3,)) if want_sat else None, satClkCorr=np.empty(shp) if want_sat else None,
                    active=np.empty(shp, dtype=np.uint8), sol=np.empty((n_rec, e_max, len(NAV_SOL_FIELDS))))
-        vp, i32 = ctypes.c_void_p, ctypes.c_int32
-        self.dll.sgx_nav_solve.argtypes = [vp, ctypes.c_int64, i32, i32, i32, vp, vp, vp, vp, vp, i32,
-                                           ctypes.POINTER(SgxNavSettings), vp, vp, vp, vp, vp, vp, vp, vp, vp]
         self.check(self.dll.sgx_nav_solve(_ptr(abs_sample), int(stride), n_rec, n_ch, int(ms), _ptr(sub_frame_start),
                                           _ptr(ready), _ptr(eph), _ptr(tow), _ptr(n_epochs), e_max,
                                           ctypes.byref(nav_settings), _ptr(out["rawP"]), _ptr(out["correctedP"]),

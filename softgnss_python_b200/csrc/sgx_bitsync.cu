@@ -221,48 +221,33 @@ extern "C" int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_c
   if (!i_p || !first_subframe || n_channels < 0 || ms <= 0 || stride < ms)
     return fail(SGX_ERR_ARG, "sgx_find_preambles", "bad argument");
   if (n_channels == 0) return SGX_OK;
-  cudaStream_t s = (cudaStream_t)cuda_stream;
-  const double* d_ip = i_p;
-  if (!is_device_ptr(i_p)) {
-    const size_t bytes = sizeof(double) * (size_t)stride * n_channels;
-    if (g_bs.ip.reserve(bytes)) return fail(SGX_ERR_CUDA, "cudaMalloc", "I_P");
-    SGX_CUDA(cudaMemcpyAsync(g_bs.ip.p, i_p, bytes, cudaMemcpyHostToDevice, s));
-    d_ip = g_bs.ip.as<double>();
-  }
-  const bool first_dev = is_device_ptr(first_subframe);
-  const bool bits_dev = nav_bits && is_device_ptr(nav_bits);
-  const bool valid_dev = nav_bits_valid && is_device_ptr(nav_bits_valid);
-  if (g_bs.first.reserve(sizeof(int) * n_channels) || g_bs.valid.reserve(sizeof(int) * n_channels) ||
-      (nav_bits && g_bs.bits.reserve((size_t)NAV_BITS * n_channels)))
-    return fail(SGX_ERR_CUDA, "cudaMalloc", "bitsync outputs");
   BitsyncArgs a;
-  a.ip = d_ip;
-  a.stride = stride;
   a.ms = ms;
   a.n_words = (ms + 31) / 32;
-  a.first = first_dev ? first_subframe : g_bs.first.as<int>();
-  a.bits = nav_bits ? (bits_dev ? nav_bits : g_bs.bits.as<unsigned char>()) : nullptr;
-  a.bits_valid = nav_bits ? (valid_dev ? nav_bits_valid : g_bs.valid.as<int>()) : nullptr;
   const size_t smem = sizeof(unsigned) * (2 * (size_t)a.n_words + 8);
   if (smem > 200 * 1024) return fail(SGX_ERR_RANGE, "sgx_find_preambles", "record longer than 800 000 ms");
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const size_t n = (size_t)n_channels;
+  int32_t* valid = nav_bits ? nav_bits_valid : nullptr;   // written only together with nav_bits
+  StagedOutputs out;
+  int r;
+  if ((r = stage_rows_in(i_p, stride, ms, n, g_bs.ip, a.ip, a.stride, s)) ||
+      (r = out.add(first_subframe, n, g_bs.first, a.first)) ||
+      (r = out.add(nav_bits, (size_t)NAV_BITS * n, g_bs.bits, a.bits)) ||
+      (r = out.add(valid, n, g_bs.valid, a.bits_valid)))
+    return r;
   if (smem > 48 * 1024)
     SGX_CUDA(cudaFuncSetAttribute(bitsync_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   SGX_COUNTED_LAUNCH(bitsync_kernel, dim3(n_channels), dim3(BS_THREADS), smem, s, a);
   SGX_CUDA(cudaGetLastError());
-  if (!first_dev)
-    SGX_CUDA(cudaMemcpyAsync(first_subframe, a.first, sizeof(int) * n_channels, cudaMemcpyDeviceToHost, s));
-  if (nav_bits && !bits_dev)
-    SGX_CUDA(cudaMemcpyAsync(nav_bits, a.bits, (size_t)NAV_BITS * n_channels, cudaMemcpyDeviceToHost, s));
-  if (nav_bits_valid && !valid_dev)
-    SGX_CUDA(cudaMemcpyAsync(nav_bits_valid, a.bits_valid, sizeof(int) * n_channels, cudaMemcpyDeviceToHost, s));
-  if (!first_dev || (nav_bits && !bits_dev) || (nav_bits_valid && !valid_dev)) SGX_CUDA(cudaStreamSynchronize(s));
-  return SGX_OK;
+  return out.finish(s);
 }
 
 // ---- relative pseudoranges (postNavigation.py:27-72), batched over recordings x measurement epochs ---------
 namespace sgx {
 struct PseudoArgs {
-  const double* trk;      // [n_rec][n_ch][SGX_TRACK_FIELDS][ms]; field 0 = absoluteSample
+  const double* abs_sample;   // row (r, c) = abs_sample + (r*n_ch + c)*stride, ms values
+  long long stride;
   const int* ms_index;    // [n_rec][n_epochs][n_ch]
   const unsigned char* active;   // [n_rec][n_epochs][n_ch]
   double* pr;             // [n_rec][n_epochs][n_ch]
@@ -280,7 +265,7 @@ __global__ void pseudorange_kernel(PseudoArgs a) {
   if (lane < a.n_ch && a.active[o]) {
     const int i = a.ms_index[o];
     if (i >= 0 && i < a.ms)
-      t = a.trk[(((long long)r * a.n_ch + lane) * SGX_TRACK_FIELDS) * a.ms + i] / a.samples_per_code;   // :60
+      t = a.abs_sample[((long long)r * a.n_ch + lane) * a.stride + i] / a.samples_per_code;   // :60
   }
   double m = t;
 #pragma unroll
@@ -301,43 +286,21 @@ extern "C" int sgx_pseudoranges(const double* track_out, int32_t n_recordings, i
   const long long units = (long long)n_recordings * n_epochs;
   if (units == 0) return SGX_OK;
   cudaStream_t s = (cudaStream_t)cuda_stream;
-  static DevBuf d_trk, d_idx, d_act, d_pr;
+  static DevBuf d_abs, d_idx, d_act, d_pr;
   const size_t n = (size_t)units * n_channels;
   PseudoArgs a;
-  a.trk = track_out;
-  if (!is_device_ptr(track_out)) {
-    const size_t bytes = sizeof(double) * (size_t)n_recordings * n_channels * SGX_TRACK_FIELDS * ms;
-    if (d_trk.reserve(bytes)) return fail(SGX_ERR_CUDA, "cudaMalloc", "tracking result");
-    SGX_CUDA(cudaMemcpyAsync(d_trk.p, track_out, bytes, cudaMemcpyHostToDevice, s));
-    a.trk = d_trk.as<double>();
-  }
-  a.ms_index = ms_index;
-  if (!is_device_ptr(ms_index)) {
-    if (d_idx.reserve(sizeof(int) * n)) return fail(SGX_ERR_CUDA, "cudaMalloc", "ms_index");
-    SGX_CUDA(cudaMemcpyAsync(d_idx.p, ms_index, sizeof(int) * n, cudaMemcpyHostToDevice, s));
-    a.ms_index = d_idx.as<int>();
-  }
-  a.active = active;
-  if (!is_device_ptr(active)) {
-    if (d_act.reserve(n)) return fail(SGX_ERR_CUDA, "cudaMalloc", "active");
-    SGX_CUDA(cudaMemcpyAsync(d_act.p, active, n, cudaMemcpyHostToDevice, s));
-    a.active = d_act.as<unsigned char>();
-  }
-  const bool out_dev = is_device_ptr(pseudoranges);
-  a.pr = pseudoranges;
-  if (!out_dev) {
-    if (d_pr.reserve(sizeof(double) * n)) return fail(SGX_ERR_CUDA, "cudaMalloc", "pseudoranges");
-    a.pr = d_pr.as<double>();
-  }
+  StagedOutputs out;
+  int r;
+  if ((r = stage_rows_in(track_out, (int64_t)SGX_TRACK_FIELDS * ms, ms, (size_t)n_recordings * n_channels, d_abs,
+                         a.abs_sample, a.stride, s)) ||
+      (r = stage_in(ms_index, n, d_idx, a.ms_index, s)) || (r = stage_in(active, n, d_act, a.active, s)) ||
+      (r = out.add(pseudoranges, n, d_pr, a.pr)))
+    return r;
   a.n_rec = n_recordings; a.n_ch = n_channels; a.n_epochs = n_epochs; a.ms = ms;
   a.samples_per_code = samples_per_code; a.start_offset = start_offset; a.c = c;
   const int threads = 256;
   const long long blocks = (units * 32 + threads - 1) / threads;
   SGX_COUNTED_LAUNCH(pseudorange_kernel, dim3((unsigned)blocks), dim3(threads), 0, s, a);
   SGX_CUDA(cudaGetLastError());
-  if (!out_dev) {
-    SGX_CUDA(cudaMemcpyAsync(pseudoranges, a.pr, sizeof(double) * n, cudaMemcpyDeviceToHost, s));
-    SGX_CUDA(cudaStreamSynchronize(s));
-  }
-  return SGX_OK;
+  return out.finish(s);
 }

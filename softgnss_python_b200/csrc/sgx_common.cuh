@@ -95,6 +95,62 @@ struct DevBuf {
   template <class T> T* as() { return (T*)p; }
 };
 
+// ---- caller operands of the C-ABI entry points: host or device memory (include/softgnss_b200.h) --------------------
+// Device view of `count` elements at p: device memory (and NULL) as it is, host memory copied into buf.
+template <class T>
+int stage_in(const T* p, size_t count, DevBuf& buf, const T*& dev, cudaStream_t s) {
+  dev = p;
+  if (!p || is_device_ptr(p)) return SGX_OK;
+  if (buf.reserve(sizeof(T) * count)) return fail(SGX_ERR_CUDA, "cudaMalloc", "input staging buffer");
+  SGX_CUDA(cudaMemcpyAsync(buf.p, p, sizeof(T) * count, cudaMemcpyHostToDevice, s));
+  dev = buf.as<T>();
+  return SGX_OK;
+}
+
+// Device view of `rows` series of ms elements that start `stride` elements apart.  Device rows are read in place
+// (dev_stride = stride); host rows are packed into buf by one 2-D copy that reads those rows and nothing between or
+// after them (dev_stride = ms).
+template <class T>
+int stage_rows_in(const T* p, int64_t stride, int32_t ms, size_t rows, DevBuf& buf, const T*& dev,
+                  long long& dev_stride, cudaStream_t s) {
+  dev = p;
+  dev_stride = stride;
+  if (is_device_ptr(p)) return SGX_OK;
+  const size_t row = sizeof(T) * (size_t)ms;
+  if (buf.reserve(row * rows)) return fail(SGX_ERR_CUDA, "cudaMalloc", "input staging buffer");
+  SGX_CUDA(cudaMemcpy2DAsync(buf.p, row, p, sizeof(T) * (size_t)stride, row, rows, cudaMemcpyHostToDevice, s));
+  dev = buf.as<T>();
+  dev_stride = ms;
+  return SGX_OK;
+}
+
+// The outputs of one call.  add() gives the kernel a device view of an output: host memory is mapped to scratch,
+// device memory and NULL stay as they are.  finish(), after the launch, copies the scratch back and synchronises the
+// stream iff an output was staged, so a call whose outputs are all device memory stays asynchronous.
+class StagedOutputs {
+  struct Copy { void* host; const void* dev; size_t bytes; };
+  Copy copies_[8];
+  int n_ = 0;
+
+ public:
+  template <class T>
+  int add(T* p, size_t count, DevBuf& buf, T*& dev) {
+    dev = p;
+    if (!p || is_device_ptr(p)) return SGX_OK;
+    if (n_ == 8) return fail(SGX_ERR_ARG, "StagedOutputs", "more than 8 host outputs");
+    if (buf.reserve(sizeof(T) * count)) return fail(SGX_ERR_CUDA, "cudaMalloc", "output staging buffer");
+    dev = buf.as<T>();
+    copies_[n_++] = {p, dev, sizeof(T) * count};
+    return SGX_OK;
+  }
+  int finish(cudaStream_t s) {
+    for (int i = 0; i < n_; ++i)
+      SGX_CUDA(cudaMemcpyAsync(copies_[i].host, copies_[i].dev, copies_[i].bytes, cudaMemcpyDeviceToHost, s));
+    if (n_) SGX_CUDA(cudaStreamSynchronize(s));
+    return SGX_OK;
+  }
+};
+
 // ---- Ampere-style 16-byte async copy global -> shared (LDGSTS) ------------------------------
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
 #ifdef SGX_EMUL

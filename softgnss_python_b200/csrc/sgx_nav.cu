@@ -610,33 +610,6 @@ __global__ void __launch_bounds__(128) nav_velocity_kernel(VelArgs a) {
 
 using namespace sgx;
 
-namespace {
-// device view of a host or device input
-template <class T>
-int stage_in(const T* p, size_t count, DevBuf& buf, const T*& out, cudaStream_t s) {
-  out = p;
-  if (is_device_ptr(p)) return SGX_OK;
-  if (buf.reserve(sizeof(T) * count)) return fail(SGX_ERR_CUDA, "cudaMalloc", "nav input");
-  SGX_CUDA(cudaMemcpyAsync(buf.p, p, sizeof(T) * count, cudaMemcpyHostToDevice, s));
-  out = buf.as<T>();
-  return SGX_OK;
-}
-template <class T>
-int stage_out(T* p, size_t count, DevBuf& buf, T*& out) {
-  out = p;
-  if (!p || is_device_ptr(p)) return SGX_OK;
-  if (buf.reserve(sizeof(T) * count)) return fail(SGX_ERR_CUDA, "cudaMalloc", "nav output");
-  out = buf.as<T>();
-  return SGX_OK;
-}
-template <class T>
-int copy_back(T* host, const T* dev, size_t count, cudaStream_t s) {
-  if (!host || host == dev) return SGX_OK;
-  SGX_CUDA(cudaMemcpyAsync(host, dev, sizeof(T) * count, cudaMemcpyDeviceToHost, s));
-  return SGX_OK;
-}
-}  // namespace
-
 extern "C" int sgx_nav_solve(const double* abs_sample, int64_t stride, int32_t n_recordings, int32_t n_channels,
                              int32_t ms, const int32_t* sub_frame_start, const uint8_t* ready, const sgx_eph* eph,
                              const double* tow, const int32_t* n_epochs, int32_t max_epochs,
@@ -653,36 +626,25 @@ extern "C" int sgx_nav_solve(const double* abs_sample, int64_t stride, int32_t n
   static DevBuf b_abs, b_sfs, b_ready, b_eph, b_tow, b_nep, b_raw, b_cor, b_el, b_az, b_pos, b_clk, b_act, b_sol;
   const size_t rc = (size_t)n_recordings * n_channels, rec = (size_t)n_recordings * max_epochs * n_channels;
   NavArgs a;
+  StagedOutputs out;
   int r;
-  if ((r = stage_in(abs_sample, (rc - 1) * (size_t)stride + ms, b_abs, a.abs_sample, s))) return r;
-  if ((r = stage_in(sub_frame_start, rc, b_sfs, a.sub_frame_start, s))) return r;
-  if ((r = stage_in(ready, rc, b_ready, a.ready, s))) return r;
-  if ((r = stage_in(eph, rc, b_eph, a.eph, s))) return r;
-  if ((r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s))) return r;
-  if ((r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s))) return r;
-  if ((r = stage_out(raw_p, rec, b_raw, a.raw_p))) return r;
-  if ((r = stage_out(corrected_p, rec, b_cor, a.corrected_p))) return r;
-  if ((r = stage_out(el, rec, b_el, a.el))) return r;
-  if ((r = stage_out(az, rec, b_az, a.az))) return r;
-  if ((r = stage_out(sat_pos, rec * 3, b_pos, a.sat_pos))) return r;
-  if ((r = stage_out(sat_clk, rec, b_clk, a.sat_clk))) return r;
-  if ((r = stage_out(active, rec, b_act, a.active))) return r;
-  if ((r = stage_out(sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, b_sol, a.sol))) return r;
-  a.stride = stride; a.n_rec = n_recordings; a.n_ch = n_channels; a.ms = ms; a.max_epochs = max_epochs; a.st = *st;
+  if ((r = stage_rows_in(abs_sample, stride, ms, rc, b_abs, a.abs_sample, a.stride, s)) ||
+      (r = stage_in(sub_frame_start, rc, b_sfs, a.sub_frame_start, s)) || (r = stage_in(ready, rc, b_ready, a.ready, s)) ||
+      (r = stage_in(eph, rc, b_eph, a.eph, s)) || (r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s)) ||
+      (r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s)))
+    return r;
+  if ((r = out.add(raw_p, rec, b_raw, a.raw_p)) || (r = out.add(corrected_p, rec, b_cor, a.corrected_p)) ||
+      (r = out.add(el, rec, b_el, a.el)) || (r = out.add(az, rec, b_az, a.az)) ||
+      (r = out.add(sat_pos, rec * 3, b_pos, a.sat_pos)) || (r = out.add(sat_clk, rec, b_clk, a.sat_clk)) ||
+      (r = out.add(active, rec, b_act, a.active)) ||
+      (r = out.add(sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, b_sol, a.sol)))
+    return r;
+  a.n_rec = n_recordings; a.n_ch = n_channels; a.ms = ms; a.max_epochs = max_epochs; a.st = *st;
   const int threads = 128;                            // 4 recordings per CTA
   const unsigned blocks = (unsigned)(((long long)n_recordings * 32 + threads - 1) / threads);
   SGX_COUNTED_LAUNCH(nav_solve_kernel, dim3(blocks), dim3(threads), 0, s, a);
   SGX_CUDA(cudaGetLastError());
-  if ((r = copy_back(raw_p, a.raw_p, rec, s))) return r;
-  if ((r = copy_back(corrected_p, a.corrected_p, rec, s))) return r;
-  if ((r = copy_back(el, a.el, rec, s))) return r;
-  if ((r = copy_back(az, a.az, rec, s))) return r;
-  if ((r = copy_back(sat_pos, a.sat_pos, rec * 3, s))) return r;
-  if ((r = copy_back(sat_clk, a.sat_clk, rec, s))) return r;
-  if ((r = copy_back(active, a.active, rec, s))) return r;
-  if ((r = copy_back(sol, a.sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, s))) return r;
-  if (!is_device_ptr(sol)) SGX_CUDA(cudaStreamSynchronize(s));
-  return SGX_OK;
+  return out.finish(s);
 }
 
 extern "C" int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t n_recordings, int32_t n_channels,
@@ -706,49 +668,25 @@ extern "C" int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t
   if (n_recordings == 0 || max_epochs == 0) return SGX_OK;
   cudaStream_t s = (cudaStream_t)cuda_stream;
   static DevBuf b_carr, b_done, b_sfs, b_eph, b_tow, b_nep, b_act, b_sol, b_vel, b_dop, b_res, b_svel, b_sclk;
-  const size_t rec = rc * max_epochs;
+  const size_t rec = rc * max_epochs, n_sol = (size_t)n_recordings * max_epochs;
   VelArgs a;
+  StagedOutputs out;
   int r;
-  a.carr_freq = carr_freq;
-  a.stride = stride;
-  if (!is_device_ptr(carr_freq)) {                    // only the carrFreq rows travel, packed [R*C][ms]
-    const size_t row = sizeof(double) * (size_t)ms;
-    if (b_carr.reserve(row * rc)) return fail(SGX_ERR_CUDA, "cudaMalloc", "carrFreq rows");
-    SGX_CUDA(cudaMemcpy2DAsync(b_carr.p, row, carr_freq, sizeof(double) * (size_t)stride, row, rc,
-                               cudaMemcpyHostToDevice, s));
-    a.carr_freq = b_carr.as<double>();
-    a.stride = ms;
-  }
-  a.ms_done = nullptr;                                // NULL: every channel completed all ms periods
-  if (ms_done) {
-    if (b_done.reserve(sizeof(int) * rc)) return fail(SGX_ERR_CUDA, "cudaMalloc", "ms_done");
-    SGX_CUDA(cudaMemcpyAsync(b_done.p, ms_done, sizeof(int) * rc, cudaMemcpyHostToDevice, s));
-    a.ms_done = b_done.as<int>();
-  }
-  if ((r = stage_in(sub_frame_start, rc, b_sfs, a.sub_frame_start, s))) return r;
-  if ((r = stage_in(eph, rc, b_eph, a.eph, s))) return r;
-  if ((r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s))) return r;
-  if ((r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s))) return r;
-  if ((r = stage_in(active, rec, b_act, a.active, s))) return r;
-  if ((r = stage_in(sol, (size_t)n_recordings * max_epochs * SGX_NAV_SOL_FIELDS, b_sol, a.sol, s))) return r;
-  const size_t n_vel = (size_t)n_recordings * max_epochs * SGX_NAV_VEL_FIELDS;
-  if ((r = stage_out(vel, n_vel, b_vel, a.vel))) return r;
-  if ((r = stage_out(doppler, rec, b_dop, a.doppler))) return r;
-  if ((r = stage_out(rr_resid, rec, b_res, a.rr_resid))) return r;
-  if ((r = stage_out(sat_vel, rec * 3, b_svel, a.sat_vel))) return r;
-  if ((r = stage_out(sat_clk_drift, rec, b_sclk, a.sat_clk_drift))) return r;
+  if ((r = stage_rows_in(carr_freq, stride, ms, rc, b_carr, a.carr_freq, a.stride, s)) ||
+      (r = stage_in(ms_done, rc, b_done, a.ms_done, s)) ||          // NULL: every channel completed all ms periods
+      (r = stage_in(sub_frame_start, rc, b_sfs, a.sub_frame_start, s)) || (r = stage_in(eph, rc, b_eph, a.eph, s)) ||
+      (r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s)) ||
+      (r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s)) ||
+      (r = stage_in(active, rec, b_act, a.active, s)) || (r = stage_in(sol, n_sol * SGX_NAV_SOL_FIELDS, b_sol, a.sol, s)))
+    return r;
+  if ((r = out.add(vel, n_sol * SGX_NAV_VEL_FIELDS, b_vel, a.vel)) || (r = out.add(doppler, rec, b_dop, a.doppler)) ||
+      (r = out.add(rr_resid, rec, b_res, a.rr_resid)) || (r = out.add(sat_vel, rec * 3, b_svel, a.sat_vel)) ||
+      (r = out.add(sat_clk_drift, rec, b_sclk, a.sat_clk_drift)))
+    return r;
   a.n_rec = n_recordings; a.n_ch = n_channels; a.ms = ms; a.max_epochs = max_epochs; a.st = *vs;
   const int threads = 128;                            // 4 (recording, epoch) warps per CTA
   const unsigned blocks = (unsigned)(((long long)n_recordings * max_epochs * 32 + threads - 1) / threads);
   SGX_COUNTED_LAUNCH(nav_velocity_kernel, dim3(blocks), dim3(threads), 0, s, a);
   SGX_CUDA(cudaGetLastError());
-  if ((r = copy_back(vel, a.vel, n_vel, s))) return r;
-  if ((r = copy_back(doppler, a.doppler, rec, s))) return r;
-  if ((r = copy_back(rr_resid, a.rr_resid, rec, s))) return r;
-  if ((r = copy_back(sat_vel, a.sat_vel, rec * 3, s))) return r;
-  if ((r = copy_back(sat_clk_drift, a.sat_clk_drift, rec, s))) return r;
-  const bool host_out = !is_device_ptr(vel) || !is_device_ptr(doppler) || !is_device_ptr(rr_resid) ||
-                        (sat_vel && !is_device_ptr(sat_vel)) || (sat_clk_drift && !is_device_ptr(sat_clk_drift));
-  if (host_out) SGX_CUDA(cudaStreamSynchronize(s));
-  return SGX_OK;
+  return out.finish(s);
 }

@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(Q_THREADS) quality_kernel(QualityArgs a) {
 }
 
 struct QualityScratch {
-  DevBuf rows, done, cn0, pll, locked;
+  DevBuf ip, qp, done, cn0, pll, locked;
 };
 static QualityScratch g_q;
 
@@ -134,39 +134,17 @@ extern "C" int sgx_track_quality(const double* i_p, const double* q_p, int64_t s
   const long long n_units = (long long)n_channels * n_win;
   if (n_units == 0) return SGX_OK;
   cudaStream_t s = (cudaStream_t)cuda_stream;
+  const size_t n = (size_t)n_channels;
   QualityArgs a;
-  a.ip = i_p;
-  a.qp = q_p;
-  a.stride = stride;
-  if (!in_dev) {
-    // only the 2 * n_channels rows (ms values each) travel, packed: [I_P rows][Q_P rows]
-    const size_t row = sizeof(double) * (size_t)ms, n = (size_t)n_channels;
-    if (g_q.rows.reserve(2 * n * row)) return fail(SGX_ERR_CUDA, "cudaMalloc", "I_P / Q_P rows");
-    double* d = g_q.rows.as<double>();
-    SGX_CUDA(cudaMemcpy2DAsync(d, row, i_p, sizeof(double) * (size_t)stride, row, n, cudaMemcpyHostToDevice, s));
-    SGX_CUDA(cudaMemcpy2DAsync(d + n * ms, row, q_p, sizeof(double) * (size_t)stride, row, n, cudaMemcpyHostToDevice,
-                               s));
-    a.ip = d;
-    a.qp = d + n * ms;
-    a.stride = ms;
-  }
-  a.ms_done = nullptr;
-  if (ms_done) {
-    if (g_q.done.reserve(sizeof(int) * (size_t)n_channels)) return fail(SGX_ERR_CUDA, "cudaMalloc", "ms_done");
-    SGX_CUDA(cudaMemcpyAsync(g_q.done.p, ms_done, sizeof(int) * (size_t)n_channels, cudaMemcpyHostToDevice, s));
-    a.ms_done = g_q.done.as<int>();
-  }
-  a.cn0 = cn0;
-  a.pll = pll_lock;
-  a.locked = locked;
-  if (!out_dev) {
-    if (g_q.cn0.reserve(sizeof(double) * n_units) || g_q.pll.reserve(sizeof(double) * n_units) ||
-        g_q.locked.reserve((size_t)n_units))
-      return fail(SGX_ERR_CUDA, "cudaMalloc", "quality outputs");
-    a.cn0 = g_q.cn0.as<double>();
-    a.pll = g_q.pll.as<double>();
-    a.locked = g_q.locked.as<unsigned char>();
-  }
+  StagedOutputs out;
+  long long q_stride;                       // equals a.stride: i_p and q_p are of one kind (checked above)
+  int r;
+  if ((r = stage_rows_in(i_p, stride, ms, n, g_q.ip, a.ip, a.stride, s)) ||
+      (r = stage_rows_in(q_p, stride, ms, n, g_q.qp, a.qp, q_stride, s)) ||
+      (r = stage_in(ms_done, n, g_q.done, a.ms_done, s)) ||      // NULL: all ms
+      (r = out.add(cn0, (size_t)n_units, g_q.cn0, a.cn0)) || (r = out.add(pll_lock, (size_t)n_units, g_q.pll, a.pll)) ||
+      (r = out.add(locked, (size_t)n_units, g_q.locked, a.locked)))
+    return r;
   a.n_units = n_units;
   a.n_win = n_win;
   a.W = qs->window_ms;
@@ -177,11 +155,5 @@ extern "C" int sgx_track_quality(const double* i_p, const double* q_p, int64_t s
   const long long blocks = (n_units * 32 + Q_THREADS - 1) / Q_THREADS;
   SGX_COUNTED_LAUNCH(quality_kernel, dim3((unsigned)blocks), dim3(Q_THREADS), 0, s, a);
   SGX_CUDA(cudaGetLastError());
-  if (!out_dev) {
-    SGX_CUDA(cudaMemcpyAsync(cn0, a.cn0, sizeof(double) * n_units, cudaMemcpyDeviceToHost, s));
-    SGX_CUDA(cudaMemcpyAsync(pll_lock, a.pll, sizeof(double) * n_units, cudaMemcpyDeviceToHost, s));
-    SGX_CUDA(cudaMemcpyAsync(locked, a.locked, (size_t)n_units, cudaMemcpyDeviceToHost, s));
-    SGX_CUDA(cudaStreamSynchronize(s));
-  }
-  return SGX_OK;
+  return out.finish(s);
 }

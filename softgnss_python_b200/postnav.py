@@ -220,19 +220,11 @@ def nav_velocity_batch(track_out, nav_out, sub_frame_start, eph, tow, settings, 
     L.require_device()
     shape = tuple(track_out.shape)
     r, c, ms = shape[0], shape[1], shape[-1]
-    on_device = hasattr(track_out, "data_ptr")
-    if not on_device:
-        track_out = np.ascontiguousarray(track_out, dtype=np.float64)
-        base = track_out.ctypes.data
-    else:
-        import torch
-        assert track_out.is_cuda and track_out.dtype == torch.float64 and track_out.is_contiguous()
-        base = track_out.data_ptr()
     if len(shape) == 4:
-        assert shape[2] == len(_native.TRACK_FIELDS), "track_out must be [R, C, 13, ms] or [R, C, ms]"
-        carr, stride = base + 8 * _native.TRACK_FIELDS.index("carrFreq") * ms, len(_native.TRACK_FIELDS) * ms
-    else:
-        carr, stride = base, ms
+        carr, stride, keep = _native.track_field(track_out, "carrFreq")
+    else:                                                    # [R, C, ms] carrFreq rows
+        carr = keep = track_out if hasattr(track_out, "data_ptr") else np.ascontiguousarray(track_out, dtype=np.float64)
+        stride = ms
     out = L.nav_velocity(carr, stride, r, c, ms, ms_done, sub_frame_start, eph, tow, nav_out["n_epochs"],
                          nav_out["active"], nav_out["sol"], vel_settings(settings), want_sat=want_sat, stream=stream)
     if not want_sat:
@@ -367,16 +359,11 @@ def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_d
     recordings with fewer than four usable satellites get ``n_epochs = 0``.  With ``velocity=True`` the dict also
     carries ``vel``, ``doppler`` and ``rrResid`` of :func:`nav_velocity_batch` (carrFreq read in place; ``ms_done``
     ``[R, C]`` as returned by ``track_batch``, None for all ms)."""
-    r, c, nf, ms = track_out.shape
+    r, c, _, ms = track_out.shape
     prn = np.asarray(prn).reshape(r, c)
-    if isinstance(track_out, np.ndarray):
-        ip = np.ascontiguousarray(track_out[:, :, 3, :]).reshape(r * c, ms)
-        first, bits, valid = find_preambles_batch(ip, stream=stream)
-        abs_in, stride = np.ascontiguousarray(track_out[:, :, 0, :]), ms
-    else:
-        ip = track_out.view(r * c, nf * ms)[:, 3 * ms:4 * ms]              # I_P rows, row stride 13 * ms
-        first, bits, valid = find_preambles_batch(ip, stream=stream)
-        abs_in, stride = track_out, nf * ms
+    L = _native.lib()
+    ip, stride, track_out = _native.track_field(track_out, "I_P")
+    first, bits, valid = L.find_preambles(ip, stride, r * c, ms, stream=stream)
     first = first.reshape(r, c)
     first[prn == 0] = 0
     ready = np.zeros((r, c), dtype=np.uint8)
@@ -393,8 +380,8 @@ def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_d
             rows[i] = eph_rows(eph, np.where(ready[i] > 0, prn[i], 0))
             tow[i] = t
             n_ep[i] = nav_epochs(settings, first[i])
-    out = _native.lib().nav_solve(abs_in, stride, r, c, ms, first, ready, rows, tow, n_ep, nav_settings(settings),
-                                  stream=stream)
+    abs_sample = _native.track_field(track_out, "absoluteSample")[0]
+    out = L.nav_solve(abs_sample, stride, r, c, ms, first, ready, rows, tow, n_ep, nav_settings(settings), stream=stream)
     out.update(subFrameStart=first, ready=ready, tow=tow, eph=ephs)
     if velocity:
         out.update(nav_velocity_batch(track_out, out, first, rows, tow, settings, ms_done=ms_done, stream=stream))

@@ -142,28 +142,21 @@ def track_quality_batch(track_out, ms_done=None, settings=None, stream=0):
     L = _native.lib()
     L.require_device()
     qs = quality_pod(settings)
-    nf = len(FIELDS)
-    on_device = hasattr(track_out, "data_ptr")
-    if not on_device:
-        track_out = np.ascontiguousarray(track_out, dtype=np.float64)
-    r, c, f, ms = track_out.shape
-    assert f == nf, "track_out must be [R, C, %d, ms]" % nf
+    r, c, _, ms = track_out.shape
+    i_p, stride, track_out = _native.track_field(track_out, "I_P")
+    q_p = _native.track_field(track_out, "Q_P")[0]
     n_win = ms // qs.window_ms if qs.window_ms >= 2 else 0   # W < 2 is refused by the library
-    if on_device:
+    if hasattr(track_out, "data_ptr"):
         import torch
-        assert track_out.is_cuda and track_out.dtype == torch.float64 and track_out.is_contiguous()
-        base = track_out.data_ptr()
         res = dict(cn0=torch.empty((r, c, n_win), dtype=torch.float64, device=track_out.device),
                    pllLock=torch.empty((r, c, n_win), dtype=torch.float64, device=track_out.device),
                    locked=torch.empty((r, c, n_win), dtype=torch.uint8, device=track_out.device))
     else:
-        base = track_out.ctypes.data
         res = dict(cn0=np.empty((r, c, n_win)), pllLock=np.empty((r, c, n_win)),
                    locked=np.empty((r, c, n_win), dtype=np.uint8))
     done = None if ms_done is None else np.ascontiguousarray(ms_done, dtype=np.int32).reshape(r * c)
-    i_p, q_p = base + 8 * FIELDS.index("I_P") * ms, base + 8 * FIELDS.index("Q_P") * ms
     if n_win or qs.window_ms < 2:           # (an empty CUDA tensor has no address to pass)
-        L.check(L.track_quality(i_p, q_p, nf * ms, r * c, ms, done, qs, res["cn0"], res["pllLock"], res["locked"],
+        L.check(L.track_quality(i_p, q_p, stride, r * c, ms, done, qs, res["cn0"], res["pllLock"], res["locked"],
                                 stream))
     res["index"] = (np.arange(n_win, dtype=np.int64) + 1) * qs.window_ms
     return res

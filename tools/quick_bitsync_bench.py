@@ -12,8 +12,6 @@ ipv = big.view(n, 13 * ms)[:, 3 * ms:4 * ms]
 first = torch.zeros(n, dtype=torch.int32, device="cuda")
 bits = torch.zeros((n, 1501), dtype=torch.uint8, device="cuda")
 valid = torch.zeros(n, dtype=torch.int32, device="cuda")
-import ctypes
-L.dll.sgx_find_preambles.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 for mode in ("device outputs", "host outputs"):
     ts = []
