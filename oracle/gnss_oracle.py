@@ -134,12 +134,14 @@ def acquire(long_signal, s, coherent_ms=1, noncoh_blocks=2, doppler_step=500.0,
     for prn in range(nprn):
         code_f = np.fft.fft(table[prn]).conj()                             # :95
         results = np.zeros((nbins, n1))
+        block_max = np.zeros((nbins, noncoh_blocks))
         for k in range(nbins):
             best = None
             for b in range(noncoh_blocks):
                 r = abs(np.fft.ifft(spec[b, k] * code_f)) ** 2             # :120-126
                 if coherent_ms > 1:
                     r = r[:n1]      # extension: the correlation repeats every code period; search one
+                block_max[k, b] = r.max()
                 # :129-133 keep block 1 only if strictly larger, later blocks win ties
                 if best is None or not (best.max() > r.max()):
                     best = r
@@ -154,7 +156,11 @@ def acquire(long_signal, s, coherent_ms=1, noncoh_blocks=2, doppler_step=500.0,
         second = results[fbin, rng].max()                                  # :162
         metric[prn] = peak / second                                        # :164
         if return_debug:
-            dbg[prn] = dict(bin=int(fbin), codePhase=cp, peak=peak, second=second)
+            # besides the decisions, what a test needs to see how clear they are: the block maxima of every bin, the
+            # row maxima (bin decision), the column maxima (code phase), the winning row and where its second peak is
+            dbg[prn] = dict(bin=int(fbin), codePhase=cp, peak=peak, second=second,
+                            secondIndex=int(rng[results[fbin, rng].argmax()]) % n1, blockMax=block_max,
+                            binMax=results.max(1), colMax=results.max(0), row=results[fbin].copy())
         if peak / second > s.acqThreshold:                                 # :166
             code = ca_code_cached(prn)
             idx = np.floor(ts * np.arange(1, 10 * n1 + 1) / (1.0 / s.codeFreqBasis))   # :172
@@ -169,6 +175,8 @@ def acquire(long_signal, s, coherent_ms=1, noncoh_blocks=2, doppler_step=500.0,
             cph[prn] = cp                                                  # :193
             if return_debug:
                 dbg[prn]["fineIndex"] = int(imax)
+                dbg[prn]["fineRunnerUp"] = float(np.delete(mag[4:uniq - 5], imax).max())
+                dbg[prn]["finePeak"] = float(mag[4 + imax])
     out = dict(carrFreq=carr, codePhase=cph, peakMetric=metric)
     if return_debug:
         out["debug"] = dbg
