@@ -184,7 +184,8 @@ int sgx_fft_c2c(const float* in, float* out, int32_t n, int32_t batch, int32_t i
  *   nav_bits_valid  optional int32 [n_channels]: 1 when that window lies inside the record; written only
  *                   when nav_bits is given
  * Candidates nearer than 40 ms to the start of the record are passed over (the reference reads
- * I_P[k-40:...] with a negative start there and raises). */
+ * I_P[k-40:...] with a negative start there and raises).  ms <= 819 072 (the search keeps two bits per ms in
+ * 200 KB of shared memory); a longer record returns SGX_ERR_RANGE before anything is launched or written. */
 int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_channels, int32_t ms,
                        int32_t* first_subframe, uint8_t* nav_bits, int32_t* nav_bits_valid,
                        void* cuda_stream);
@@ -194,7 +195,8 @@ int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_channels, in
  * fix stay with the reference's host code).
  *   track_out     double [n_recordings][n_channels][SGX_TRACK_FIELDS][ms] as written by sgx_track; only
  *                 field 0 (absoluteSample) is read
- *   ms_index      int32 [n_recordings][n_epochs][n_channels]: msOfTheSignal per channel
+ *   ms_index      int32 [n_recordings][n_epochs][n_channels]: msOfTheSignal per channel; an index outside
+ *                 [0, ms) counts as not listed (the reference would wrap a negative index or raise)
  *   active        uint8 [n_recordings][n_epochs][n_channels]: 1 = channel is in channelList (others get +inf
  *                 travel time, i.e. an infinite pseudorange, as in the reference)
  *   pseudoranges  double [n_recordings][n_epochs][n_channels], metres:

@@ -225,7 +225,8 @@ extern "C" int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_c
   a.ms = ms;
   a.n_words = (ms + 31) / 32;
   const size_t smem = sizeof(unsigned) * (2 * (size_t)a.n_words + 8);
-  if (smem > 200 * 1024) return fail(SGX_ERR_RANGE, "sgx_find_preambles", "record longer than 800 000 ms");
+  // 200 KB holds the sign and candidate words of 819 072 ms (25 596 words); longer records are refused
+  if (smem > 200 * 1024) return fail(SGX_ERR_RANGE, "sgx_find_preambles", "record longer than 819 072 ms");
   cudaStream_t s = (cudaStream_t)cuda_stream;
   const size_t n = (size_t)n_channels;
   int32_t* valid = nav_bits ? nav_bits_valid : nullptr;   // written only together with nav_bits
@@ -236,7 +237,11 @@ extern "C" int sgx_find_preambles(const double* i_p, int64_t stride, int32_t n_c
       (r = out.add(nav_bits, (size_t)NAV_BITS * n, g_bs.bits, a.bits)) ||
       (r = out.add(valid, n, g_bs.valid, a.bits_valid)))
     return r;
-  if (smem > 48 * 1024)
+  // above 48 KB a block's shared memory, its static part included, needs the opt-in attribute.  The static part is
+  // `best` placed ahead of the 1024-byte aligned dynamic array: 2 KB in the sm_100a build, so not negligible.
+  cudaFuncAttributes fa;
+  SGX_CUDA(cudaFuncGetAttributes(&fa, bitsync_kernel));
+  if (smem + fa.sharedSizeBytes > 48 * 1024)
     SGX_CUDA(cudaFuncSetAttribute(bitsync_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   SGX_COUNTED_LAUNCH(bitsync_kernel, dim3(n_channels), dim3(BS_THREADS), smem, s, a);
   SGX_CUDA(cudaGetLastError());

@@ -246,8 +246,9 @@ def build_chain_case(seed=2, ms=NAV_MS, n_code=38192, fs=38.192e6, first_boundar
     return track, np.array(truth["prn"], dtype=np.int64), truth
 
 
-def oracle_chain(track, prn, settings_kw):
-    """The same chain with the oracle: find_preambles, nav_bits, ephemeris, nav_solve.  Returns (first, nav dict | None)."""
+def oracle_chain(track, prn, settings_kw, samples_per_code=38192):
+    """The same chain with the oracle: find_preambles, nav_bits, ephemeris, nav_solve.  Returns (first, nav dict | None).
+    ``samples_per_code``: settings.samplesPerCode of the rate the absoluteSample series was made for."""
     from oracle import gnss_oracle as orc
     n_ch, _, ms = track.shape
     first, active = orc.find_preambles([track[c, 3] for c in range(n_ch)])
@@ -262,4 +263,5 @@ def oracle_chain(track, prn, settings_kw):
             ready.append(ch)
     if len(ready) < 4:
         return first, None
-    return first, orc.nav_solve([track[c, 0] for c in range(n_ch)], prn, first, ready, eph, tow, float(ms), 38192, **settings_kw)
+    return first, orc.nav_solve([track[c, 0] for c in range(n_ch)], prn, first, ready, eph, tow, float(ms), samples_per_code,
+                                  **settings_kw)

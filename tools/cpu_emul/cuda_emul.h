@@ -394,6 +394,8 @@ static inline cudaError_t cudaPointerGetAttributes(cudaPointerAttributes* a, con
   return 0;
 }
 template <class F> static inline cudaError_t cudaFuncSetAttribute(F, cudaFuncAttribute, int) { return 0; }
+struct cudaFuncAttributes { size_t sharedSizeBytes; };
+template <class F> static inline cudaError_t cudaFuncGetAttributes(cudaFuncAttributes* a, F) { a->sharedSizeBytes = 0; return 0; }
 enum cudaDeviceAttr { cudaDevAttrMultiProcessorCount = 16 };
 static inline cudaError_t cudaDeviceGetAttribute(int* v, cudaDeviceAttr, int) { *v = 8; return 0; }
 template <class F> static inline cudaError_t cudaOccupancyMaxActiveBlocksPerMultiprocessor(int* n, F, int, size_t) { *n = 2; return 0; }
