@@ -213,6 +213,15 @@ __device__ __forceinline__ unsigned lds_u32(const void* base, unsigned base_s, i
   return v;
 #endif
 }
+__device__ __forceinline__ uint2 lds_u32x2(const void* base, unsigned base_s, int byte_off) {   // 8-byte aligned
+#ifdef SGX_EMUL
+  (void)base_s; return *reinterpret_cast<const uint2*>(reinterpret_cast<const char*>(base) + byte_off);
+#else
+  (void)base; uint2 v;
+  asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(base_s + (unsigned)byte_off));
+  return v;
+#endif
+}
 __device__ __forceinline__ uint4 lds_u32x4(const void* base, unsigned base_s, int byte_off) {   // 16-byte aligned
 #ifdef SGX_EMUL
   (void)base_s; return *reinterpret_cast<const uint4*>(reinterpret_cast<const char*>(base) + byte_off);

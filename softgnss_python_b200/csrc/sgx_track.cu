@@ -32,6 +32,7 @@
 //    -fmad=false) exactly in the reference's order, and the carrier thread's warp rebuilds the twiddle tables.
 //  * host recordings are streamed in chunks (pause/resume through TrackState); files through two pinned staging
 //    buffers (sgx_track_file).
+#include <algorithm>
 #include <vector>
 #include <fcntl.h>
 #include <sys/stat.h>
@@ -46,6 +47,26 @@ constexpr int TRK_MARGIN = 256;  // extra samples staged beyond samplesPerCode
 // SGX_TRK_PROF phases, stamped by lane 0 of every warp: window wait + prefetch issue, correlate, reduce + barrier,
 // bookkeeping (loop filters, next period's parameters and tables), end-of-period barrier
 constexpr int TRK_PROF_N = 5;
+// SGX_TRK_PROF per-CTA record: SM id, global timer (ns) at the start and at the end of the CTA
+constexpr int TRK_CTA_N = 3;
+__device__ __forceinline__ long long sm_id() {
+#ifdef SGX_EMUL
+  return 0;
+#else
+  unsigned v;
+  asm volatile("mov.u32 %0, %%smid;" : "=r"(v));
+  return v;
+#endif
+}
+__device__ __forceinline__ long long global_ns() {
+#ifdef SGX_EMUL
+  return 0;
+#else
+  unsigned long long v;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(v));
+  return (long long)v;
+#endif
+}
 
 struct TrackArgs {
   const int8_t* rec;
@@ -61,7 +82,8 @@ struct TrackArgs {
   int resume;           // continue every channel from `state` (streaming ingest: the recording arrives in chunks)
   long long avail;      // bytes of every recording that are resident so far (>= rec_len when complete)
   struct TrackState* state;  // [R*C]
-  long long* prof;      // optional [R*C][warp][TRK_PROF_N] cycle counters per period phase (SGX_TRK_PROF=1)
+  long long* prof;      // optional [R*C][warp][TRK_PROF_N] cycle counters per period phase, then [R*C][TRK_CTA_N]
+                        // per-CTA records (SGX_TRK_PROF=1)
   int win;              // bytes per staging buffer, multiple of 16
   long long skip;
   long long abs_base;   // sample index of rec[0] in the file (streamed windows start at the first byte that is needed)
@@ -634,18 +656,23 @@ __device__ __forceinline__ double flip_sign(double x, unsigned m) {
 
 // exact double of the 46-bit integer lo + mid*2^16 + hi*2^32 (|value| < 2^51) without an int->double conversion
 // instruction: the integer, offset by 2^51, is written straight into the mantissa of 2^52 and the offset removed by
-// one exact subtraction
+// one exact subtraction.  hi and the exponent pattern only touch the high word, so they join it in one 32-bit add
+// instead of a carried 64-bit one.
 __device__ __forceinline__ double digits_to_double(int lo, int mid, int hi) {
-  long long v = (long long)mid * 65536 + (long long)lo;
-  v += (long long)hi << 32;
-  v += 0x4338000000000000LL;            // 2^52 exponent pattern, plus the 2^51 offset inside the mantissa
-  return __longlong_as_double(v) - 6755399441055744.0;   // 2^52 + 2^51
+  const long long v = (long long)mid * 65536 + (long long)lo;   // |v| < 2^43
+  // 0x43380000 in the high word: 2^52 exponent pattern, plus the 2^51 offset inside the mantissa
+  return __hiloint2double((int)(v >> 32) + hi + 0x43380000, (int)v) - 6755399441055744.0;   // 2^52 + 2^51
 }
 
-// Exact correlator.  Thread tid walks the SEGS half-chip segments n = SEGS*tid - 1 ... in a ROLLED loop: one copy
-// of the segment body (about 170 instructions) instead of eight keeps the whole period loop inside the SM's
-// instruction cache (the unrolled kernel fetched instructions from the GPC-level cache at 88 % of that cache's
+// Exact correlator.  Thread tid walks the SEGS half-chip segments n = SEGS*tid - 1 ... in a ROLLED loop of one chip
+// (two segments): two copies of the segment body instead of eight keep the whole period loop inside the SM's
+// instruction cache (the fully unrolled kernel fetched instructions from the GPC-level cache at 88 % of that cache's
 // peak and stalled on it -- profiles/ncu_summary_r1_v3.md).
+// With +-0.5-chip spacing segment s (n = SEGS*tid - 1 + s) has, relative to chip 4 tid, E = floor(s/2), L = E + 1
+// and P = floor((s+1)/2): each replica keeps one chip over two consecutive segments.  So each accumulator is kept
+// in the sign frame of its replica's current chip (it holds code sign * sum) and takes the segment sums unsigned;
+// it is negated only where the code sign changes between consecutive chips.  Negation is exact and rounding is
+// symmetric in sign, so the sums are bit for bit those of applying the code sign to every segment sum.
 template <int NW, int SEGS>
 __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParams& Pcold, const int8_t* cur,
                                                 const unsigned char* codeB, const ExactTables& T, int tid,
@@ -658,29 +685,22 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
   const int n0 = SEGS * tid - 1;
   // boundaries are equally spaced in the predicted (real-valued) sample index q_n = (n/2 - rem) / step;
   // the prediction runs in Q40 fixed point (error < 1e-9 samples over the 2046 thresholds)
-  const long long FR_ONE = 1LL << 40, FR_EPS = 1099512;   // 1e-6 in Q40
   long long qf = P.q0_fix + (long long)n0 * P.h_fix;
-  // boundary of threshold n -> first sample of segment n, with IRREGULAR possibly set
+  // boundary of threshold n >= 0 -> first sample of segment n, with IRREGULAR possibly set
   auto boundary = [&](int n, long long q) -> int {
-    if (n < 0) return 0;
     if (n > 2046) return P.blk;
-    const long long fr = q & (FR_ONE - 1);
-    // too close to a sample instant: settle with the exact expressions (Pcold: the shared-memory copy of the
-    // parameters, so that P can stay in registers)
-    if (fr < FR_EPS || fr > FR_ONE - FR_EPS) return settle_boundary(n, Pcold);
+    // too close to a sample instant (fraction within 1e-6 = 1099512 / 2^40 of an integer): settle with the exact
+    // expressions (Pcold: the shared-memory copy of the parameters, so that P can stay in registers).  The test
+    // runs on the top 32 of the 40 fraction bits with a margin of one unit, so it flags a superset of those
+    // fractions; in the extra 2^-32-wide band the prediction and the settled boundary agree.
+    constexpr unsigned EPS32 = 1099512 / 256 + 2;
+    if ((unsigned)(q >> 8) + EPS32 < 2 * EPS32) return settle_boundary(n, Pcold);
     return max(0, min((int)(q >> 40) + 1, P.blk));   // (a prediction of -1 occurs when rem is within rounding of one step)
   };
-  int a = boundary(n0, qf);
+  int a;
+  if (n0 < 0) a = 0;
+  else a = boundary(n0, qf);
   if ((a & ~IRREGULAR) >= P.blk) return;
-  // Thread 0's first segment (n = -1: the samples before the first prompt threshold) is empty unless the block starts
-  // at or before a threshold.  Skipping it makes that thread's first rotor evaluation (start_rotor, below) fall in
-  // the same iteration as its warp's other lanes: one evaluation per warp instead of two (measured at 32 recordings:
-  // warp 0's correlation ended ~820 cycles after the other warps' with the second evaluation, ~460 without).
-  int s0 = 0;
-  if (n0 < 0) {
-    const int b0 = boundary(0, qf + P.h_fix);
-    if ((b0 & ~IRREGULAR) == (a & ~IRREGULAR)) { s0 = 1; qf += P.h_fix; a = b0; }
-  }
   // packed twiddle digits: tw[c][d] word q holds samples 4q .. 4q+3
   int twr[ND][NW], twi[ND][NW];
 #pragma unroll
@@ -694,60 +714,74 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
   // two conflict-free aligned words per period instead of three float64 table reads per segment
   unsigned sg_lo = reinterpret_cast<const unsigned*>(codeB)[tid];       // chips 4 tid .. 4 tid + 3
   unsigned sg_hi = reinterpret_cast<const unsigned*>(codeB)[tid + 1];   // chip 4 tid + 4 in its low byte
-  double rotr = 1.0, roti = 0.0;
-  double aEr = 0, aEi = 0, aPr = 0, aPi = 0, aLr = 0, aLi = 0;
-  bool fresh = true;
+  // The rotor of the first segment, evaluated before the loop so that all lanes of a warp evaluate it together
+  // (thread 0's first segment, n = -1, is usually empty; evaluated inside the loop its rotor fell one segment later
+  // than its warp's other lanes', a second evaluation per warp: measured at 32 recordings, warp 0's correlation
+  // ended ~820 cycles after the other warps' with it, ~460 without).  An empty segment leaves a, so the rotor, as is.
+  double rotr, roti;
+  {
+    const double2 r0 = start_rotor(a & ~IRREGULAR, Pcold);
+    rotr = r0.x; roti = r0.y;
+  }
+  double aEr = 0, aEi = 0, aPr = 0, aPi = 0, aLr = 0, aLi = 0;   // in the sign frames of the current chips
+  // a segment that leaves no valid rotor for the next one (a rare path) evaluates the next one's start rotor itself,
+  // unless no segment of this thread follows
+  auto restart_rotor = [&](int s, int b) {
+    if (s + 1 < SEGS && (b & ~IRREGULAR) < P.blk) {
+      const double2 r0 = start_rotor(b & ~IRREGULAR, Pcold);
+      rotr = r0.x; roti = r0.y;
+    }
+  };
   const unsigned cur_s = smem_addr(cur), z_s = smem_addr(&T.z[0][0]);
-#pragma unroll 1
-  for (int s = s0; s < SEGS; ++s) {
+  // byte c: code sign byte of chip c XOR that of chip c + 1 (chips relative to 4 tid, c = 0 .. 3; zeros above)
+  unsigned dsg = sg_lo ^ __funnelshift_r(sg_lo, sg_hi, 8);
+  auto segment = [&](const int s) {
     qf += P.h_fix;
     const int b = boundary(n0 + s + 1, qf);
     const int len = (b & ~IRREGULAR) - (a & ~IRREGULAR);
     if (len > 0) {
       if (len > LMAX || ((a | b) & IRREGULAR)) {
         // rare: a segment longer than the twiddle table, or one whose boundary is not shared by E, P and L.
-        // Per-sample evaluation; its sums join the scaled accumulators through an exact power of two.
+        // Per-sample evaluation; its sums (code signs applied) join the scaled accumulators through an exact power
+        // of two, in the accumulators' sign frames.
         double acc[6] = {0, 0, 0, 0, 0, 0};
         correlate_per_sample(Pcold, cur, codeB, off, a & ~IRREGULAR, b & ~IRREGULAR, acc);
         const double up = (double)(1LL << (8 * ND - 2));
-        aEr += acc[0] * up; aEi += acc[1] * up; aPr += acc[2] * up; aPi += acc[3] * up; aLr += acc[4] * up; aLi += acc[5] * up;
-        fresh = true;
+        const unsigned mE = (unsigned)codeB[4 * tid + (s >> 1)] << 24, mL = (unsigned)codeB[4 * tid + (s >> 1) + 1] << 24;
+        const unsigned mP = (s & 1) ? mL : mE;
+        aEr += flip_sign(acc[0] * up, mE); aEi += flip_sign(acc[1] * up, mE);
+        aPr += flip_sign(acc[2] * up, mP); aPi += flip_sign(acc[3] * up, mP);
+        aLr += flip_sign(acc[4] * up, mL); aLi += flip_sign(acc[5] * up, mL);
+        restart_rotor(s, b);
       } else {
-        // chips relative to 4 tid: E = floor(s/2), L = E + 1, P = floor((s+1)/2) = E (s even) or L (s odd)
-        // (n = 8 tid - 1 + s); the sign bytes are shifted down by one chip after every odd s
-        const unsigned mE = sg_lo << 24, mL = __byte_perm(sg_lo, 0u, 0x1444), mP = (s & 1) ? mL : mE;
-        if (fresh) {
-          const double2 r0 = start_rotor(a, Pcold);
-          rotr = r0.x; roti = r0.y;
-          fresh = false;
+        // The NW + 1 words from the one holding sample a onwards.  8-byte loads from the 8-byte aligned base leave
+        // one select level (odd word: shift the loaded words down by one) instead of two for 16-byte loads.  At
+        // the lanes' ~150-byte stride a half warp's 8-byte loads fall on banks at most 3 deep: ~3 wavefronts per
+        // word against ~2 for 16-byte and ~6 for 32-bit loads, and no more words loaded per segment than with
+        // 16-byte loads.  The extra word is fetched only by the lanes that need it; no word beyond word NW of
+        // sample a's is read.
+        const int sa = off + a;
+        const int sh = (sa & 3) * 8;
+        const bool odd = (sa & 4) != 0;
+        constexpr int NP = (NW + 2) / 2;          // 8-byte pairs: words 0 .. 2 NP - 1 from the aligned base
+        unsigned wd[2 * NP + 1];
+#pragma unroll
+        for (int p = 0; p < NP; ++p) {
+          const uint2 v = lds_u32x2(cur, cur_s, (sa & ~7) + 8 * p);
+          wd[2 * p] = v.x; wd[2 * p + 1] = v.y;
         }
-        const int sh = ((off + a) & 3) * 8;
-        unsigned raw[NW + 1];   // the NW + 1 words from the one holding sample a onwards
-        {
-          // 16-byte loads from the aligned base: lanes sit ~150 bytes apart, which put the 32-bit loads of a warp
-          // on ~6 distinct banks (6 wavefronts per load); a 16-byte load spreads a quarter warp over 8 bank quads
-          // (2 wavefronts per quarter).  The last quad is fetched only by the lanes that need a word of it.
-          constexpr int NQ = (NW + 7) / 4;          // quads covering words j .. j + NW for every j in 0 .. 3
-          const int ab = (off + a) & ~15, j = ((off + a) >> 2) & 3;
-          unsigned wd[4 * NQ];
+        wd[2 * NP] = 0u;
+        if (2 * NP < NW + 2 && odd) wd[2 * NP] = lds_u32(cur, cur_s, (sa & ~7) + 8 * NP);
+        unsigned raw[NW + 1];
 #pragma unroll
-          for (int q = 0; q < NQ; ++q) {
-            uint4 v = make_uint4(0u, 0u, 0u, 0u);
-            if (q < NQ - 1 || j + NW >= 4 * (NQ - 1)) v = lds_u32x4(cur, cur_s, ab + 16 * q);
-            wd[4 * q] = v.x; wd[4 * q + 1] = v.y; wd[4 * q + 2] = v.z; wd[4 * q + 3] = v.w;
-          }
-          unsigned t[NW + 2];
-#pragma unroll
-          for (int q = 0; q < NW + 2; ++q) t[q] = (j & 2) ? wd[q + 2] : wd[q];
-#pragma unroll
-          for (int q = 0; q <= NW; ++q) raw[q] = (j & 1) ? t[q + 1] : t[q];
-        }
-        // bytes at and beyond len are not part of this segment: the last word is always masked, the others only
-        // in a short segment (fewer than LMAX - 4 samples: block edges)
+        for (int q = 0; q <= NW; ++q) raw[q] = odd ? wd[q + 1] : wd[q];
+        // bytes at and beyond len are not part of this segment: the last word is always masked (8 (LMAX - len) >= 0
+        // bits off its top, clamped at 32), the others only in a short segment (fewer than LMAX - 4 samples: block
+        // edges)
         unsigned w[NW];
 #pragma unroll
         for (int q = 0; q < NW; ++q) w[q] = __funnelshift_r(raw[q], raw[q + 1], sh);
-        w[NW - 1] &= __funnelshift_lc(0xFFFFFFFFu, 0u, max(8 * (len - 4 * (NW - 1)), 0));
+        w[NW - 1] &= __funnelshift_rc(0xFFFFFFFFu, 0u, 8 * (LMAX - len));
         if (len < LMAX - 4) {
 #pragma unroll
           for (int q = 0; q < NW - 1; ++q) w[q] &= __funnelshift_lc(0xFFFFFFFFu, 0u, max(8 * (len - 4 * q), 0));
@@ -768,23 +802,41 @@ __device__ __forceinline__ void correlate_exact(const MsParams& P, const MsParam
         const double Sr = digits_to_double(xr[1] * 256 + xr[0], xr[3] * 256 + xr[2], ND == 5 ? xr[ND - 1] : 0);
         const double Si = digits_to_double(xi[1] * 256 + xi[0], xi[3] * 256 + xi[2], ND == 5 ? xi[ND - 1] : 0);
         const double Rr = fma(rotr, Sr, -(roti * Si)), Ri = fma(rotr, Si, roti * Sr);
-        aEr += flip_sign(Rr, mE); aEi += flip_sign(Ri, mE);
-        aPr += flip_sign(Rr, mP); aPi += flip_sign(Ri, mP);
-        aLr += flip_sign(Rr, mL); aLi += flip_sign(Ri, mL);
+        aEr += Rr; aEi += Ri; aPr += Rr; aPi += Ri; aLr += Rr; aLi += Ri;
+        // rotor of the next segment: one step e^{j 2 pi len cps} for the usual lengths LMAX - 4 .. LMAX, a fresh
+        // evaluation after a short segment
         const int j = len - (LMAX - 4);
-        if (j >= 0) {
-          const double2 z = lds_f64x2(&T.z[0][0], z_s, 16 * j);
-          const double zr = z.x, zi = z.y;
-          const double nr = fma(rotr, zr, -(roti * zi)), ni = fma(rotr, zi, roti * zr);
-          rotr = nr; roti = ni;
-        } else {
-          fresh = true;
-        }
+        const double2 z = lds_f64x2(&T.z[0][0], z_s, 16 * max(j, 0));
+        const double zr = z.x, zi = z.y;
+        const double nr = fma(rotr, zr, -(roti * zi)), ni = fma(rotr, zi, roti * zr);
+        rotr = nr; roti = ni;
+        if (j < 0) restart_rotor(s, b);
       }
     }
     a = b;
-    if (s & 1) { sg_lo = __funnelshift_r(sg_lo, sg_hi, 8); sg_hi >>= 8; }
+    // chip changes (s is the same on every lane of the warp): after an odd segment E and L move on by a chip, after
+    // an even one P
+    const unsigned d0 = dsg << 24;
+    if (s & 1) {
+      const unsigned d1 = __byte_perm(dsg, 0u, 0x1444);
+      aEr = flip_sign(aEr, d0); aEi = flip_sign(aEi, d0);
+      aLr = flip_sign(aLr, d1); aLi = flip_sign(aLi, d1);
+      dsg >>= 8;
+    } else {
+      aPr = flip_sign(aPr, d0); aPi = flip_sign(aPi, d0);
+    }
+  };
+  // one chip per iteration: the parity of s is known in each copy of the segment body
+#pragma unroll 1
+  for (int s = 0; s < SEGS; s += 2) {
+    segment(s);
+    segment(s + 1);
   }
+  // all three frames end on chip 4 tid + 4 (E after its last change, L with no change after chip 4 tid + 4 -- zero
+  // byte -- and P after its last even segment)
+  const unsigned m4 = reinterpret_cast<const unsigned*>(codeB)[tid + 1] << 24;
+  aEr = flip_sign(aEr, m4); aEi = flip_sign(aEi, m4); aPr = flip_sign(aPr, m4); aPi = flip_sign(aPi, m4);
+  aLr = flip_sign(aLr, m4); aLi = flip_sign(aLi, m4);
   const double sc = 1.0 / (double)(1LL << (8 * ND - 2));   // 2^-30 or 2^-38
   tEr += aEr * sc; tEi += aEi * sc; tPr += aPr * sc; tPi += aPi * sc; tLr += aLr * sc; tLi += aLi * sc;
 }
@@ -811,6 +863,9 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
   const int cid = blockIdx.x;  // recording * n_channels + channel
   const int rid = cid / a.n_channels;
   const sgx_channel chn = a.ch[cid];
+  // (recomputed where it is used: a pointer held across the period loop would take a register from it)
+  auto cta_prof = [&]() { return a.prof + (long long)gridDim.x * (NT / 32) * TRK_PROF_N + (long long)cid * TRK_CTA_N; };
+  if (a.prof && tid == 0) { long long* c = cta_prof(); c[0] = sm_id(); c[1] = global_ns(); c[2] = c[1]; }
   if (chn.prn == 0) {  // tracking.py:99 -- idle channel, no record
     if (tid == 0) {
       a.ms_done[cid] = 0;
@@ -1021,6 +1076,7 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
     cp_async_wait_all();
   }
   if (tid == 0) {
+    if (a.prof) cta_prof()[2] = global_ns();
     const int status = (k == a.ms) ? SGX_OK : prm.stop;
     a.ms_done[cid] = k;
     a.status[cid] = status;
@@ -1034,6 +1090,46 @@ __global__ void __launch_bounds__(NT, 2) track_kernel(TrackArgs a) {
 }
 
 // --------------------------------------------------------------------------- host entry
+// SGX_TRK_PROF: what sets the launch's run time -- the spread of the CTAs' start and end times, and the CTAs per SM
+// with the time each SM was busy (first start to last end of its CTAs)
+static void print_cta_makespan(const long long* r, int nch) {
+  long long t0 = r[1], t1 = r[2];
+  for (int i = 0; i < nch; ++i) { t0 = std::min(t0, r[TRK_CTA_N * i + 1]); t1 = std::max(t1, r[TRK_CTA_N * i + 2]); }
+  std::vector<double> dur(nch), endt(nch), startt(nch);
+  int nsm = 0;
+  for (int i = 0; i < nch; ++i) {
+    nsm = std::max(nsm, (int)r[TRK_CTA_N * i] + 1);
+    startt[i] = 1e-3 * (double)(r[TRK_CTA_N * i + 1] - t0);
+    endt[i] = 1e-3 * (double)(r[TRK_CTA_N * i + 2] - t0);
+    dur[i] = endt[i] - startt[i];
+  }
+  std::vector<int> per_sm(nsm, 0);
+  std::vector<double> sm_first(nsm, 1e300), sm_last(nsm, 0.0);
+  for (int i = 0; i < nch; ++i) {
+    const int sm = (int)r[TRK_CTA_N * i];
+    ++per_sm[sm];
+    sm_first[sm] = std::min(sm_first[sm], startt[i]);
+    sm_last[sm] = std::max(sm_last[sm], endt[i]);
+  }
+  auto q = [](std::vector<double> v, double f) { std::sort(v.begin(), v.end()); return v[(size_t)(f * (v.size() - 1))]; };
+  fprintf(stderr, "[sgx prof] CTAs %d, kernel span %.1f us (first CTA start to last CTA end)\n", nch, 1e-3 * (double)(t1 - t0));
+  fprintf(stderr, "[sgx prof]   us:        min      p10   median      p90      max\n");
+  fprintf(stderr, "[sgx prof]   start  %8.1f %8.1f %8.1f %8.1f %8.1f\n", q(startt, 0), q(startt, .1), q(startt, .5), q(startt, .9), q(startt, 1));
+  fprintf(stderr, "[sgx prof]   end    %8.1f %8.1f %8.1f %8.1f %8.1f\n", q(endt, 0), q(endt, .1), q(endt, .5), q(endt, .9), q(endt, 1));
+  fprintf(stderr, "[sgx prof]   CTA    %8.1f %8.1f %8.1f %8.1f %8.1f\n", q(dur, 0), q(dur, .1), q(dur, .5), q(dur, .9), q(dur, 1));
+  for (int c = 1; c <= 8; ++c) {
+    int n = 0;
+    double busy_min = 1e300, busy_max = 0.0, busy_sum = 0.0;
+    for (int sm = 0; sm < nsm; ++sm)
+      if (per_sm[sm] == c) {
+        const double b = sm_last[sm] - sm_first[sm];
+        ++n; busy_sum += b; busy_min = std::min(busy_min, b); busy_max = std::max(busy_max, b);
+      }
+    if (n) fprintf(stderr, "[sgx prof]   SMs with %d CTAs: %3d, busy min / mean / max %.1f / %.1f / %.1f us\n", c, n, busy_min,
+                   busy_sum / n, busy_max);
+  }
+}
+
 struct TrackScratch {
   DevBuf rec, len, ch, chips, out, done, status, state, prof;
   cudaStream_t copy_stream = nullptr;
@@ -1120,7 +1216,7 @@ static int track_core(const int8_t* rec, int64_t rec_stride, const int64_t* rec_
   a.avail = 0x7fffffffffffffffLL;
   a.state = g_trk.state.as<TrackState>();
   a.prof = nullptr;
-  const size_t prof_n = (size_t)nch * TRK_WARPS * TRK_PROF_N;
+  const size_t prof_n = (size_t)nch * TRK_WARPS * TRK_PROF_N + (size_t)nch * TRK_CTA_N;
   if (getenv("SGX_TRK_PROF")) {
     if (g_trk.prof.reserve(sizeof(long long) * prof_n)) return fail(SGX_ERR_CUDA, "cudaMalloc", "prof");
     SGX_CUDA(cudaMemsetAsync(g_trk.prof.p, 0, sizeof(long long) * prof_n, s));
@@ -1253,6 +1349,7 @@ static int track_core(const int8_t* rec, int64_t rec_stride, const int64_t* rec_
       fprintf(stderr, "[sgx prof] %d: %8.0f %8.0f %8.0f %8.0f %8.0f | %8.0f\n", w, acc[0] / per, acc[1] / per, acc[2] / per,
               acc[3] / per, acc[4] / per, tot / per);
     }
+    print_cta_makespan(hp.data() + (size_t)nch * TRK_WARPS * TRK_PROF_N, nch);
   }
   int rc = SGX_OK;
   for (int i = 0; i < nch; ++i)
