@@ -13,7 +13,7 @@
  * SGX_ERR_NODEV.
  *
  * Operands of the stages after tracking (sgx_find_preambles, sgx_pseudoranges, sgx_track_quality,
- * sgx_nav_solve, sgx_nav_velocity):
+ * sgx_nav_solve, sgx_nav_velocity, sgx_nav_integrity):
  *   - device operands are read and written in place, in the order of cuda_stream;
  *   - host inputs are copied to device scratch first.  An input that holds one series of ms values per
  *     channel, `stride` elements apart, is read in exactly those rows: nothing between or after them;
@@ -335,6 +335,69 @@ int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t n_recordin
                      const int32_t* n_epochs, int32_t max_epochs, const uint8_t* active, const double* sol,
                      const sgx_vel_settings* vs, double* vel, double* doppler, double* rr_resid, double* sat_vel,
                      double* sat_clk_drift, void* cuda_stream);
+
+/* ---- RAIM: fault detection and exclusion, protection levels (extension; no reference behaviour) ---------------- */
+#define SGX_INTEG_MAX_DOF 28   /* dof = channels - 4 <= 32 - 4 */
+
+/* The host computes the tables (postnav.raim_tables); the kernel evaluates no distribution.  Entry k is for
+ * dof = k + 1.  thresh[k]: chi-square upper quantile at the false-alarm probability Pfa, T = chi2.isf(Pfa, dof).
+ * pbias[k]: sqrt(lambda), lambda the noncentrality with ncx2.cdf(T, dof, lambda) = Pmd (missed detection). */
+typedef struct sgx_integ_settings {
+  double sigma;                         /* m: standard deviation of one pseudorange error */
+  double thresh[SGX_INTEG_MAX_DOF];
+  double pbias[SGX_INTEG_MAX_DOF];
+} sgx_integ_settings;
+
+#define SGX_NAV_INTEG_FIELDS 16  /* X Y Z dt latitude longitude height | q T dof | qFinal | HPL VPL |
+                                    status excluded nUsed */
+#define SGX_INTEG_NO_FIX 0       /* values of the status field */
+#define SGX_INTEG_UNAVAILABLE 1
+#define SGX_INTEG_OK 2
+#define SGX_INTEG_EXCLUDED 3
+#define SGX_INTEG_FAULT 4
+
+/* Receiver autonomous integrity monitoring of the fixes of sgx_nav_solve: a residual test of each epoch's pseudoranges,
+ * exclusion of one faulty channel, and horizontal / vertical protection levels.  Post hoc: an exclusion does not feed
+ * back into sgx_nav_solve's channel list or its next epoch.  Float64 throughout.
+ * For recording r and epoch e < n_epochs[r] whose fix sol[r][e][0..3] is finite:
+ *   S0 = channels with active[r][e][c] == 1, n = |S0|; p0 = (X, Y, Z, dt) = sol[r][e][0..3]; transmit time t = tow[r]
+ *   advanced by e repeated additions of nav_sol_period / 1000 (as sgx_nav_solve).
+ * Measurement model of a channel at p = (x, dt): satpos at t gives x_s and clk; obs = raw_p + clk*c; x_s rotated about
+ * z by 7.292115147e-5 * |x_s - x| / c (e_r_corr); trop = use_trop_corr ? tropo(sin el) with sgx_nav_solve's elevation
+ * at x and its constants : 0; rho = |x_s,rot - x|; y = obs - rho - dt - trop; row a = [-(x_s,rot - x)/rho, 1].
+ * The row is a true unit vector.  sgx_nav_solve divides its rows by obs instead (leastSquarePos's quirk, kept there for
+ * parity with the reference); the test does not inherit it.
+ * Test of a set S at p: N = sum a a^T (xor-butterfly sums over the lanes), x^ = N^-1 sum a y (Cholesky);
+ *   e_j = y_j - a_j . x^, SSE = sum e_j^2, q = SSE / sigma^2, dof = |S| - 4;
+ *   z_j = N^-1 a_j (column j of (H^T H)^-1 H^T), h_j = a_j . z_j; w_j = e_j / (sigma sqrt(1 - h_j)); a channel with
+ *   1 - h_j <= 1e-12 is not testable (w_j NaN);
+ *   z_j[0..2] rotated to ENU at sol's latitude and longitude: Hslope_j = sqrt(zE^2 + zN^2) / sqrt(1 - h_j),
+ *   Vslope_j = |zU| / sqrt(1 - h_j); HPL = sigma * pbias[dof-1] * max_j Hslope_j, VPL likewise with Vslope_j; both
+ *   +inf when a channel of S is not testable.
+ * Decision (status):
+ *   n < 5, or a Cholesky pivot of S0's N not above 1e-13 of its trace: UNAVAILABLE; q, T, qFinal, HPL, VPL NaN.
+ *   q <= thresh[dof-1]: OK.  The fix is sol's, bit for bit.
+ *   otherwise, when n >= 6: SSE_(j) = SSE - e_j^2 / (1 - h_j) for each testable j, j* = argmin (ties: lowest channel).
+ *     If SSE_(j*) / sigma^2 <= thresh[dof-2]: EXCLUDED.  S1 = S0 \ {j*} is solved by Gauss-Newton from p0 with the
+ *     model re-evaluated at every iterate, until the position step is below 1e-4 m or for 6 iterations; qFinal, HPL and
+ *     VPL are S1's test at the final iterate; latitude, longitude, height from cart2geo (sgx_nav_solve's).
+ *   otherwise (n == 5, no subset passes, or S1's normal matrix fails Cholesky): FAULT; the fix stays sol's, q, HPL, VPL
+ *   are S0's.
+ *   Epochs without a finite fix and epochs >= n_epochs[r]: NO_FIX, every value NaN, excluded -1, nUsed 0.
+ *   raw_p, active, sol  sgx_nav_solve's outputs [R][E][C], [R][E][C], [R][E][SGX_NAV_SOL_FIELDS], E = max_epochs
+ *   n_epochs, eph, tow  as given to sgx_nav_solve
+ *   st                  sgx_nav_solve's settings: c, nav_sol_period and use_trop_corr are read
+ * Outputs:
+ *   integ       double [R][E][SGX_NAV_INTEG_FIELDS]: the final fix (X Y Z dt latitude longitude height), q of S0,
+ *               thresh[dof-1], dof (= n - 4) of S0, qFinal (the final set's q; q unless EXCLUDED), HPL, VPL (m),
+ *               status, excluded channel (-1 for none), nUsed (channels of the final set)
+ *   norm_resid  double [R][E][C]: w_j of S0, NaN for channels outside S0 or not testable
+ * Deterministic: fixed reduction order, no atomics.  SGX_ERR_ARG for NULL pointers, 1..32 channels, n_recordings or
+ * max_epochs < 0, nav_sol_period < 1, c or sigma not finite and > 0, a thresh or pbias entry not finite and > 0. */
+int sgx_nav_integrity(const double* raw_p, const uint8_t* active, const double* sol, int32_t n_recordings,
+                      int32_t n_channels, int32_t max_epochs, const int32_t* n_epochs, const sgx_eph* eph,
+                      const double* tow, const sgx_nav_settings* st, const sgx_integ_settings* is, double* integ,
+                      double* norm_resid, void* cuda_stream);
 
 #ifdef __cplusplus
 }

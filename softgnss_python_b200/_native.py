@@ -36,7 +36,8 @@ def track_field(track_out, field):
 
 EXPORTS = ("sgx_abi_version", "sgx_last_error", "sgx_device_count", "sgx_set_device", "sgx_fp32_peak",
            "sgx_kernel_launch_count", "sgx_acquire", "sgx_track", "sgx_track_file", "sgx_synth_generate", "sgx_fft_c2c",
-           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality", "sgx_nav_velocity")
+           "sgx_find_preambles", "sgx_pseudoranges", "sgx_nav_solve", "sgx_track_quality", "sgx_nav_velocity",
+           "sgx_nav_integrity")
 
 
 class NativeError(RuntimeError):
@@ -54,6 +55,10 @@ EPH_FIELDS = ("t_oc", "a_f2", "a_f1", "a_f0", "T_GD", "sqrtA", "t_oe", "deltan",
               "C_uc", "C_us", "C_rc", "C_rs", "i_0", "iDot", "C_ic", "C_is", "omega_0", "omegaDot")   # sgx_eph, in order
 NAV_SOL_FIELDS = ("X", "Y", "Z", "dt", "GDOP", "PDOP", "HDOP", "VDOP", "TDOP", "latitude", "longitude", "height")
 NAV_VEL_FIELDS = ("VX", "VY", "VZ", "clkDrift", "VE", "VN", "VU", "nUsed")                  # SGX_NAV_VEL_FIELDS
+NAV_INTEG_FIELDS = ("X", "Y", "Z", "dt", "latitude", "longitude", "height", "q", "T", "dof", "qFinal", "HPL", "VPL",
+                    "status", "excluded", "nUsed")                                          # SGX_NAV_INTEG_FIELDS
+INTEG_STATUS = ("NO_FIX", "UNAVAILABLE", "OK", "EXCLUDED", "FAULT")                         # status field value = index
+INTEG_MAX_DOF = 28                                                                          # SGX_INTEG_MAX_DOF
 
 
 class SgxNavSettings(ctypes.Structure):
@@ -70,6 +75,11 @@ class SgxQualitySettings(ctypes.Structure):
 class SgxVelSettings(ctypes.Structure):
     _fields_ = [("IF", ctypes.c_double), ("c", ctypes.c_double), ("f_L1", ctypes.c_double),
                 ("nav_sol_period", ctypes.c_double), ("doppler_avg_ms", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
+class SgxIntegSettings(ctypes.Structure):
+    _fields_ = [("sigma", ctypes.c_double), ("thresh", ctypes.c_double * INTEG_MAX_DOF),
+                ("pbias", ctypes.c_double * INTEG_MAX_DOF)]
 
 
 class SgxSynthSpec(ctypes.Structure):
@@ -123,6 +133,8 @@ class Lib(object):
                                     vp, vp, vp, vp, vp, vp, vp, vp, vp]
         d.sgx_nav_velocity.argtypes = [vp, i64, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp,
                                        ctypes.POINTER(SgxVelSettings), vp, vp, vp, vp, vp, vp]
+        d.sgx_nav_integrity.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, vp, ctypes.POINTER(SgxNavSettings),
+                                        ctypes.POINTER(SgxIntegSettings), vp, vp, vp]
 
     def check(self, rc):
         if rc != 0:
@@ -269,6 +281,33 @@ class Lib(object):
                                              _ptr(active), _ptr(sol), ctypes.byref(vel_settings), _ptr(out["vel"]),
                                              _ptr(out["doppler"]), _ptr(out["rrResid"]), _ptr(out.get("satVel")),
                                              _ptr(out.get("satClkDrift")), ctypes.c_void_p(stream)))
+        return out
+
+    def nav_integrity(self, raw_p, active, sol, n_epochs, eph, tow, nav_settings, integ_settings, out=None, stream=0):
+        """RAIM fault detection / exclusion and protection levels per epoch (sgx_nav_integrity).  raw_p float64 /
+        active uint8 [n_rec][E][n_ch] and sol float64 [n_rec][E][12]: nav_solve's outputs (numpy or CUDA tensors);
+        n_epochs int32 [n_rec], eph float64 [n_rec][n_ch][21], tow float64 [n_rec] as for nav_solve; nav_settings:
+        SgxNavSettings; integ_settings: SgxIntegSettings.  ``out``: optional dict of preallocated outputs (integ
+        [n_rec][E][16], normResid [n_rec][E][n_ch]; numpy or CUDA tensors); by default numpy arrays are allocated.
+        Returns that dict."""
+        self.require_device()
+        if isinstance(raw_p, np.ndarray):
+            raw_p = np.ascontiguousarray(raw_p, dtype=np.float64)
+        if isinstance(active, np.ndarray):
+            active = np.ascontiguousarray(active, dtype=np.uint8)
+        if isinstance(sol, np.ndarray):
+            sol = np.ascontiguousarray(sol, dtype=np.float64)
+        n_rec, e_max, n_ch = (int(v) for v in active.shape)
+        assert tuple(raw_p.shape) == (n_rec, e_max, n_ch) and tuple(sol.shape) == (n_rec, e_max, len(NAV_SOL_FIELDS))
+        eph = np.ascontiguousarray(eph, dtype=np.float64).reshape(n_rec, n_ch, len(EPH_FIELDS))
+        tow = np.ascontiguousarray(tow, dtype=np.float64).reshape(n_rec)
+        n_epochs = np.ascontiguousarray(n_epochs, dtype=np.int32).reshape(n_rec)
+        if out is None:
+            out = dict(integ=np.empty((n_rec, e_max, len(NAV_INTEG_FIELDS))), normResid=np.empty((n_rec, e_max, n_ch)))
+        self.check(self.dll.sgx_nav_integrity(_ptr(raw_p), _ptr(active), _ptr(sol), n_rec, n_ch, e_max, _ptr(n_epochs),
+                                              _ptr(eph), _ptr(tow), ctypes.byref(nav_settings),
+                                              ctypes.byref(integ_settings), _ptr(out["integ"]), _ptr(out["normResid"]),
+                                              ctypes.c_void_p(stream)))
         return out
 
     # ------------------------------------------------------------------ synthetic recordings

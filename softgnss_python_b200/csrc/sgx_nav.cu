@@ -21,6 +21,8 @@
 //
 // nav_velocity_kernel (K10, an extension with no reference behaviour) reuses satpos_one and the helpers above: receiver
 // velocity and clock drift at the same epochs from the PLL's carrier frequency, one warp per (recording, epoch).
+// nav_integrity_kernel (K11, likewise an extension) runs a RAIM residual test on each fix, excludes one faulty channel
+// and gives protection levels, one warp per (recording, epoch), post hoc (nothing feeds back into K8).
 #include <math.h>
 
 #include "sgx_common.cuh"
@@ -606,6 +608,209 @@ __global__ void __launch_bounds__(128) nav_velocity_kernel(VelArgs a) {
   }
 }
 
+// ---- K11: RAIM fault detection and exclusion, protection levels (extension; contract in softgnss_b200.h) ----------
+struct IntegArgs {
+  const double* raw_p;         // [R][E][C]
+  const unsigned char* active; // [R][E][C]
+  const double* sol;           // [R][E][SGX_NAV_SOL_FIELDS]
+  const int* n_epochs;         // [R]
+  const sgx_eph* eph;          // [R][C]
+  const double* tow;           // [R]
+  int n_rec, n_ch, max_epochs;
+  sgx_nav_settings st;
+  sgx_integ_settings is;
+  double* integ;               // [R][E][SGX_NAV_INTEG_FIELDS]
+  double* norm_resid;          // [R][E][C]
+};
+
+// Prefit residual y and row a = [-(xs_rot - x)/rho, 1] of one channel at p = (x, dt).  Unlike K8 the row is a true
+// unit vector (K8 divides by obs, leastSquarePos's quirk), so N^-1 and the slopes below are those of the geometry.
+__device__ void integ_model(const double p[4], const double xs[3], double obs, double c_light, bool trop_on, double& y,
+                            double row[4]) {
+  const double dtr_deg = 3.141592653589793 / 180;
+  const double dx0 = xs[0] - p[0], dx1 = xs[1] - p[1], dx2 = xs[2] - p[2];
+  const double omegatau = 7.292115147e-05 * (sqrt(dx0 * dx0 + dx1 * dx1 + dx2 * dx2) / c_light);   // e_r_corr
+  double so, co;
+  sincos(omegatau, &so, &co);
+  const double r0 = co * xs[0] + so * xs[1], r1 = -so * xs[0] + co * xs[1], r2 = xs[2];
+  const double d0 = r0 - p[0], d1 = r1 - p[1], d2 = r2 - p[2];
+  double trop = 0.0;
+  if (trop_on) {                                       // K8's topocent and tropo at x
+    double phi, lam, hh;
+    togeod(p[0], p[1], p[2], phi, lam, hh);
+    double sl, cl, sb, cb;
+    sincos(lam * dtr_deg, &sl, &cl);
+    sincos(phi * dtr_deg, &sb, &cb);
+    const double E = -sl * d0 + cl * d1;
+    const double N = (-sb * cl) * d0 + (-sb * sl) * d1 + cb * d2;
+    const double U = (cb * cl) * d0 + (cb * sl) * d1 + sb * d2;
+    const double hor = sqrt(E * E + N * N);
+    const double el = hor < 1e-20 ? 90.0 : atan2(U, hor) / dtr_deg;
+    trop = tropo(sin(el * dtr_deg), 0.0, 1013.0, 293.0, 50.0, 0.0, 0.0, 0.0);
+  }
+  const double rho = sqrt(d0 * d0 + d1 * d1 + d2 * d2);
+  y = obs - rho - p[3] - trop;
+  row[0] = -d0 / rho; row[1] = -d1 / rho; row[2] = -d2 / rho; row[3] = 1.0;
+}
+
+// N = sum a a^T and the solution of N x = sum a y over the lanes (lanes outside the set pass a = 0, y = 0).
+__device__ __forceinline__ bool integ_normal(const double row[4], double y, double nrm[10], double x[4]) {
+  double rhs[4];
+  int k = 0;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+#pragma unroll
+    for (int j = i; j < 4; ++j) nrm[k++] = warp_add(row[i] * row[j]);
+    rhs[i] = warp_add(row[i] * y);
+  }
+  return chol4(nrm, rhs, x, nullptr);
+}
+
+__device__ __forceinline__ double warp_max(double v) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, d));
+  return v;
+}
+
+// Residual test of the channel set {lanes with `use`} at the point the rows were evaluated at.  Per lane: the
+// post-fit residual e and 1 - h (h = a . N^-1 a); for the set: SSE and the protection levels (+inf when a channel of
+// the set is not testable).  ENU at (sl, cl) = sin, cos of the longitude and (sb, cb) of the latitude.  false when
+// a Cholesky pivot of N is not above 1e-13 of its trace.
+struct IntegTest {
+  double sse, e, omh, hpl, vpl;
+};
+
+__device__ bool integ_test(bool use, double y, const double row[4], double sigma_pb, double sl, double cl, double sb,
+                           double cb, IntegTest& t) {
+  double nrm[10], xh[4], z[4];
+  if (!integ_normal(row, y, nrm, xh)) return false;
+  t.e = use ? y - (row[0] * xh[0] + row[1] * xh[1] + row[2] * xh[2] + row[3] * xh[3]) : 0.0;
+  t.sse = warp_add(t.e * t.e);
+  chol4(nrm, row, z, nullptr);                         // z = N^-1 a: column of (H^T H)^-1 H^T
+  t.omh = 1.0 - (row[0] * z[0] + row[1] * z[1] + row[2] * z[2] + row[3] * z[3]);
+  const bool testable = use && t.omh > 1e-12;
+  double hs = 0.0, vs = 0.0;
+  if (testable) {
+    const double ze = -sl * z[0] + cl * z[1];
+    const double zn = (-sb * cl) * z[0] + (-sb * sl) * z[1] + cb * z[2];
+    const double zu = (cb * cl) * z[0] + (cb * sl) * z[1] + sb * z[2];
+    const double s = sqrt(t.omh);
+    hs = sqrt(ze * ze + zn * zn) / s;
+    vs = fabs(zu) / s;
+  }
+  const bool untestable = __ballot_sync(0xffffffffu, use && !testable) != 0;
+  hs = warp_max(hs);
+  vs = warp_max(vs);
+  t.hpl = untestable ? inf_f64() : sigma_pb * hs;
+  t.vpl = untestable ? inf_f64() : sigma_pb * vs;
+  return true;
+}
+
+// One warp per (recording, epoch), lane = channel, after K8 and independent of K8's next epoch (post hoc).
+__global__ void __launch_bounds__(128) nav_integrity_kernel(IntegArgs a) {
+  const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (warp >= (long long)a.n_rec * a.max_epochs) return;
+  const int rec = (int)(warp / a.max_epochs), ep = (int)(warp % a.max_epochs);
+  const int C = a.n_ch;
+  const bool mine = lane < C;
+  const long long o = warp * C + lane;
+  double* out = a.integ + warp * SGX_NAV_INTEG_FIELDS;
+  const double* sol = a.sol + warp * SGX_NAV_SOL_FIELDS;
+  const int n_ep = min(a.n_epochs[rec], a.max_epochs);
+  if (ep >= n_ep || !(isfinite(sol[0]) && isfinite(sol[1]) && isfinite(sol[2]) && isfinite(sol[3]))) {
+    if (mine) a.norm_resid[o] = nan_f64();
+    if (lane < SGX_NAV_INTEG_FIELDS)
+      out[lane] = lane == 13 ? (double)SGX_INTEG_NO_FIX : lane == 14 ? -1.0 : lane == 15 ? 0.0 : nan_f64();
+    return;
+  }
+  const double c_light = a.st.c, sigma = a.is.sigma, dtr_deg = 3.141592653589793 / 180;
+  const bool trop_on = a.st.use_trop_corr != 0;
+  double transmit_time = a.tow[rec];                   // advanced as nav_solve_kernel does, bit for bit
+  for (int k = 0; k < ep; ++k) transmit_time += a.st.nav_sol_period / 1000;
+  const bool use0 = mine && a.active[o] != 0;
+  const int n = __popc(__ballot_sync(0xffffffffu, use0));
+  double xs[3] = {0.0, 0.0, 0.0}, obs = 0.0;
+  if (use0) {
+    double clk;
+    satpos_one(transmit_time, a.eph[(long long)rec * C + lane], xs, clk);
+    obs = a.raw_p[o] + clk * c_light;
+  }
+  double fix[7] = {sol[0], sol[1], sol[2], sol[3], sol[9], sol[10], sol[11]};
+  double q = nan_f64(), thr = nan_f64(), q_final = nan_f64(), hpl = nan_f64(), vpl = nan_f64(), w = nan_f64();
+  int status = SGX_INTEG_UNAVAILABLE, excluded = -1, n_used = n;
+  const int dof = n - 4;
+  double sl, cl, sb, cb;
+  sincos(sol[10] * dtr_deg, &sl, &cl);
+  sincos(sol[9] * dtr_deg, &sb, &cb);
+  const double sigma_pb = dof >= 1 ? sigma * a.is.pbias[dof - 1] : 0.0;
+  double y = 0.0, row[4] = {0.0, 0.0, 0.0, 0.0};
+  IntegTest t0;
+  if (n >= 5) {
+    const double p0[4] = {sol[0], sol[1], sol[2], sol[3]};
+    if (use0) integ_model(p0, xs, obs, c_light, trop_on, y, row);
+    if (integ_test(use0, y, row, sigma_pb, sl, cl, sb, cb, t0)) {
+      const bool testable = use0 && t0.omh > 1e-12;
+      q = t0.sse / (sigma * sigma);
+      thr = a.is.thresh[dof - 1];
+      q_final = q; hpl = t0.hpl; vpl = t0.vpl;
+      if (testable) w = t0.e / (sigma * sqrt(t0.omh));
+      if (q <= thr) {
+        status = SGX_INTEG_OK;
+      } else {
+        status = SGX_INTEG_FAULT;
+        if (n >= 6) {
+          // SSE without channel j, argmin with ties to the lowest channel
+          double smin = testable ? t0.sse - (t0.e * t0.e) / t0.omh : inf_f64();
+          int jstar = lane;
+#pragma unroll
+          for (int d = 16; d > 0; d >>= 1) {
+            const double ov = __shfl_xor_sync(0xffffffffu, smin, d);
+            const int oj = __shfl_xor_sync(0xffffffffu, jstar, d);
+            if (ov < smin || (ov == smin && oj < jstar)) { smin = ov; jstar = oj; }
+          }
+          if (smin / (sigma * sigma) <= a.is.thresh[dof - 2]) {
+            // Gauss-Newton on S1 = S0 \ {j*} from K8's fix, the model re-evaluated at every iterate
+            const bool use1 = use0 && lane != jstar;
+            const double sigma_pb1 = sigma * a.is.pbias[dof - 2];
+            double p[4] = {p0[0], p0[1], p0[2], p0[3]};
+            bool ok = true;
+            for (int it = 0; it < 6 && ok; ++it) {
+              double y1 = 0.0, row1[4] = {0.0, 0.0, 0.0, 0.0}, nrm[10], dx[4];
+              if (use1) integ_model(p, xs, obs, c_light, trop_on, y1, row1);
+              ok = integ_normal(row1, y1, nrm, dx);
+              if (ok) {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) p[i] = p[i] + dx[i];
+                if (sqrt(dx[0] * dx[0] + dx[1] * dx[1] + dx[2] * dx[2]) < 1e-4) break;
+              }
+            }
+            double y1 = 0.0, row1[4] = {0.0, 0.0, 0.0, 0.0};
+            IntegTest t1;
+            if (ok && use1) integ_model(p, xs, obs, c_light, trop_on, y1, row1);
+            if (ok && integ_test(use1, y1, row1, sigma_pb1, sl, cl, sb, cb, t1)) {
+              status = SGX_INTEG_EXCLUDED;
+              excluded = jstar;
+              n_used = n - 1;
+              q_final = t1.sse / (sigma * sigma);
+              hpl = t1.hpl; vpl = t1.vpl;
+              fix[0] = p[0]; fix[1] = p[1]; fix[2] = p[2]; fix[3] = p[3];
+              cart2geo(p[0], p[1], p[2], fix[4], fix[5], fix[6]);
+            }
+          }
+        }
+      }
+    }
+  }
+  if (mine) a.norm_resid[o] = w;
+  if (lane == 0) {
+#pragma unroll
+    for (int i = 0; i < 7; ++i) out[i] = fix[i];
+    out[7] = q; out[8] = thr; out[9] = (double)dof; out[10] = q_final; out[11] = hpl; out[12] = vpl;
+    out[13] = (double)status; out[14] = (double)excluded; out[15] = (double)n_used;
+  }
+}
+
 }  // namespace sgx
 
 using namespace sgx;
@@ -687,6 +892,44 @@ extern "C" int sgx_nav_velocity(const double* carr_freq, int64_t stride, int32_t
   const int threads = 128;                            // 4 (recording, epoch) warps per CTA
   const unsigned blocks = (unsigned)(((long long)n_recordings * max_epochs * 32 + threads - 1) / threads);
   SGX_COUNTED_LAUNCH(nav_velocity_kernel, dim3(blocks), dim3(threads), 0, s, a);
+  SGX_CUDA(cudaGetLastError());
+  return out.finish(s);
+}
+
+extern "C" int sgx_nav_integrity(const double* raw_p, const uint8_t* active, const double* sol, int32_t n_recordings,
+                                 int32_t n_channels, int32_t max_epochs, const int32_t* n_epochs, const sgx_eph* eph,
+                                 const double* tow, const sgx_nav_settings* st, const sgx_integ_settings* is,
+                                 double* integ, double* norm_resid, void* cuda_stream) {
+  if (sgx_device_count() <= 0) return fail(SGX_ERR_NODEV, "sgx_nav_integrity", "no CUDA device");
+  SGX_API_GUARD();
+  if (!raw_p || !active || !sol || !n_epochs || !eph || !tow || !st || !is || !integ || !norm_resid || n_channels < 1 ||
+      n_channels > 32 || n_recordings < 0 || max_epochs < 0)
+    return fail(SGX_ERR_ARG, "sgx_nav_integrity", "bad argument (NULL pointer, 1..32 channels, counts >= 0)");
+  if (!(st->nav_sol_period >= 1.0) || !isfinite(st->nav_sol_period) || !(st->c > 0) || !isfinite(st->c) ||
+      !(is->sigma > 0) || !isfinite(is->sigma))
+    return fail(SGX_ERR_ARG, "sgx_nav_integrity", "bad settings (nav_sol_period >= 1, c and sigma finite and > 0)");
+  for (int k = 0; k < SGX_INTEG_MAX_DOF; ++k)
+    if (!(is->thresh[k] > 0) || !isfinite(is->thresh[k]) || !(is->pbias[k] > 0) || !isfinite(is->pbias[k]))
+      return fail(SGX_ERR_ARG, "sgx_nav_integrity", "thresh and pbias entries must be finite and > 0");
+  if (n_recordings == 0 || max_epochs == 0) return SGX_OK;
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  static DevBuf b_raw, b_act, b_sol, b_nep, b_eph, b_tow, b_integ, b_res;
+  const size_t rc = (size_t)n_recordings * n_channels, rec = rc * max_epochs, n_sol = (size_t)n_recordings * max_epochs;
+  IntegArgs a;
+  StagedOutputs out;
+  int r;
+  if ((r = stage_in(raw_p, rec, b_raw, a.raw_p, s)) || (r = stage_in(active, rec, b_act, a.active, s)) ||
+      (r = stage_in(sol, n_sol * SGX_NAV_SOL_FIELDS, b_sol, a.sol, s)) ||
+      (r = stage_in(n_epochs, (size_t)n_recordings, b_nep, a.n_epochs, s)) || (r = stage_in(eph, rc, b_eph, a.eph, s)) ||
+      (r = stage_in(tow, (size_t)n_recordings, b_tow, a.tow, s)))
+    return r;
+  if ((r = out.add(integ, n_sol * SGX_NAV_INTEG_FIELDS, b_integ, a.integ)) ||
+      (r = out.add(norm_resid, rec, b_res, a.norm_resid)))
+    return r;
+  a.n_rec = n_recordings; a.n_ch = n_channels; a.max_epochs = max_epochs; a.st = *st; a.is = *is;
+  const int threads = 128;                            // 4 (recording, epoch) warps per CTA
+  const unsigned blocks = (unsigned)(((long long)n_recordings * max_epochs * 32 + threads - 1) / threads);
+  SGX_COUNTED_LAUNCH(nav_integrity_kernel, dim3(blocks), dim3(threads), 0, s, a);
   SGX_CUDA(cudaGetLastError());
   return out.finish(s);
 }

@@ -11,12 +11,16 @@ Mirrors, with the reference's names and conventions:
 
 Extension (no reference behaviour): receiver velocity and clock drift from the PLL's Doppler at the same epochs
 (``nav_velocity_batch``, ``post_navigate_batch(..., velocity=True)``, ``postNavigateVelocity``), computed by
-``sgx_nav_velocity`` (csrc/sgx_nav.cu).
+``sgx_nav_velocity`` (csrc/sgx_nav.cu).  Receiver autonomous integrity monitoring of the fix: a residual test, exclusion of
+one faulty channel and horizontal / vertical protection levels (``raim_tables``, ``nav_integrity_batch``,
+``post_navigate_batch(..., integrity=True)``, ``postNavigateIntegrity``), computed by ``sgx_nav_integrity``.
 
 ``find_preambles_batch`` is the batched entry point over a float64 ``[channels, ms]`` array or CUDA tensor
 (e.g. field 3 of ``track_batch``'s device-resident output).  There is no CPU implementation here: the
 work is done by ``sgx_find_preambles`` (csrc/sgx_bitsync.cu) and the call fails without a CUDA device.
 """
+import math
+
 import numpy as np
 
 from . import _native
@@ -232,6 +236,119 @@ def nav_velocity_batch(track_out, nav_out, sub_frame_start, eph, tow, settings, 
     return out
 
 
+# ---- RAIM tables: chi-square and noncentral chi-square in float64 with math only (scipy is not a dependency) -------------
+def _gamma_pq(a, x):
+    """Regularised incomplete gamma functions (P(a, x), Q(a, x)): series for x < a + 1, else Lentz's continued fraction
+    for Q (each accurate to a few ulp relative; the complement then to a few ulp absolute)."""
+    if x <= 0.0:
+        return 0.0, 1.0
+    lead = math.exp(a * math.log(x) - x - math.lgamma(a))
+    if x < a + 1.0:
+        term = s = 1.0 / a
+        n = 1
+        while term > s * 1e-17:
+            term *= x / (a + n)
+            s += term
+            n += 1
+        p = s * lead
+        return p, 1.0 - p
+    tiny = 1e-300
+    b = x + 1.0 - a
+    c, d = 1.0 / tiny, 1.0 / b
+    h = d
+    for i in range(1, 10000):
+        an = -i * (i - a)
+        b += 2.0
+        d = an * d + b
+        d = tiny if abs(d) < tiny else d
+        c = b + an / c
+        c = tiny if abs(c) < tiny else c
+        d = 1.0 / d
+        delta = d * c
+        h *= delta
+        if abs(delta - 1.0) < 1e-16:
+            break
+    q = lead * h
+    return 1.0 - q, q
+
+
+def _ncx2_cdf(x, k, lam):
+    """Noncentral chi-square CDF: sum_j Poisson(j; lam/2) P(k/2 + j, x/2), with P(a + 1, y) = P(a, y) - y^a e^-y /
+    Gamma(a + 1) from one accurate P(k/2, x/2)."""
+    y, a, m = 0.5 * x, 0.5 * k, 0.5 * lam
+    p = _gamma_pq(a, y)[0]
+    g = math.exp(a * math.log(y) - y - math.lgamma(a + 1.0))           # y^a e^-y / Gamma(a + 1)
+    total, j = 0.0, 0
+    while True:
+        w = math.exp(-m + (j * math.log(m) if m > 0 else 0.0) - math.lgamma(j + 1.0)) if (m > 0 or j == 0) else 0.0
+        total += w * p
+        if (j > m and w * p < 1e-20 * total) or p <= 0.0 or j > 100000:
+            return total
+        p = max(p - g, 0.0)
+        g *= y / (a + j + 1.0)
+        j += 1
+
+
+def _bisect(f, lo, hi):
+    """Root of a decreasing f on [lo, hi] (f(lo) > 0 > f(hi)) to the last bit."""
+    while True:
+        mid = 0.5 * (lo + hi)
+        if mid <= lo or mid >= hi:
+            return mid
+        if f(mid) > 0:
+            lo = mid
+        else:
+            hi = mid
+
+
+def raim_tables(pfa, pmd, max_dof=_native.INTEG_MAX_DOF):
+    """``(thresh, pbias)``, float64 ``[max_dof]``, entry k for dof = k + 1: the chi-square threshold T with upper tail
+    ``pfa`` (false alarm) and sqrt(lambda) of the noncentrality lambda whose noncentral chi-square CDF at T is ``pmd``
+    (missed detection).  The inputs of ``sgx_integ_settings``."""
+    assert 0 < pfa < 1 and 0 < pmd < 1 and max_dof >= 1
+    thresh, pbias = np.empty(max_dof), np.empty(max_dof)
+    for k in range(1, max_dof + 1):
+        hi = 2.0 * k + 10.0
+        while _gamma_pq(0.5 * k, 0.5 * hi)[1] > pfa:
+            hi *= 2.0
+        t = _bisect(lambda v: _gamma_pq(0.5 * k, 0.5 * v)[1] - pfa, 0.0, hi)
+        hi = t + 10.0
+        while _ncx2_cdf(t, k, hi) > pmd:
+            hi *= 2.0
+        lam = _bisect(lambda v: _ncx2_cdf(t, k, v) - pmd, 0.0, hi)
+        thresh[k - 1], pbias[k - 1] = t, math.sqrt(lam)
+    return thresh, pbias
+
+
+_TABLES = {}
+
+
+def integ_settings(settings):
+    """``sgx_integ_settings`` from the extension attributes ``raimSigma``, ``raimPfa`` and ``raimPmd``; an object without
+    them (the reference's own Settings) gets 5.0 m, 1e-5 and 1e-3."""
+    pfa, pmd = float(getattr(settings, "raimPfa", 1e-5)), float(getattr(settings, "raimPmd", 1e-3))
+    if (pfa, pmd) not in _TABLES:
+        _TABLES[(pfa, pmd)] = raim_tables(pfa, pmd)
+    thresh, pbias = _TABLES[(pfa, pmd)]
+    st = _native.SgxIntegSettings()
+    st.sigma = float(getattr(settings, "raimSigma", 5.0))
+    st.thresh[:] = thresh.tolist()
+    st.pbias[:] = pbias.tolist()
+    return st
+
+
+def nav_integrity_batch(nav_out, eph, tow, settings, stream=0):
+    """RAIM at the epochs of ``nav_out`` (the dict of :func:`nav_solve_batch` or :func:`post_navigate_batch`; ``rawP``,
+    ``active``, ``sol`` and ``n_epochs`` are read), computed by ``sgx_nav_integrity`` (csrc/sgx_nav.cu; contract in
+    include/softgnss_b200.h).  ``eph`` ``[R, C, 21]`` and ``tow`` ``[R]``: what the fix was computed from.  Returns numpy
+    ``integ`` ``[R, E, 16]`` (``_native.NAV_INTEG_FIELDS``; status values index ``_native.INTEG_STATUS``) and
+    ``normResid`` ``[R, E, C]``.  There is no host implementation: without a device this raises NativeError."""
+    L = _native.lib()
+    L.require_device()
+    return L.nav_integrity(nav_out["rawP"], nav_out["active"], nav_out["sol"], nav_out["n_epochs"], eph, tow,
+                           nav_settings(settings), integ_settings(settings), stream=stream)
+
+
 def eph_rows(eph, prn):
     """Rows of ``_native.EPH_FIELDS`` for the channels' PRNs from the reference's ephemeris recarray
     (postNavigation.py:120-140: ``eph[PRN - 1].<field>``); channels without an ephemeris get zeros."""
@@ -350,7 +467,27 @@ def postNavigateVelocity(trackResults, settings):
     return nav, eph, velocities
 
 
-def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_done=None):
+def postNavigateIntegrity(trackResults, settings):
+    """:func:`postNavigate` plus the integrity of every measurement epoch (extension; no reference behaviour).  Returns
+    ``(navSolutions, eph, navIntegrity)``, ``(None, None, None)`` where postNavigate returns ``(None, None)``.
+    ``navIntegrity`` is a one-record recarray with the length-E fields of ``_native.NAV_INTEG_FIELDS`` -- the final fix
+    ``X Y Z dt latitude longitude height`` (K8's unless a channel was excluded), the all-in-view statistic ``q``, its
+    threshold ``T`` and ``dof``, ``qFinal``, the protection levels ``HPL VPL`` (m), ``status`` (index into
+    ``_native.INTEG_STATUS``), ``excluded`` (channel, -1 for none), ``nUsed`` -- and ``normResid``
+    ``[numberOfChannels, E]``.  Settings: ``raimSigma`` (m), ``raimPfa``, ``raimPmd``."""
+    r = _post_navigate(trackResults, settings)
+    if r is None:
+        return None, None, None
+    nav, eph, out = r
+    g = nav_integrity_batch(out, out["ephRows"], out["tow"], settings)
+    integ = g["integ"][0]
+    cols = [integ[:, k].copy() for k in range(len(_native.NAV_INTEG_FIELDS))]
+    integrity = np.rec.array([tuple(cols) + (g["normResid"][0].T.copy(),)], formats=['O'] * 17,
+                             names=','.join(_native.NAV_INTEG_FIELDS) + ',normResid')
+    return nav, eph, integrity
+
+
+def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_done=None, integrity=False):
     """The same chain for R recordings whose tracking result ``track_out`` (float64 ``[R, C, 13, ms]``, numpy or
     CUDA tensor as written by ``track_batch``) stays where it is: ``I_P`` and ``absoluteSample`` are read in
     place by the two device stages; only the 1501 hard bits per channel and the solutions cross to the host.
@@ -358,7 +495,8 @@ def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_d
     ``subFrameStart`` ``[R, C]``, ``ready`` ``[R, C]``, ``tow`` ``[R]`` and ``eph`` (R lists indexed by PRN-1);
     recordings with fewer than four usable satellites get ``n_epochs = 0``.  With ``velocity=True`` the dict also
     carries ``vel``, ``doppler`` and ``rrResid`` of :func:`nav_velocity_batch` (carrFreq read in place; ``ms_done``
-    ``[R, C]`` as returned by ``track_batch``, None for all ms)."""
+    ``[R, C]`` as returned by ``track_batch``, None for all ms).  With ``integrity=True`` it also carries ``integ`` and
+    ``normResid`` of :func:`nav_integrity_batch`."""
     r, c, _, ms = track_out.shape
     prn = np.asarray(prn).reshape(r, c)
     L = _native.lib()
@@ -385,6 +523,8 @@ def post_navigate_batch(track_out, prn, settings, stream=0, velocity=False, ms_d
     out.update(subFrameStart=first, ready=ready, tow=tow, eph=ephs)
     if velocity:
         out.update(nav_velocity_batch(track_out, out, first, rows, tow, settings, ms_done=ms_done, stream=stream))
+    if integrity:
+        out.update(nav_integrity_batch(out, rows, tow, settings, stream=stream))
     return out
 
 

@@ -22,6 +22,10 @@ object lacks them): ``CNoVSMinterval`` (40 code periods per C/N0 estimate, Matla
 (0.5, cos 2 dphi): a window counts as locked when its C/N0 and its carrier-lock indicator reach both.
 Velocity extensions, read by ``postnav.nav_velocity_batch`` / ``postNavigateVelocity`` (same defaults for an object
 without them): ``dopplerAvgMs`` (100 code periods of carrFreq averaged per Doppler) and ``L1Freq`` (1575.42e6 Hz).
+Integrity (RAIM) extensions, read by ``postnav.nav_integrity_batch`` / ``postNavigateIntegrity`` (same defaults for an
+object without them): ``raimSigma`` (5.0 m, the standard deviation assumed for one pseudorange error -- a judgement, not
+a measurement of tracked-range noise), ``raimPfa`` (1e-5, false-alarm probability of the residual test) and ``raimPmd``
+(1e-3, missed-detection probability behind the protection levels).
 """
 import ctypes
 
@@ -80,7 +84,7 @@ class Settings(object):
         # extensions (defaults == reference behaviour)
         acqDopplerStep=500.0, acqCoherentMs=1, acqNonCoherentBlocks=2,
         CNoVSMinterval=40, CNoAccTime=0.001, lockCNoMin=30.0, lockPllMin=0.5,
-        dopplerAvgMs=100, L1Freq=1575.42e6,
+        dopplerAvgMs=100, L1Freq=1575.42e6, raimSigma=5.0, raimPfa=1e-5, raimPmd=1e-3,
     )
 
     def __init__(self, **overrides):
